@@ -2,6 +2,7 @@
 """bench.py — throughput of the light-cone mass-map hot path on B200 (and of the reference's CPU path beside it).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c4|c5] [--scaling strong|weak]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (BASELINE.json configs; synthetic uniform particles from a counter hash, resident in HBM before the timed region):
@@ -393,6 +394,56 @@ def run_light_cones(wl: Workload, steps, warmup, world, barrier, max_over_ranks)
     return ms, st, (t0, t1), int(st.flagged_pairs - f0)
 
 
+DUMP_MAP_BYTES = 40 << 20  # the maps; with the sample's float64 pixel indices and the small arrays < 64e6 bytes in all
+DUMP_SEED = 20240229
+
+
+def dump_outputs(wl: Workload, out_dir, rank=0, world=1):
+    """The planes of every group of the last timed light cone, as slicer_fetch hands them to a caller: per plane (and map type)
+    the float32 map, accepted and in-grid counts, plus the map's float64 sum over all pixels.  The last two groups are read from
+    the accumulator slots the timed step left them in.  The two slot ranges alternate, so the earlier groups were overwritten
+    within the step: they are deposited again here, after the timed region, with the calls the step makes (integer accumulators:
+    the same planes).  Maps larger than the budget are cut to one fixed, seeded sample of pixels, the same for every map
+    (pixel_index.npy).  Every rank takes part (the reduces); rank 0 writes DIR/group<g>_*.npy."""
+    W = wl.W
+    npix, ngr = W["npix"], W["ngroups"]
+    types = [0, 1, 4] if W["per_type"] else [-1]  # per-type maps: the types _stage_hydro stages
+    nmaps = ngr * LENS_PER_SNAP * len(types)
+    size = npix * npix
+    sample = None
+    if nmaps * size * 4 > DUMP_MAP_BYTES:
+        sample = np.sort(np.random.default_rng(DUMP_SEED).choice(size, DUMP_MAP_BYTES // (4 * nmaps), replace=False))
+    sfx = {t: "" if t < 0 else f"_type{t}" for t in types}
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+    # the groups still in their slots first, then the earlier ones through slot 0
+    for g in [g for g in (ngr - 1, ngr - 2) if g >= 0] + list(range(ngr - 2)):
+        slot = (g & 1) * LENS_PER_SNAP if g >= ngr - 2 else 0
+        if g < ngr - 2:
+            wl.s.deposit_slots(wl.groups[g], slot)
+            if world > 1:
+                wl.s.reduce_slots(slot, LENS_PER_SNAP, 0)
+            else:
+                wl.s.settle_slots(slot, LENS_PER_SNAP)
+        if rank != 0:
+            continue
+        out = {"counts": [], "ingrid": []}
+        for t in types:
+            out["maps" + sfx[t]], out["map_sums" + sfx[t]] = [], []
+        for k in range(LENS_PER_SNAP):
+            for t in types:
+                m, c, i = wl.s.fetch(slot + k, t, npix)
+                m = m.reshape(-1)
+                out["map_sums" + sfx[t]].append(m.sum(dtype=np.float64))
+                out["maps" + sfx[t]].append(m if sample is None else m[sample])
+            out["counts"].append(c.astype(np.float64))  # accepted pairs per type, whichever map was fetched
+            out["ingrid"].append(i.astype(np.float64))
+        for key, v in out.items():
+            np.save(os.path.join(out_dir, f"group{g}_{key}.npy"), np.stack(v))
+    if sample is not None and rank == 0:
+        np.save(os.path.join(out_dir, "pixel_index.npy"), sample.astype(np.float64))
+
+
 def per_group_times(wl: Workload):
     out = []
     for g in range(wl.W["ngroups"]):
@@ -476,8 +527,9 @@ def verify_reduce(wl: Workload, world, rank, dist, group=-1):
     return bool(flag[0])
 
 
-def measure(args, name, scaling, steps, warmup, rank, world, local_rank, dist, sample_clocks, verify=True):
-    """One workload at the current world size -> dict of results (rank 0 holds the aggregated numbers)."""
+def measure(args, name, scaling, steps, warmup, rank, world, local_rank, dist, sample_clocks, verify=True, dump_dir=None):
+    """One workload at the current world size -> dict of results (rank 0 holds the aggregated numbers).  With `dump_dir`, rank 0
+    writes the planes of the last timed step there (dump_outputs)."""
     import torch
 
     def barrier():
@@ -505,6 +557,8 @@ def measure(args, name, scaling, steps, warmup, rank, world, local_rank, dist, s
         time.sleep(0.25)
         sampler.stop()
         clocks = sampler.summary(t0, t1)
+    if dump_dir:
+        dump_outputs(wl, dump_dir, rank, world)  # before per_group_times and the self-checks reuse the accumulator slots
     ngr = wl.W["ngroups"]
     passes = steps * ngr
     value = wl.total * passes / (ms * 1e-3)
@@ -563,7 +617,8 @@ def ours(args, rank, world, local_rank):
     except Exception:
         pass
 
-    res, wl = measure(args, args.workload, args.scaling, args.steps, args.warmup, rank, world, local_rank, dist, True)
+    res, wl = measure(args, args.workload, args.scaling, args.steps, args.warmup, rank, world, local_rank, dist, True,
+                      dump_dir=args.dump_outputs)
     W = wl.W
     roofline = roofline_of(res, peaks)
 
@@ -712,7 +767,15 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--deposit-mode", type=int, default=0, help="0 auto, 1 direct map atomics, 2 binned shared-memory tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the planes of every group of the last step (maps, map sums, counts, in-grid "
+                         "counts) as DIR/*.npy, < 64 MB in all: maps as one fixed, seeded sample of pixels where they are larger; "
+                         "the groups the step overwrote are deposited again, outside the timed region")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the planes of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -28,7 +28,7 @@ def reflib():
     from oracle import ref_bindings
 
     if not ref_bindings.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+        pytest.skip("the original SLICER build (oracle/_ref, made by oracle/Makefile from its sources) is absent")
     return ref_bindings.RefLib(ngp=False)
 
 
@@ -37,7 +37,7 @@ def reflib_ngp():
     from oracle import ref_bindings
 
     if not ref_bindings.available(ngp=True):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
+        pytest.skip("the original SLICER build (oracle/_ref, made by oracle/Makefile from its sources) is absent")
     return ref_bindings.RefLib(ngp=True)
 
 
