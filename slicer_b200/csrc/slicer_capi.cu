@@ -940,8 +940,9 @@ static int binned_gshift(const PassParams &P)
   return g;
 }
 
-// 0: direct map atomics; 1: binned.  When the planes' tiles exceed MAX_BINS (8192^2 maps) the records are still
-// produced once; the sort and the tile deposit then run window by window over the bins (binned_pass).
+// 0: direct map atomics; 1: binned.  When the planes' tiles exceed MAX_BINS even in groups of four (8192^2 maps from 8 planes
+// up, 16384^2 from 3) the records are still produced once; the sort and the tile deposit then run window by window over the
+// bins (binned_pass).
 static int use_binned(const slicer_handle *h, const PassParams &P, const SegmentDev &D)
 {
   if (!P.fast || h->cfg.deposit_mode == SLICER_DEPOSIT_DIRECT)

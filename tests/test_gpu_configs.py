@@ -88,9 +88,10 @@ def _oracle_group(oracle, pos, planes, npix, massarr1, frac_bits, do_ngp=False):
 @pytest.mark.parametrize("name,box,npix,ngroups,group", [("C3", 256000.0, 2048, 9, 8), ("C3", 256000.0, 2048, 9, 2), ("C5", 1000000.0, 8192, 6, 5)])
 def test_one_subfile_at_c3_and_c5_geometry_matches_oracle(oracle, name, box, npix, ngroups, group):
     """SURVEY.md §8(d): 'one sub-file x one plane' parity at the C3 (2048^2, 5 deg) and C5 (8192^2, 5 deg, piled boxes) geometries:
-    a 2^22-particle window of the bench's synthetic snapshot through the production path (AUTO: binned for these groups, with
-    bin windows at 8192^2) and through the forced-direct path, all four planes of the group against the oracle: accepted counts,
-    in-grid counts and int64 maps bit for bit."""
+    a 2^22-particle window of the bench's synthetic snapshot through the production path (AUTO: binned for these groups; at
+    8192^2 the four planes sort by groups of two tiles in a single window of 5000 bins) and through the forced-direct path, all
+    four planes of the group against the oracle: accepted counts, in-grid counts and int64 maps bit for bit.  The windowed
+    sorts and groups of four are held to the oracle in test_gpu_binned_regimes.py."""
     n = 1 << 22
     mass = 5.2
     raw = _light_cone_planes(box, 5.0, ngroups)[group * LENS_PER_SNAP:(group + 1) * LENS_PER_SNAP]
