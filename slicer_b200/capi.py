@@ -16,7 +16,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 # SLICER_B200_LIB: another build of the same CUDA library, e.g. the checked one (`make -C slicer_b200/csrc checked`)
 LIB_PATH = os.environ.get("SLICER_B200_LIB") or os.path.join(HERE, "_build", "libslicer_b200.so")
 
-MAX_PLANES = 16
+MAX_PLANES = 16  # planes per pass
+MAX_SLOTS = 64  # plane accumulators per handle (Config.max_planes)
 MAX_XFORMS = 8
 NTYPES = 6
 MAS_TSC, MAS_NGP = 0, 1
@@ -88,7 +89,7 @@ EXPORTS = [
     "slicer_frac_bits", "slicer_comm_unique_id", "slicer_comm_init_rank", "slicer_comm_init_all",
     "slicer_reduce_all", "slicer_wait_staging", "slicer_count_accepted", "slicer_deposit_degraded", "slicer_reset_stats", "slicer_timer_begin", "slicer_timer_end",
     "slicer_selftest_arith", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
-    "slicer_stage_synthetic_window", "slicer_settle_slots",
+    "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory",
 ]
 
 
@@ -114,6 +115,7 @@ def lib() -> C.CDLL:
     L = C.CDLL(LIB_PATH)
     L.slicer_last_error.restype = C.c_char_p
     L.slicer_device_count.argtypes = [C.POINTER(C.c_int)]
+    L.slicer_device_memory.argtypes = [C.c_int, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
     L.slicer_create.argtypes = [C.POINTER(Config), C.POINTER(C.c_void_p)]
     L.slicer_destroy.argtypes = [C.c_void_p]
     L.slicer_destroy.restype = None
@@ -162,6 +164,13 @@ def device_count() -> int:
     n = C.c_int(0)
     _check(lib().slicer_device_count(C.byref(n)))
     return n.value
+
+
+def device_memory(device: int = 0):
+    """-> (free, total) bytes of CUDA device `device`."""
+    free, total = C.c_size_t(0), C.c_size_t(0)
+    _check(lib().slicer_device_memory(int(device), C.byref(free), C.byref(total)))
+    return free.value, total.value
 
 
 def plane_desc(sgn, face, centre, rcase, ld, ld2, fovradiants, npix, nrepperp=0) -> PlaneDesc:

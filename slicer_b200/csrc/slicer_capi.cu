@@ -124,8 +124,8 @@ struct slicer_handle
   cudaEvent_t ev_zero_start = nullptr, ev_zero_done = nullptr;
   bool zero_pending = false;                       // the compute stream has not yet waited for ev_zero_done
   cudaEvent_t ev_pass_done = nullptr;              // compute -> comm_stream: the passes a reduce sums
-  cudaEvent_t ev_slot[SLICER_MAX_PLANES];          // comm_stream -> compute: the last reduce of accumulator slot q
-  bool slot_reducing[SLICER_MAX_PLANES];           // ev_slot[q] is pending
+  cudaEvent_t ev_slot[SLICER_MAX_SLOTS];           // comm_stream -> compute: the last reduce of accumulator slot q
+  bool slot_reducing[SLICER_MAX_SLOTS];            // ev_slot[q] is pending
   cudaEvent_t ev_copy = nullptr;
   cudaEvent_t ev_buf_done[2] = {nullptr, nullptr}; // last pass that read staging pool b
   cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;    // slicer_timer_*
@@ -149,7 +149,7 @@ struct slicer_handle
   double boxsize = 0;
   double massarr[SLICER_NTYPES] = {0, 0, 0, 0, 0, 0};
   int hydro = 0;
-  int plane_npix[SLICER_MAX_PLANES];
+  int plane_npix[SLICER_MAX_SLOTS];
   bool copy_pending = false;
   slicer_stats stats;
   size_t device_bytes = 0;
@@ -165,6 +165,7 @@ struct slicer_handle
   // Two banks: the passes of one set of planes (a non-accumulating pass and the accumulating ones behind it) append to one
   // bank, the next set to the other, so that a set can be settled — waiting for ITS last pass only, with the few deposits
   // on a stream of their own — while the passes of the next set run (slicer_settle_slots, slicer_reduce_slots).
+  // Which bank a new set takes: run_pass.
   struct DeferBank
   {
     DeferEntry *buf = nullptr;
@@ -173,7 +174,7 @@ struct slicer_handle
     unsigned *host_count = nullptr; // pinned: the counter as of the end of the bank's last pass (copied behind every pass)
     std::vector<SavedPass> passes;  // passes since the last settle; DeferEntry::pass indexes it
     cudaEvent_t ev_done = nullptr;  // behind the bank's last pass and the copies of its counter / list head
-    unsigned slot_mask = 0;         // accumulator slots the bank's passes deposit into
+    uint64_t slot_mask = 0;         // accumulator slots the bank's passes deposit into (bit q: slot q)
   };
   struct
   {
@@ -187,9 +188,9 @@ struct slicer_handle
   cudaEvent_t ev_settled = nullptr; // settle -> compute / comm_stream
   bool settle_pending = false;      // `compute` has not yet waited for ev_settled
   bool settle_pending_comm = false; // nor has `comm_stream`
-  cudaEvent_t slot_pass_ev[SLICER_MAX_PLANES]; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
+  cudaEvent_t slot_pass_ev[SLICER_MAX_SLOTS]; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
   bool fence_all = false;           // something other than a pass wrote accumulators on `compute` (degraded deposit): the next reduce waits for the whole stream
-  unsigned long long slot_epoch[SLICER_MAX_PLANES];
+  unsigned long long slot_epoch[SLICER_MAX_SLOTS];
   size_t pos_stride = 0, mass_stride = 0; // floats per staging pool (16-byte multiples)
   size_t pcap = 0, mcap = 0;              // particles / masses a pool holds, padding of the segments included
   // particles per slice the binned path will use (before allocation: what it would allocate)
@@ -234,6 +235,24 @@ extern "C" int slicer_device_count(int *count)
   return 0;
 }
 
+extern "C" int slicer_device_memory(int device, size_t *free_bytes, size_t *total_bytes)
+{
+  if (!free_bytes || !total_bytes)
+    return fail("slicer_device_memory: null argument");
+  int ndev = 0;
+  CU(cudaGetDeviceCount(&ndev));
+  if (device < 0 || device >= ndev)
+    return fail("slicer_device_memory: device %d out of range (have %d)", device, ndev);
+  int prev = 0;
+  CU(cudaGetDevice(&prev));
+  CU(cudaSetDevice(device));
+  const cudaError_t e = cudaMemGetInfo(free_bytes, total_bytes);
+  cudaSetDevice(prev);
+  if (e != cudaSuccess)
+    return fail("cudaMemGetInfo failed: %s", cudaGetErrorString(e));
+  return 0;
+}
+
 extern "C" int slicer_alloc_pinned(size_t bytes, void **out)
 {
   CU(cudaHostAlloc(out, bytes, cudaHostAllocDefault));
@@ -259,8 +278,8 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
 {
   if (!cfg || !out)
     return fail("slicer_create: null argument");
-  if (cfg->max_planes < 1 || cfg->max_planes > SLICER_MAX_PLANES)
-    return fail("slicer_create: max_planes must be 1..%d", SLICER_MAX_PLANES);
+  if (cfg->max_planes < 1 || cfg->max_planes > SLICER_MAX_SLOTS)
+    return fail("slicer_create: max_planes must be 1..%d (SLICER_MAX_SLOTS)", SLICER_MAX_SLOTS);
   if (cfg->npix_max < 1)
     return fail("slicer_create: npix_max must be positive");
   if (cfg->mas != SLICER_MAS_TSC && cfg->mas != SLICER_MAS_NGP)
@@ -273,7 +292,7 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
   if (cfg->device < 0 || cfg->device >= ndev)
     return fail("slicer_create: device %d out of range (have %d)", cfg->device, ndev);
   slicer_handle *h = new slicer_handle;
-  for (int q = 0; q < SLICER_MAX_PLANES; q++)
+  for (int q = 0; q < SLICER_MAX_SLOTS; q++)
   {
     h->ev_slot[q] = nullptr;
     h->slot_reducing[q] = false;
@@ -339,7 +358,7 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
     TRY(cudaEventCreateWithFlags(&h->ev_zero_start, cudaEventDisableTiming));
     TRY(cudaEventCreateWithFlags(&h->ev_zero_done, cudaEventDisableTiming));
     TRY(cudaEventCreateWithFlags(&h->ev_pass_done, cudaEventDisableTiming));
-    for (int q = 0; q < SLICER_MAX_PLANES; q++)
+    for (int q = 0; q < cfg->max_planes; q++)
       TRY(cudaEventCreateWithFlags(&h->ev_slot[q], cudaEventDisableTiming));
     TRY(cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
     TRY(cudaEventCreateWithFlags(&h->ev_buf_done[0], cudaEventDisableTiming));
@@ -370,7 +389,9 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
       break;
     if (cfg->mass_capacity && (rc = dev_alloc(h, &h->d_mass_pool, h->nbuf * h->mass_stride)))
       break;
-    h->defer.cap = 1u << 19;
+    // 2^19 entries (12 MiB) per bank and per 16 slots: one bank may hold the passes of every slot range (run_pass), and the
+    // flagged pairs (about 8 per million accepted pairs at the default guard) grow with the planes deposited between settles
+    h->defer.cap = (1u << 19) * (unsigned)((cfg->max_planes + SLICER_MAX_PLANES - 1) / SLICER_MAX_PLANES);
     if ((rc = dev_alloc(h, &h->d_ovf, 1)))
       break;
     for (int b = 0; b < 2 && !rc; b++)
@@ -393,7 +414,7 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
     h->d_mass = h->d_mass_pool;
     if ((rc = dev_alloc(h, &h->d_acc, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max)))
       break;
-    if ((rc = dev_alloc(h, &h->d_counts, (size_t)SLICER_MAX_PLANES * SLICER_NTYPES * 2)))
+    if ((rc = dev_alloc(h, &h->d_counts, (size_t)cfg->max_planes * SLICER_NTYPES * 2)))
       break;
     if ((rc = dev_alloc(h, &h->d_out, h->npix2max)))
       break;
@@ -406,7 +427,7 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
       break;
     }
     if (cudaMemsetAsync(h->d_acc, 0, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max * 8, h->compute) != cudaSuccess ||
-        cudaMemsetAsync(h->d_counts, 0, (size_t)SLICER_MAX_PLANES * SLICER_NTYPES * 2 * 8, h->compute) != cudaSuccess ||
+        cudaMemsetAsync(h->d_counts, 0, (size_t)cfg->max_planes * SLICER_NTYPES * 2 * 8, h->compute) != cudaSuccess ||
         cudaMemsetAsync(h->defer.bank[0].count, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
         cudaMemsetAsync(h->defer.bank[1].count, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
         cudaMemsetAsync(h->d_ovf, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
@@ -504,7 +525,7 @@ extern "C" void slicer_destroy(slicer_handle *h)
     cudaEventDestroy(h->ev_zero_done);
   if (h->ev_pass_done)
     cudaEventDestroy(h->ev_pass_done);
-  for (int q = 0; q < SLICER_MAX_PLANES; q++)
+  for (int q = 0; q < SLICER_MAX_SLOTS; q++)
     if (h->ev_slot[q])
       cudaEventDestroy(h->ev_slot[q]);
   if (h->compute)
@@ -727,6 +748,8 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
 {
   if (nplanes < 1 || nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: nplanes %d outside 1..%d (max_planes)", nplanes, h->cfg.max_planes);
+  if (nplanes > SLICER_MAX_PLANES) // (a handle may have more slots than one pass can fill)
+    return fail("slicer_deposit: %d planes in one pass, more than SLICER_MAX_PLANES (%d)", nplanes, SLICER_MAX_PLANES);
   memset(P, 0, sizeof(*P));
   // group planes by randomisation
   int xf_of[SLICER_MAX_PLANES];
@@ -1252,12 +1275,12 @@ static int resolve_bank(slicer_handle *h, int bi)
 // Settle what the passes into accumulator slots [lo, lo + n) deferred (n < 0: every pass submitted so far): the older bank first.
 static int resolve_deferred(slicer_handle *h, int lo = 0, int n = -1)
 {
-  unsigned mask = 0xffffffffu;
+  uint64_t mask = ~(uint64_t)0;
   if (n >= 0)
   {
     mask = 0;
-    for (int q = lo; q < lo + n && q < SLICER_MAX_PLANES; q++)
-      mask |= 1u << q;
+    for (int q = lo; q < lo + n && q < SLICER_MAX_SLOTS; q++)
+      mask |= (uint64_t)1 << q;
   }
   for (int k = 1; k <= 2; k++)
   {
@@ -1287,7 +1310,7 @@ static int wait_settled(slicer_handle *h, bool comm)
 // compute-stream work on accumulator slots [lo, lo + n) must follow the reduces still running on them
 static int wait_slot_reduces(slicer_handle *h, int lo, int n)
 {
-  for (int q = lo; q < lo + n && q < SLICER_MAX_PLANES; q++)
+  for (int q = lo; q < lo + n && q < SLICER_MAX_SLOTS; q++)
     if (h->slot_reducing[q])
     {
       CU(cudaStreamWaitEvent(h->compute, h->ev_slot[q], 0));
@@ -1304,6 +1327,8 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     return 1;
   if (first_slot < 0 || nplanes < 1 || first_slot + nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: slots %d..%d outside 0..%d (max_planes)", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
+  if (nplanes > SLICER_MAX_PLANES)
+    return fail("slicer_deposit: %d planes in one pass, more than SLICER_MAX_PLANES (%d)", nplanes, SLICER_MAX_PLANES);
   int slot_of[SLICER_MAX_PLANES];
   for (int i = 0; i < nplanes; i++)
     slot_of[i] = first_slot + i;
@@ -1318,12 +1343,24 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     CU(cudaStreamWaitEvent(h->compute, h->ev_copy, 0));
     h->copy_pending = false;
   }
-  // a new set of planes takes the other bank (settled first, if the caller has not done so: its passes are two sets back)
+  // A new set of planes takes the other bank when that bank is settled (a caller that alternates between two slot ranges and
+  // settles or reduces one range behind the next pass finds it so every time), or when it zeroes slots the current bank holds
+  // (the other bank is then settled first: its passes are two sets back).  A set into other slots, submitted while both banks
+  // hold passes, joins the current bank: several sets deposited before any is settled (the first passes of several light cones
+  // over one sub-file: A, B, C non-accumulating, then A, B, C accumulating) so never make the host wait for a running pass.
+  // Every pass sits in one bank with the epochs of its slots; resolve_deferred settles each bank that holds a pass into the
+  // slots it is asked for.
   if (!accumulate)
   {
-    h->defer.cur ^= 1;
-    if (resolve_bank(h, h->defer.cur))
-      return 1;
+    uint64_t mine = 0;
+    for (int q = first_slot; q < first_slot + nplanes; q++)
+      mine |= (uint64_t)1 << q;
+    if (h->defer.bank[h->defer.cur ^ 1].passes.empty() || (h->defer.bank[h->defer.cur].slot_mask & mine))
+    {
+      h->defer.cur ^= 1;
+      if (resolve_bank(h, h->defer.cur))
+        return 1;
+    }
   }
   if (h->defer.bank[h->defer.cur].passes.size() >= 4096 && resolve_bank(h, h->defer.cur))
     return 1;
@@ -1362,7 +1399,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     for (int k = 0; k < P.nplanes; k++)
     {
       sp.epoch[k] = h->slot_epoch[P.pl[k].slot];
-      B.slot_mask |= 1u << P.pl[k].slot;
+      B.slot_mask |= (uint64_t)1 << P.pl[k].slot;
     }
     B.passes.push_back(sp);
   }
@@ -1465,6 +1502,8 @@ static int degrade_prepare(slicer_handle *h, const slicer_plane_desc *planes, in
     return fail("null argument");
   if (set_device(h))
     return 1;
+  if (nplanes > SLICER_MAX_PLANES)
+    return fail("Part. Degradation: %d planes in one pass, more than SLICER_MAX_PLANES (%d)", nplanes, SLICER_MAX_PLANES);
   if (build_pass(h, planes, nplanes, P))
     return 1;
   for (int q = 0; q < nplanes; q++)

@@ -31,6 +31,7 @@ def lib():
         L.shost_write_fits.argtypes = [C.c_char_p, _f32p, C.c_int, C.c_int, C.POINTER(C.c_char_p), _f64p, C.c_int, C.POINTER(C.c_char_p),
                                        np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS")]
         L.shost_run_light_cone.argtypes = [C.c_char_p, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.shost_run_light_cones.argtypes = [C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
         _lib = L
     return _lib
 
@@ -110,6 +111,16 @@ def write_fits(path, image, dkeys, ikeys):
 def run_light_cone(ini, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0):
     dev = np.ascontiguousarray(devices, np.int32)
     return lib().shost_run_light_cone(ini.encode(), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode))
+
+
+def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0, max_slots=0):
+    """One light cone per ini (realisations of one plan: other seeds, other outputs), every snapshot read once for all (once per
+    group of planes that fits `max_slots` accumulators per GPU, when given).  Returns 0 on success; inis that disagree on the
+    plan are refused before anything is written."""
+    dev = np.ascontiguousarray(devices, np.int32)
+    arr = (C.c_char_p * len(inis))(*[str(i).encode() for i in inis])
+    return lib().shost_run_light_cones(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
+                                       int(max_slots))
 
 
 def read_fits(path):

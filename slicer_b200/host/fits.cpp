@@ -150,7 +150,7 @@ void writeMaps(const InputParams &p, const Header &data, const Lens &lens, int i
       order.push_back("m" + std::to_string(i));
     }
     const std::string fileoutput = fileOutput(p, snappl);
-    std::cout << "Saving the maps on: " << fileoutput << std::endl;
+    std::cout << "Saving the maps on: " + fileoutput + "\n" << std::flush; // one insertion: planes are written on several threads
     writeFitsImage(fileoutput, &mapxytotrecv[0], p.npix, d, k, order);
     return;
   }

@@ -202,4 +202,19 @@ extern "C"
     o.quiet = true;
     return runLightCone(ini, o);
   }
+
+  // one light cone per ini, every snapshot read once for all (runLightCones)
+  int shost_run_light_cones(const char **inis, int nini, const int *devices, int ndev, int replication, int fixed_vertex, int ngp,
+                            int deposit_mode, int max_slots)
+  {
+    RunOptions o;
+    o.devices.assign(devices, devices + ndev);
+    o.replication = replication != 0;
+    o.fixed_vertex = fixed_vertex != 0;
+    o.mas = ngp ? SLICER_MAS_NGP : SLICER_MAS_TSC;
+    o.deposit_mode = deposit_mode;
+    o.quiet = true;
+    o.max_slots = max_slots;
+    return runLightCones(std::vector<std::string>(inis, inis + nini), o);
+  }
 }

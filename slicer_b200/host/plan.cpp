@@ -409,19 +409,25 @@ int buildPlanes(InputParams &p, Lens &lens, std::vector<double> &snapred, std::v
   lens.nplanes = total;
   if (myid != 0)
     return 0;
-  // report + planes_list_<suffix>.txt: one row per plane, columns as Lens/kslicer.py:29 reads them
-  //   index   z(middle)   near edge   far edge   last plane of the snapshot run   snapshot   z(snapshot)  first of a group
   std::cout << " light cone to " << p.Ds << " Mpc/h comoving: " << total << " planes from " << snapred.size() << " snapshots" << std::endl;
-  std::ofstream list((p.directory + "planes_list_" + p.suffix + ".txt").c_str());
   for (int i = 0; i < total; i++)
   {
     const PlanePlan &pl = plan[i];
     std::cout << "   plane " << i << ": " << pl.near_edge << " - " << pl.far_edge << " Mpc/h, z = " << pl.z_mid << ", cut from " << snappath[pl.snap]
               << (pl.new_group ? "  [new randomisation]" : "") << std::endl;
-    list << i << "   " << pl.z_mid << "   " << pl.near_edge << "   " << pl.far_edge << "   " << pl.run_end << "   " << snappath[pl.snap] << "   "
-         << snapred[pl.snap] << "  " << pl.new_group << std::endl;
   }
+  writePlanesList(p, lens);
   return 0;
+}
+
+// planes_list_<suffix>.txt: one row per plane, columns as Lens/kslicer.py:29 reads them
+//   index   z(middle)   near edge   far edge   last plane of the snapshot run   snapshot   z(snapshot)  first of a group
+void writePlanesList(const InputParams &p, const Lens &lens)
+{
+  std::ofstream list((p.directory + "planes_list_" + p.suffix + ".txt").c_str());
+  for (int i = 0; i < lens.nplanes; i++)
+    list << i << "   " << lens.zsimlens[i] << "   " << lens.ld[i] << "   " << lens.ld2[i] << "   " << lens.replication[i] << "   " << lens.fromsnap[i]
+         << "   " << lens.zfromsnap[i] << "  " << (bool)lens.randomize[i] << std::endl;
 }
 
 void GlibcRand::seed(unsigned int s)
