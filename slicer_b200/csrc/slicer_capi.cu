@@ -189,7 +189,6 @@ struct slicer_handle
   bool settle_pending = false;      // `compute` has not yet waited for ev_settled
   bool settle_pending_comm = false; // nor has `comm_stream`
   cudaEvent_t slot_pass_ev[SLICER_MAX_SLOTS]; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
-  bool fence_all = false;           // something other than a pass wrote accumulators on `compute` (degraded deposit): the next reduce waits for the whole stream
   unsigned long long slot_epoch[SLICER_MAX_SLOTS];
   size_t pos_stride = 0, mass_stride = 0; // floats per staging pool (16-byte multiples)
   size_t pcap = 0, mcap = 0;              // particles / masses a pool holds, padding of the segments included
@@ -217,6 +216,7 @@ struct slicer_handle
     unsigned char *cnt = nullptr, *keep = nullptr;
     unsigned *rank = nullptr, *block_sums = nullptr;
     size_t stride = 0, nblocks = 0, keep_cap = 0;
+    size_t bytes = 0; // device bytes of cnt, rank and block_sums
     int nplanes = 0;
     bool valid = false;
     unsigned long long plane_total[SLICER_MAX_PLANES];
@@ -743,8 +743,8 @@ static float float_floor(double d)
 }
 static bool is_f32(double d) { return (double)(float)d == d; }
 
-// slot_of: accumulator slot (the caller's plane index) of planes[i]; nullptr => i (the usual case)
-static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, PassParams *P, const int *slot_of = nullptr)
+// planes[i] deposits into accumulator slot first_slot + i
+static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, PassParams *P, int first_slot = 0)
 {
   if (nplanes < 1 || nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: nplanes %d outside 1..%d (max_planes)", nplanes, h->cfg.max_planes);
@@ -871,7 +871,7 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
         if (L.nt > 20)
           L.nt = 0;
       }
-      const int slot = slot_of ? slot_of[i] : i;
+      const int slot = first_slot + i;
       L.acc = h->d_acc + (size_t)slot * h->ntypes_alloc * h->npix2max;
       L.counts = h->d_counts + (size_t)slot * SLICER_NTYPES * 2;
       L.type_stride = h->cfg.per_type_maps ? h->npix2max : 0;
@@ -1319,6 +1319,57 @@ static int wait_slot_reduces(slicer_handle *h, int lo, int n)
   return 0;
 }
 
+// staged particles must be on the device before the compute stream reads them
+static int staging_fence(slicer_handle *h)
+{
+  if (h->copy_pending)
+  {
+    CU(cudaEventRecord(h->ev_copy, h->copy));
+    CU(cudaStreamWaitEvent(h->compute, h->ev_copy, 0));
+    h->copy_pending = false;
+  }
+  return 0;
+}
+
+// Every write into accumulator slots [lo, lo + n) on the compute stream claims them first: it follows the reduces still reading
+// them and the deposits of the pairs libm settled.  A write that does not accumulate also zeroes them and voids the pairs earlier
+// passes into them deferred; large accumulators are zeroed on `aux`, so the writer calls maps_ready before it touches them.
+static int claim_slots(slicer_handle *h, int lo, int n, bool accumulate)
+{
+  if (wait_slot_reduces(h, lo, n) || wait_settled(h, false))
+    return 1;
+  if (accumulate)
+    return 0;
+  const size_t zbytes = (size_t)n * h->ntypes_alloc * h->npix2max * sizeof(unsigned long long);
+  unsigned long long *zptr = h->d_acc + (size_t)lo * h->ntypes_alloc * h->npix2max;
+  if (zbytes >= ((size_t)64 << 20))
+  { // (8192^2 planes: 2 GiB per pass, 0.7 ms on the compute stream) after everything queued so far, beside what comes next
+    if (maps_ready(h))
+      return 1;
+    CU(cudaEventRecord(h->ev_zero_start, h->compute));
+    CU(cudaStreamWaitEvent(h->aux, h->ev_zero_start, 0));
+    CU(cudaMemsetAsync(zptr, 0, zbytes, h->aux));
+    CU(cudaEventRecord(h->ev_zero_done, h->aux));
+    h->zero_pending = true;
+  }
+  else
+    CU(cudaMemsetAsync(zptr, 0, zbytes, h->compute));
+  CU(cudaMemsetAsync(h->d_counts + (size_t)lo * SLICER_NTYPES * 2, 0, (size_t)n * SLICER_NTYPES * 2 * sizeof(unsigned long long), h->compute));
+  for (int q = lo; q < lo + n; q++)
+    h->slot_epoch[q]++; // deferred particles of earlier passes into these accumulators are void
+  return 0;
+}
+
+// After a write into slots [lo, lo + n) on the compute stream: a reduce of them waits for `done`, or for the whole compute stream
+// when `done` is nullptr; the staging pool the write read may be overwritten behind it.
+static int slots_written(slicer_handle *h, int lo, int n, cudaEvent_t done)
+{
+  for (int q = lo; q < lo + n; q++)
+    h->slot_pass_ev[q] = done;
+  CU(cudaEventRecord(h->ev_buf_done[h->cur_buf], h->compute));
+  return 0;
+}
+
 static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, bool accumulate, int first_slot = 0)
 {
   if (!h || !planes)
@@ -1327,22 +1378,9 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     return 1;
   if (first_slot < 0 || nplanes < 1 || first_slot + nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: slots %d..%d outside 0..%d (max_planes)", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
-  if (nplanes > SLICER_MAX_PLANES)
-    return fail("slicer_deposit: %d planes in one pass, more than SLICER_MAX_PLANES (%d)", nplanes, SLICER_MAX_PLANES);
-  int slot_of[SLICER_MAX_PLANES];
-  for (int i = 0; i < nplanes; i++)
-    slot_of[i] = first_slot + i;
   PassParams P;
-  if (build_pass(h, planes, nplanes, &P, slot_of))
+  if (build_pass(h, planes, nplanes, &P, first_slot) || staging_fence(h))
     return 1;
-  if (wait_slot_reduces(h, first_slot, nplanes))
-    return 1;
-  if (h->copy_pending)
-  {
-    CU(cudaEventRecord(h->ev_copy, h->copy));
-    CU(cudaStreamWaitEvent(h->compute, h->ev_copy, 0));
-    h->copy_pending = false;
-  }
   // A new set of planes takes the other bank when that bank is settled (a caller that alternates between two slot ranges and
   // settles or reduces one range behind the next pass finds it so every time), or when it zeroes slots the current bank holds
   // (the other bank is then settled first: its passes are two sets back).  A set into other slots, submitted while both banks
@@ -1364,29 +1402,8 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
   }
   if (h->defer.bank[h->defer.cur].passes.size() >= 4096 && resolve_bank(h, h->defer.cur))
     return 1;
-  if (wait_settled(h, false))
+  if (claim_slots(h, first_slot, nplanes, accumulate))
     return 1;
-  if (!accumulate)
-  {
-    const size_t zbytes = (size_t)nplanes * h->ntypes_alloc * h->npix2max * sizeof(unsigned long long);
-    unsigned long long *zptr = h->d_acc + (size_t)first_slot * h->ntypes_alloc * h->npix2max;
-    if (zbytes >= ((size_t)64 << 20))
-    { // (8192^2 planes: 2 GiB per pass, 0.7 ms on the compute stream) after everything queued so far, beside what comes next
-      if (maps_ready(h))
-        return 1;
-      CU(cudaEventRecord(h->ev_zero_start, h->compute));
-      CU(cudaStreamWaitEvent(h->aux, h->ev_zero_start, 0));
-      CU(cudaMemsetAsync(zptr, 0, zbytes, h->aux));
-      CU(cudaEventRecord(h->ev_zero_done, h->aux));
-      h->zero_pending = true;
-    }
-    else
-      CU(cudaMemsetAsync(zptr, 0, zbytes, h->compute));
-    CU(cudaMemsetAsync(h->d_counts + (size_t)first_slot * SLICER_NTYPES * 2, 0, (size_t)nplanes * SLICER_NTYPES * 2 * sizeof(unsigned long long),
-                       h->compute));
-    for (int q = first_slot; q < first_slot + nplanes; q++)
-      h->slot_epoch[q]++; // deferred particles of earlier passes into these accumulators are void
-  }
   slicer_handle::DeferBank &B = h->defer.bank[h->defer.cur];
   DeferDev F;
   F.buf = B.buf;
@@ -1449,13 +1466,12 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
   if (maps_ready(h)) // (a pass without particles still leaves zeroed planes behind it in stream order)
     return 1;
   CU(cudaEventRecord(e1, h->compute));
-  for (int k = 0; k < P.nplanes; k++)
-    h->slot_pass_ev[P.pl[k].slot] = e1; // (a recycled ring entry stands for a later pass: waiting for it is still sufficient)
   // the bank's deferred list as of now, for resolve_bank
   CU(cudaMemcpyAsync(B.host_count, B.count, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaMemcpyAsync(B.host, B.buf, (size_t)DEFER_HEAD * sizeof(DeferEntry), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaEventRecord(B.ev_done, h->compute));
-  CU(cudaEventRecord(h->ev_buf_done[h->cur_buf], h->compute));
+  if (slots_written(h, first_slot, nplanes, e1)) // (a recycled ring entry stands for a later pass: waiting for it is still sufficient)
+    return 1;
   h->pass_head++;
   return 0;
 }
@@ -1500,21 +1516,11 @@ static int degrade_prepare(slicer_handle *h, const slicer_plane_desc *planes, in
 {
   if (!h || !planes)
     return fail("null argument");
-  if (set_device(h))
-    return 1;
-  if (nplanes > SLICER_MAX_PLANES)
-    return fail("Part. Degradation: %d planes in one pass, more than SLICER_MAX_PLANES (%d)", nplanes, SLICER_MAX_PLANES);
-  if (build_pass(h, planes, nplanes, P))
+  if (set_device(h) || build_pass(h, planes, nplanes, P))
     return 1;
   for (int q = 0; q < nplanes; q++)
     if ((2 * planes[q].nrepperp + 1) * (2 * planes[q].nrepperp + 1) > 255)
       return fail("Part. Degradation supports nrepperp <= 7");
-  if (h->copy_pending)
-  {
-    CU(cudaEventRecord(h->ev_copy, h->copy));
-    CU(cudaStreamWaitEvent(h->compute, h->ev_copy, 0));
-    h->copy_pending = false;
-  }
   size_t n = 0;
   for (size_t i = 0; i < h->segs.size(); i++)
     n += h->segs[i].n;
@@ -1522,11 +1528,38 @@ static int degrade_prepare(slicer_handle *h, const slicer_plane_desc *planes, in
   return 0;
 }
 
+// one degrade_kernel launch per resident segment with particles; G.seg_base: the segment's first particle in the batch
+template <int MODE>
+static int degrade_launch(slicer_handle *h, const PassParams &P, degrade::Dev G)
+{
+  G.seg_base = 0;
+  for (size_t si = 0; si < h->segs.size(); si++)
+  {
+    SegmentDev D;
+    fill_segment(h, h->segs[si], &D);
+    if (D.n)
+    {
+      const size_t want = (D.n + 255) / 256, cap = (size_t)h->sm_count * 16;
+      const int blocks = (int)(want < cap ? want : cap);
+      if (h->cfg.mas == SLICER_MAS_NGP)
+        degrade::degrade_kernel<SLICER_MAS_NGP, MODE><<<blocks, 256, 0, h->compute>>>(P, D, G);
+      else
+        degrade::degrade_kernel<SLICER_MAS_TSC, MODE><<<blocks, 256, 0, h->compute>>>(P, D, G);
+      CU(cudaGetLastError());
+      h->stats.launches++;
+      if (MODE == degrade::DEPOSIT)
+        h->stats.particles_streamed += D.n;
+    }
+    G.seg_base += D.n;
+  }
+  return 0;
+}
+
 extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, long long *counts)
 {
   PassParams P;
   size_t total = 0;
-  if (degrade_prepare(h, planes, nplanes, &P, &total))
+  if (degrade_prepare(h, planes, nplanes, &P, &total) || staging_fence(h))
     return 1;
   if (!counts)
     return fail("slicer_count_accepted: null output");
@@ -1548,14 +1581,18 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
     cudaFree(h->deg.cnt);
     cudaFree(h->deg.rank);
     cudaFree(h->deg.block_sums);
+    h->device_bytes -= h->deg.bytes;
     h->deg.cnt = nullptr;
     h->deg.rank = nullptr;
     h->deg.block_sums = nullptr;
     const size_t stride = total + total / 8 + 1024;
     const size_t nblocks = (stride + 1 + degrade::SCAN_BLOCK * degrade::SCAN_PER - 1) / (degrade::SCAN_BLOCK * degrade::SCAN_PER);
     const int np = nplanes > h->deg.nplanes ? nplanes : h->deg.nplanes;
-    if (dev_alloc(h, &h->deg.cnt, (size_t)np * stride) || dev_alloc(h, &h->deg.rank, (size_t)np * (stride + 1)) ||
-        dev_alloc(h, &h->deg.block_sums, (size_t)np * nblocks))
+    const size_t before = h->device_bytes;
+    const int rc = dev_alloc(h, &h->deg.cnt, (size_t)np * stride) || dev_alloc(h, &h->deg.rank, (size_t)np * (stride + 1)) ||
+                   dev_alloc(h, &h->deg.block_sums, (size_t)np * nblocks);
+    h->deg.bytes = h->device_bytes - before;
+    if (rc)
       return 1;
     h->deg.stride = stride;
     h->deg.nblocks = nblocks;
@@ -1568,28 +1605,11 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
   G.cnt = h->deg.cnt;
   G.rank = h->deg.rank;
   G.stride = stride;
-  std::vector<size_t> seg_start;
-  size_t base = 0;
-  for (size_t si = 0; si < h->segs.size(); si++)
-  {
-    SegmentDev D;
-    fill_segment(h, h->segs[si], &D);
-    seg_start.push_back(base);
-    if (D.n)
-    {
-      G.seg_base = base;
-      const size_t want = (D.n + 255) / 256, cap = (size_t)h->sm_count * 16;
-      const int blocks = (int)(want < cap ? want : cap);
-      if (h->cfg.mas == SLICER_MAS_NGP)
-        degrade::degrade_kernel<SLICER_MAS_NGP, degrade::MARK><<<blocks, 256, 0, h->compute>>>(P, D, G);
-      else
-        degrade::degrade_kernel<SLICER_MAS_TSC, degrade::MARK><<<blocks, 256, 0, h->compute>>>(P, D, G);
-      CU(cudaGetLastError());
-      h->stats.launches++;
-    }
-    base += D.n;
-  }
-  seg_start.push_back(base);
+  if (degrade_launch<degrade::MARK>(h, P, G))
+    return 1;
+  std::vector<size_t> seg_start(1, 0); // first particle of each segment in the batch, then the total
+  for (const Segment &sg : h->segs)
+    seg_start.push_back(seg_start.back() + sg.n);
   const size_t nb = (total + 1 + degrade::SCAN_BLOCK * degrade::SCAN_PER - 1) / (degrade::SCAN_BLOCK * degrade::SCAN_PER);
   const dim3 grid((unsigned)nb, (unsigned)nplanes);
   degrade::scan_block_sums<<<grid, degrade::SCAN_BLOCK, 0, h->compute>>>(h->deg.cnt, stride, total, h->deg.block_sums, h->deg.nblocks);
@@ -1614,6 +1634,8 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
   return 0;
 }
 
+// Writes accumulator slots [0, nplanes) like a pass, but leaves their slot_pass_ev empty: a reduce of them waits for the whole
+// compute stream.
 extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, int snopt,
                                        const unsigned char *const *keep, int accumulate)
 {
@@ -1625,18 +1647,6 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
     return fail("slicer_deposit_degraded: snopt %d outside 1..30", snopt);
   if (!h->deg.valid || h->deg.nplanes < nplanes)
     return fail("slicer_deposit_degraded: call slicer_count_accepted for this batch and these planes first");
-  if (wait_settled(h, false))
-    return 1;
-  h->fence_all = true;
-  if (!accumulate)
-  {
-    CU(cudaMemsetAsync(h->d_acc, 0, (size_t)nplanes * h->ntypes_alloc * h->npix2max * sizeof(unsigned long long), h->compute));
-    CU(cudaMemsetAsync(h->d_counts, 0, (size_t)nplanes * SLICER_NTYPES * 2 * sizeof(unsigned long long), h->compute));
-    for (int q = 0; q < nplanes; q++)
-      h->slot_epoch[q]++;
-  }
-  if (total == 0)
-    return 0;
   degrade::Dev G;
   memset(&G, 0, sizeof(G));
   size_t need = 0;
@@ -1647,11 +1657,17 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
     if (h->deg.plane_total[q] && (!keep || !keep[q]))
       return fail("slicer_deposit_degraded: keep table of plane %d is missing", q);
   }
+  if (staging_fence(h) || claim_slots(h, 0, nplanes, accumulate != 0))
+    return 1;
+  if (total == 0)
+    return maps_ready(h) || slots_written(h, 0, nplanes, nullptr);
   if (need > h->deg.keep_cap)
   {
     CU(cudaStreamSynchronize(h->compute));
     cudaFree(h->deg.keep);
+    h->device_bytes -= h->deg.keep_cap;
     h->deg.keep = nullptr;
+    h->deg.keep_cap = 0;
     if (dev_alloc(h, &h->deg.keep, need + need / 4 + 4096))
       return 1;
     h->deg.keep_cap = need + need / 4 + 4096;
@@ -1664,27 +1680,8 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
   G.keep = h->deg.keep;
   G.stride = h->deg.stride;
   G.snopt = snopt;
-  size_t base = 0;
-  for (size_t si = 0; si < h->segs.size(); si++)
-  {
-    SegmentDev D;
-    fill_segment(h, h->segs[si], &D);
-    if (D.n)
-    {
-      G.seg_base = base;
-      const size_t want = (D.n + 255) / 256, cap = (size_t)h->sm_count * 16;
-      const int blocks = (int)(want < cap ? want : cap);
-      if (h->cfg.mas == SLICER_MAS_NGP)
-        degrade::degrade_kernel<SLICER_MAS_NGP, degrade::DEPOSIT><<<blocks, 256, 0, h->compute>>>(P, D, G);
-      else
-        degrade::degrade_kernel<SLICER_MAS_TSC, degrade::DEPOSIT><<<blocks, 256, 0, h->compute>>>(P, D, G);
-      CU(cudaGetLastError());
-      h->stats.launches++;
-      h->stats.particles_streamed += D.n;
-    }
-    base += D.n;
-  }
-  CU(cudaEventRecord(h->ev_buf_done[h->cur_buf], h->compute));
+  if (maps_ready(h) || degrade_launch<degrade::DEPOSIT>(h, P, G) || slots_written(h, 0, nplanes, nullptr))
+    return 1;
   CU(cudaStreamSynchronize(h->compute)); // the caller's keep tables may be freed on return
   return 0;
 }
@@ -1944,14 +1941,13 @@ static int reduce_fence_before(slicer_handle *h, int first_slot, int nplanes)
     return 1;
   // after the last pass into each of these slots (not after passes into other slots submitted since) and after the deposits
   // of the pairs libm settled
-  bool all = h->fence_all;
+  bool all = false;
   for (int q = first_slot; q < first_slot + nplanes; q++)
     all = all || !h->slot_pass_ev[q];
   if (all)
   {
     CU(cudaEventRecord(h->ev_pass_done, h->compute));
     CU(cudaStreamWaitEvent(h->comm_stream, h->ev_pass_done, 0));
-    h->fence_all = false;
   }
   else
   {

@@ -171,9 +171,11 @@ def test_driver_resume_skips_existing_planes(tmp_path):
     assert {f: open(out / f, "rb").read() for f in files} == keep  # the missing plane is rebuilt bit for bit, the rest untouched
 
 
-def test_driver_two_gpus_matches_one_gpu(tmp_path):
+@pytest.mark.parametrize("snopt", [0, 1])
+def test_driver_two_gpus_matches_one_gpu(tmp_path, snopt):
     """Sub-files dealt over two GPUs + ncclReduce(int64) of the planes == the single-GPU run, bit for bit
-    (integer accumulators make the sum independent of how the particles are sharded)."""
+    (integer accumulators make the sum independent of how the particles are sharded), also with Part. Degradation: its two
+    sweeps over the sub-files run on both GPUs at once."""
     from slicer_b200 import capi
 
     if capi.device_count() < 2:
@@ -184,7 +186,7 @@ def test_driver_two_gpus_matches_one_gpu(tmp_path):
         out = tmp_path / tag
         out.mkdir()
         ini = tmp_path / f"{tag}.ini"
-        ini.write_text(INI.format(npix=64, zs=0.1, fov=6.0, list=lst, snapdir=snapdir, outdir=str(out) + "/t_", pip=0, snopt=0))
+        ini.write_text(INI.format(npix=64, zs=0.1, fov=6.0, list=lst, snapdir=snapdir, outdir=str(out) + "/t_", pip=0, snopt=snopt))
         r = subprocess.run([host.EXE_PATH, "--quiet", "--gpus", gpus, str(ini)], cwd=tmp_path, capture_output=True, text=True, timeout=900)
         assert r.returncode == 0, r.stderr[-2000:]
         outs[tag] = out

@@ -1,8 +1,8 @@
 """Several light-cone realisations in one run (SLICER_b200 A.ini B.ini ...): one read of every snapshot for all of them.
 
 Driver: every realisation's files are byte-identical to a run of its ini alone (TSC, NGP, perpendicular replication,
-per-type files, physical pixels; more realisations than accumulator slots; resume; two GPUs); mismatched inis are refused
-before anything is written (CPU).  Library: accumulator slots above 16 per handle, three slot ranges deposited interleaved
+per-type files, physical pixels; more realisations than accumulator slots; resume; two GPUs; a degrading ini among normal
+ones); mismatched inis are refused before anything is written (CPU).  Library: accumulator slots above 16 per handle, three slot ranges deposited interleaved
 with the rounding guard's libm path busy, and eight randomisations from different seed triples in one dense pass, all
 against the oracle bit for bit."""
 import itertools
@@ -184,6 +184,30 @@ def test_two_gpus_match_one_gpu(tmp_path):
         assert r.returncode == 0, r.stderr[-3000:]
         outs[tag] = tree(tmp_path / tag)
     assert len(outs["g1"]) >= 3 * 8 and outs["g1"] == outs["g2"]
+
+
+@pytest.mark.gpu
+def test_a_degrading_ini_among_normal_ones(tmp_path):
+    """Part. Degradation = 1 in the second of three inis (4 snapshots of 3 sub-files): the degrading light cone takes its own two
+    sweeps over each snapshot after the shared passes of the others, and every file is still the bytes of each ini's own run."""
+    snapdir, lst = make_dataset(tmp_path, nsnap=4, numfiles=3)
+
+    def inis(tag):
+        out = realisation_inis(tmp_path, tag, lst, snapdir, 3)
+        out[1].write_text(out[1].read_text().replace("Part. Degradation ####\n0\n", "Part. Degradation ####\n1\n"))
+        return out
+
+    r = run_exe(inis("together"), tmp_path, quiet=False)
+    assert r.returncode == 0, r.stderr[-3000:]
+    reads = [line for line in r.stdout.splitlines() if line.startswith(" sub-file ")]
+    degraded = [line for line in reads if line.endswith(" (degradation 2^-1)")]
+    assert degraded and 2 * len(degraded) == len(reads)  # sweep 2 logs each sub-file the shared passes log; sweep 1 is silent
+    for ini in inis("alone"):
+        r = run_exe([ini], tmp_path)
+        assert r.returncode == 0, r.stderr[-3000:]
+    a, b = tree(tmp_path / "together"), tree(tmp_path / "alone")
+    assert sorted(a) == sorted(b) and sum(f.endswith("_r1.fits") for f in a) >= 8
+    assert all(a[f] == b[f] for f in a), [f for f in a if a[f] != b[f]]
 
 
 # ---- library: slots above 16, interleaved sets, eight randomisations --------------------------------------------------------
