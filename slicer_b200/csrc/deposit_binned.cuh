@@ -27,18 +27,12 @@
 namespace binned
 {
 
-#ifndef SLICER_TILE
-#define SLICER_TILE 166
-#endif
-#ifndef SLICER_TILE_CTAS
-#define SLICER_TILE_CTAS 1
-#endif
-constexpr int TILE = SLICER_TILE;  // interior cells per tile side (166: one 1024-thread CTA per SM owns 226 KB; 116: two CTAs)
+constexpr int TILE = 166;          // interior cells per tile side: one 1024-thread CTA per SM owns 226 KB
 constexpr int TW = TILE + 2;       // + 1-cell halo for the 3x3 stencil
 constexpr int TCELLS = TW * TW;    // 28,224 cells x 8 B = 225,792 B of shared memory
 constexpr int MAX_BINS = 5120; // bins per sort window: 3 tables of MAX_BINS words + the 16K-record batch fill the scatter kernel's shared memory
 constexpr int SCATTER_THREADS = 1024;
-constexpr int DEPOSIT_THREADS = 1024 / SLICER_TILE_CTAS;
+constexpr int DEPOSIT_THREADS = 1024;
 
 struct EmitDev
 {
@@ -512,7 +506,7 @@ __device__ __forceinline__ void tile_tsc(unsigned *lo, unsigned *hi, int x0, int
 
 // K3: one CTA per (plane, tile) bin
 template <int MAS>
-__global__ void __launch_bounds__(DEPOSIT_THREADS, SLICER_TILE_CTAS)
+__global__ void __launch_bounds__(DEPOSIT_THREADS, 1)
     tile_deposit_kernel(const __grid_constant__ PassParams P, const __grid_constant__ SortDev D, int ntile, int ntx, int gshift, int type,
                         float const_mass)
 {

@@ -37,7 +37,7 @@
 // Per-pass constants of the lean projection (uniform over the pass: every plane shares field and map size).
 struct LeanDev
 {
-  int enabled;   // the pass qualifies (PassParams::pair) and the box is in the fast transform's range
+  int enabled;   // the pass qualifies (slicer_capi.cu: build_pass) and the box is in the fast transform's range
   int K;         // series terms beyond the linear one: asin(s) ~ s + s^3 (a_1 + a_2 s^2 + ... + a_K s^(2K-2))
   double A;      // 1 / fovradiants
   double w_in;   // |w| <= w_in   => inside the field for sure        (T/fov - ETA)

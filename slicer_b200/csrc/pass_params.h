@@ -85,10 +85,7 @@ struct PassParams
   int nxform;
   int nplanes;
   int fast;  // every plane: npix a power of two, no perpendicular replication, disjoint slabs per randomisation
-  int pair;  // fast, and all planes share one field (T, fovrad) with a small-angle series: two survivors per lane
-  double est_accept; // host estimate of the accepted fraction of a uniform snapshot (chooses the deposit path)
-  int debug; // measurement aid (env SLICER_B200_DEBUG): bit0 skip the map atomics, bit1 skip the exact chain; 0 in production
-  LeanDev lean; // lean projection + ambiguity guard (lean_math.h); enabled for `pair` passes
+  LeanDev lean; // lean projection + ambiguity guard (lean_math.h); enabled for fast passes whose planes share one narrow field
   XformDev xf[SLICER_MAX_XFORMS];
   PlaneDev pl[SLICER_MAX_PLANES];
 };

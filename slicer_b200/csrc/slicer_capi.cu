@@ -132,9 +132,6 @@ struct slicer_handle
   std::vector<cudaEvent_t> pass_ev;                // ring of (start, stop) pairs, resolved lazily
   size_t pass_head = 0, pass_tail = 0;             // pairs [tail, head) are pending
   int nbuf = 1, cur_buf = 0;
-  int debug = 0;
-  bool no_series = false; // env SLICER_B200_NO_SERIES: always use libdevice asin/atan2 (A/B checks)
-  bool no_lean = false;   // env SLICER_B200_NO_LEAN: general exact chain instead of the lean projection + guard (A/B checks)
   float *d_pos_pool = nullptr;  // nbuf * (particle_capacity * 3 + 64) floats
   float *d_mass_pool = nullptr; // nbuf * (mass_capacity + 64) floats
   float *d_pos = nullptr;  // current pool
@@ -155,7 +152,7 @@ struct slicer_handle
   size_t device_bytes = 0;
   ncclComm_t comm = nullptr;
   int nranks = 1, rank = 0;
-  PipelinedScratch pipe;
+  int grid_max = 0; // CTAs of a persistent pipelined-kernel grid (pipelined_init)
   // lean exact phase: particles it could not decide (lean_math.h), settled with the host's libm by resolve_deferred()
   struct SavedPass
   {
@@ -308,10 +305,6 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
   if (h->cfg.max_m <= 0)
     h->cfg.max_m = 1e3; /* densitymaps.h:21 */
   h->ntypes_alloc = cfg->per_type_maps ? SLICER_NTYPES : 1;
-  h->no_series = getenv("SLICER_B200_NO_SERIES") != nullptr;
-  h->no_lean = getenv("SLICER_B200_NO_LEAN") != nullptr;
-  if (const char *dbg = getenv("SLICER_B200_DEBUG"))
-    h->debug = atoi(dbg);
   h->npix2max = (size_t)cfg->npix_max * (size_t)cfg->npix_max;
   memset(&h->stats, 0, sizeof(h->stats));
   memset(h->plane_npix, 0, sizeof(h->plane_npix));
@@ -421,7 +414,7 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
     if ((rc = dev_alloc(h, &h->d_sum, h->npix2max)))
       break;
     t_alloc = now();
-    if ((rc = pipelined_init(&h->pipe, h->sm_count)))
+    if ((rc = pipelined_init(h->sm_count, &h->grid_max)))
     {
       rc = fail("pipelined kernel set-up failed: %s", cudaGetErrorString(cudaGetLastError()));
       break;
@@ -462,7 +455,6 @@ extern "C" void slicer_destroy(slicer_handle *h)
     cudaStreamSynchronize(h->comm_stream);
   if (h->comm && g_nccl.CommDestroy)
     g_nccl.CommDestroy(h->comm);
-  pipelined_destroy(&h->pipe);
   cudaFree(h->deg.cnt);
   cudaFree(h->deg.keep);
   cudaFree(h->deg.rank);
@@ -743,8 +735,10 @@ static float float_floor(double d)
 }
 static bool is_f32(double d) { return (double)(float)d == d; }
 
-// planes[i] deposits into accumulator slot first_slot + i
-static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, PassParams *P, int first_slot = 0)
+// planes[i] deposits into accumulator slot first_slot + i.  *est_accept: the fraction of a uniform snapshot the pass accepts
+// (use_binned)
+static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, PassParams *P, int first_slot = 0,
+                      double *est_accept = nullptr)
 {
   if (nplanes < 1 || nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: nplanes %d outside 1..%d (max_planes)", nplanes, h->cfg.max_planes);
@@ -790,10 +784,8 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
   }
   P->nxform = nx;
   P->nplanes = nplanes;
-  P->debug = h->debug;
   P->fast = 1;
-  P->est_accept = 0;
-  P->pair = 0;
+  double accept = 0;
   static const int perm_of_face[7][3] = {{0, 1, 2}, {0, 1, 2}, {0, 2, 1}, {1, 2, 0}, {1, 0, 2}, {2, 0, 1}, {2, 1, 0}}; /* gadget2io.cpp:223-252 */
   int slot = 0;
   for (int t = 0; t < nx; t++)
@@ -862,7 +854,7 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
       L.arg_lim = 0;
       L.guard_eta = h->cfg.guard_eta >= LEAN_ETA ? h->cfg.guard_eta : LEAN_ETA;
       L.guard_T = 2.0 * L.guard_eta * L.T; // an angle is (map coordinate - 0.5) * fov: the same guard, in radians
-      if (!h->no_series && isfinite(L.pre_tx) && (double)L.pre_tx * 1.01 <= 0.385)
+      if (isfinite(L.pre_tx) && (double)L.pre_tx * 1.01 <= 0.385)
       {
         L.arg_lim = (double)L.pre_tx * 1.01;
         L.nt = (int)ceil(55.0 * log(2.0) / (2.0 * log(1.0 / L.arg_lim)));
@@ -880,7 +872,7 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
       {
         // fraction of a uniform snapshot this plane accepts: slab thickness x (field width / box)^2 at mid-distance
         const double w = L.T < 1.5 ? 2.0 * tan(L.T) * 0.5 * (minDist + maxDist) : 1.0;
-        P->est_accept += (maxDist - minDist) * (w < 1.0 ? w * w : 1.0);
+        accept += (maxDist - minDist) * (w < 1.0 ? w * w : 1.0);
       }
     }
     for (int a = X.first_plane; a < X.first_plane + X.nplanes; a++)
@@ -913,17 +905,18 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
     for (int k = 0; k < 3; k++)
       X.wadd[k] = X.sgn[k] < 0.f ? 1.f : 0.f;
   }
-  P->pair = P->fast && P->pl[0].nt > 0;
+  // lean exact phase (lean_math.h, deposit_pipelined.cuh: drain_lean): a fast pass with one narrow field (small-angle series) and
+  // map size for all planes, float-exact box and centres, and a box size for which the unchecked float division cannot leave the
+  // normal range
+  bool lean = P->fast && P->pl[0].nt > 0 && h->boxsize >= 0x1p-40 && h->boxsize <= 0x1p40;
   for (int t = 0; t < P->nxform; t++)
     if (!P->xf[t].exact_f32)
-      P->pair = 0; // the lean exact phase assumes a float-exact box and centre
+      lean = false;
   for (int q = 1; q < P->nplanes; q++)
     if (P->pl[q].T != P->pl[0].T || P->pl[q].fovrad != P->pl[0].fovrad || P->pl[q].npix != P->pl[0].npix)
-      P->pair = 0;
-  // lean exact phase (lean_math.h, deposit_pipelined.cuh: drain_lean): one narrow field and map size for all planes, float-exact
-  // box and centres, and a box size for which the unchecked float division cannot leave the normal range
+      lean = false;
   P->lean.enabled = 0;
-  if (P->pair && h->boxsize >= 0x1p-40 && h->boxsize <= 0x1p40 && !h->no_lean)
+  if (lean)
   {
     lean_setup(&P->lean, P->pl[0].fovrad, P->pl[0].T, h->cfg.guard_eta);
     if (!(P->xf[0].raw_hi > P->lean.umin))
@@ -933,6 +926,8 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
         if (!(P->xf[t].cf[k] >= 0.f && P->xf[t].cf[k] <= 1.f))
           P->lean.enabled = 0; // lean_axis assumes a centre inside the box (randomizeBox draws it in [0, 1])
   }
+  if (est_accept)
+    *est_accept = accept;
   return 0;
 }
 
@@ -966,7 +961,7 @@ static int binned_gshift(const PassParams &P)
 // 0: direct map atomics; 1: binned.  When the planes' tiles exceed MAX_BINS even in groups of four (8192^2 maps from 8 planes
 // up, 16384^2 from 3) the records are still produced once; the sort and the tile deposit then run window by window over the
 // bins (binned_pass).
-static int use_binned(const slicer_handle *h, const PassParams &P, const SegmentDev &D)
+static int use_binned(const slicer_handle *h, const PassParams &P, double est_accept, const SegmentDev &D)
 {
   if (!P.fast || h->cfg.deposit_mode == SLICER_DEPOSIT_DIRECT)
     return 0;
@@ -980,12 +975,12 @@ static int use_binned(const slicer_handle *h, const PassParams &P, const Segment
     return 1;
   // the sort + tile kernels cost ~65 us per segment before the first record; a record then costs ~50 ps against ~105 ps of
   // direct atomics (measured on 2^24- and 2^27-particle segments): worth it from ~1.2 million expected records
-  if (P.est_accept * (double)D.n < 1.2e6)
+  if (est_accept * (double)D.n < 1.2e6)
     return 0;
   // measured break-even (DESIGN.md §5): 3 % of the snapshot accepted; 1.5 % when one slice holds the whole batch, or when
   // the planes' accumulators are several times the L2 (> 256 MiB, e.g. 4096^2 and 8192^2 maps: the direct path's atomics go to HBM)
   const bool big_maps = (size_t)P.nplanes * P.pl[0].npix * P.pl[0].npix * sizeof(unsigned long long) > ((size_t)256 << 20);
-  return P.est_accept > (h->bin_slice_hint() >= D.n || big_maps ? 0.015 : 0.03) ? 1 : 0;
+  return est_accept > (h->bin_slice_hint() >= D.n || big_maps ? 0.015 : 0.03) ? 1 : 0;
 }
 
 static int binned_alloc(slicer_handle *h, bool need_mass)
@@ -1005,13 +1000,13 @@ static int binned_alloc(slicer_handle *h, bool need_mass)
     slice = cap_particles;
   slice = (slice + pipe::CHUNK - 1) / pipe::CHUNK * pipe::CHUNK;
   // every CTA region is rounded up to whole chunks, times the randomisations of a pass (one record per particle and randomisation)
-  const size_t cap = slice + ((size_t)h->pipe.grid_max + 1) * pipe::CHUNK * SLICER_MAX_XFORMS;
+  const size_t cap = slice + ((size_t)h->grid_max + 1) * pipe::CHUNK * SLICER_MAX_XFORMS;
   if (dev_alloc(h, &h->bin.rec_u, cap) || dev_alloc(h, &h->bin.rec_s, cap) || dev_alloc(h, &h->bin.key_u, cap))
     return 1;
   if ((h->cfg.mass_capacity || need_mass) && (dev_alloc(h, &h->bin.mass_u, cap) || dev_alloc(h, &h->bin.mass_s, cap)))
     return 1;
-  if (dev_alloc(h, &h->bin.region_count, (size_t)h->pipe.grid_max) ||
-      dev_alloc(h, &h->bin.region_hist, (size_t)binned::MAX_BINS * h->pipe.grid_max) ||
+  if (dev_alloc(h, &h->bin.region_count, (size_t)h->grid_max) ||
+      dev_alloc(h, &h->bin.region_hist, (size_t)binned::MAX_BINS * h->grid_max) ||
       dev_alloc(h, &h->bin.bin_count, (size_t)binned::MAX_BINS) || dev_alloc(h, &h->bin.bin_start, (size_t)binned::MAX_BINS + 1))
     return 1;
   h->bin.slice = slice;
@@ -1054,7 +1049,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     S.n = D.n - off < slice ? D.n - off : slice;
     S.pos = D.layout == SLICER_LAYOUT_AOS ? D.pos + 3ull * off : D.pos + off;
     S.mass = D.mass ? D.mass + off : nullptr;
-    const int grid = pipelined_grid(&h->pipe, S.n);
+    const int grid = pipelined_grid(h->grid_max, S.n);
     const unsigned long long nchunks = (S.n + pipe::CHUNK - 1) / pipe::CHUNK;
     const unsigned long long cmax = (nchunks + grid - 1) / grid;
     binned::EmitDev E;
@@ -1089,7 +1084,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     Q.rec_s = h->bin.rec_s;
     Q.mass_s = D.mass ? h->bin.mass_s : nullptr;
     Q.capacity = h->bin.capacity;
-    if (pipelined_launch_emit(grid, P, S, E, F, h->compute))
+    if (pipelined_launch(grid, h->cfg.mas, true, P, S, E, F, h->compute))
       return fail("record kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     const int nwin = (nbins + binned::MAX_BINS - 1) / binned::MAX_BINS;
     const int wbins = (nbins + nwin - 1) / nwin;
@@ -1104,13 +1099,10 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
       binned::launch_bin_scatter(Q, nwin > 1, h->compute);
       if (maps_ready(h))
         return 1;
-      if (!(h->debug & 4)) // measurement aid: SLICER_B200_DEBUG bit 2 skips the tile deposit
-      {
-        if (h->cfg.mas == SLICER_MAS_NGP)
-          binned::tile_deposit_kernel<SLICER_MAS_NGP><<<Q.nbins << gshift, binned::DEPOSIT_THREADS, binned::TCELLS * 8, h->compute>>>(P, Q, nt, ntx, gshift, D.type, D.const_mass);
-        else
-          binned::tile_deposit_kernel<SLICER_MAS_TSC><<<Q.nbins << gshift, binned::DEPOSIT_THREADS, binned::TCELLS * 8, h->compute>>>(P, Q, nt, ntx, gshift, D.type, D.const_mass);
-      }
+      if (h->cfg.mas == SLICER_MAS_NGP)
+        binned::tile_deposit_kernel<SLICER_MAS_NGP><<<Q.nbins << gshift, binned::DEPOSIT_THREADS, binned::TCELLS * 8, h->compute>>>(P, Q, nt, ntx, gshift, D.type, D.const_mass);
+      else
+        binned::tile_deposit_kernel<SLICER_MAS_TSC><<<Q.nbins << gshift, binned::DEPOSIT_THREADS, binned::TCELLS * 8, h->compute>>>(P, Q, nt, ntx, gshift, D.type, D.const_mass);
       h->stats.launches += k1_hist ? 3 : 4;
     }
     CU(cudaGetLastError());
@@ -1159,8 +1151,6 @@ __global__ void resolved_deposit_kernel(const __grid_constant__ PassParams P, co
   const ResolvedRec e = r[i];
   const PlaneDev &L = P.pl[e.plane];
   atomicAdd(L.counts + 2 * e.type, 1ull);
-  if (P.debug & 1)
-    return;
   if (chain::deposit<MAS>(e.xs, e.ys, e.m, L, L.acc + L.type_stride * (unsigned long long)e.type))
     atomicAdd(L.counts + 2 * e.type + 1, 1ull);
 }
@@ -1379,7 +1369,8 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
   if (first_slot < 0 || nplanes < 1 || first_slot + nplanes > h->cfg.max_planes)
     return fail("slicer_deposit: slots %d..%d outside 0..%d (max_planes)", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
   PassParams P;
-  if (build_pass(h, planes, nplanes, &P, first_slot) || staging_fence(h))
+  double est_accept = 0;
+  if (build_pass(h, planes, nplanes, &P, first_slot, &est_accept) || staging_fence(h))
     return 1;
   // A new set of planes takes the other bank when that bank is settled (a caller that alternates between two slot ranges and
   // settles or reduces one range behind the next pass finds it so every time), or when it zeroes slots the current bank holds
@@ -1437,13 +1428,13 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
       return fail("slicer_deposit: a segment with per-particle masses holds %llu particles; stage it in batches of fewer than 2^32", D.n);
     if (kernel == SLICER_KERNEL_PIPELINED)
     {
-      const int ub = use_binned(h, P, D);
+      const int ub = use_binned(h, P, est_accept, D);
       if (ub == 1)
       {
         if (binned_pass(h, P, D, F))
           return 1;
       }
-      else if (maps_ready(h) || pipelined_launch(&h->pipe, h->cfg.mas, P, D, F, h->compute))
+      else if (maps_ready(h) || pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F, h->compute))
         return fail("pipelined launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
     else

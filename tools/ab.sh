@@ -1,7 +1,7 @@
 #!/bin/bash
 # measurement aid: A/B two builds of the CUDA library in ONE gpurun call (same box, same clocks).
 #   tools/ab.sh "<nvcc flags of A>" "<nvcc flags of B>" [PGROUPS, default 0,2,4,8]
-# e.g. tools/ab.sh "" "-DSLICER_MIN_CTAS=2"      (A = the default build)
+# e.g. tools/ab.sh "" "-DSLICER_CHECKS"      (A = the default build, B = the build with device-side bounds checks)
 # Builds slicer_b200/_build/libslicer_b200_{a,b}.so here, then runs tools/probe_groups.py twice per variant on the GPU box.
 set -e
 HERE="$(cd "$(dirname "$0")/.." && pwd)"
