@@ -89,7 +89,7 @@ EXPORTS = [
     "slicer_frac_bits", "slicer_comm_unique_id", "slicer_comm_init_rank", "slicer_comm_init_all",
     "slicer_reduce_all", "slicer_wait_staging", "slicer_count_accepted", "slicer_deposit_degraded", "slicer_reset_stats", "slicer_timer_begin", "slicer_timer_end",
     "slicer_selftest_arith", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
-    "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory",
+    "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory", "slicer_comm_init_ranks",
 ]
 
 
@@ -150,6 +150,7 @@ def lib() -> C.CDLL:
     L.slicer_comm_unique_id.argtypes = [C.c_char_p]
     L.slicer_comm_init_rank.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int]
     L.slicer_comm_init_all.argtypes = [C.POINTER(C.c_void_p), C.c_int]
+    L.slicer_comm_init_ranks.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_char_p, C.c_int, C.c_int]
     L.slicer_reduce_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int]
     _lib = L
     return L

@@ -60,6 +60,7 @@ struct NcclApi
   ncclResult_t (*GroupStart)() = nullptr;
   ncclResult_t (*GroupEnd)() = nullptr;
   ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
+  ncclResult_t (*CommAbort)(ncclComm_t) = nullptr;
   const char *(*GetErrorString)(ncclResult_t) = nullptr;
 };
 static NcclApi g_nccl;
@@ -84,6 +85,7 @@ static int load_nccl()
   SYM(GroupStart, "ncclGroupStart");
   SYM(GroupEnd, "ncclGroupEnd");
   SYM(CommDestroy, "ncclCommDestroy");
+  SYM(CommAbort, "ncclCommAbort");
   SYM(GetErrorString, "ncclGetErrorString");
 #undef SYM
   return 0;
@@ -1883,6 +1885,50 @@ extern "C" int slicer_comm_init_rank(slicer_handle *h, const char id[128], int n
   return 0;
 }
 
+extern "C" int slicer_comm_init_ranks(slicer_handle **handles, int n, const char id[128], int nranks, int first_rank)
+{
+  if (!handles || n < 1 || first_rank < 0 || first_rank + n > nranks)
+    return fail("slicer_comm_init_ranks: bad arguments (%d handles as ranks %d.. of %d)", n, first_rank, nranks);
+  if (load_nccl())
+    return 1;
+  for (int i = 0; i < n; i++)
+    if (!handles[i] || handles[i]->comm)
+      return fail("slicer_comm_init_ranks: handle %d null or already in a communicator", i);
+  ncclUniqueId u;
+  memcpy(&u, id, 128);
+  std::vector<ncclComm_t> comms(n, nullptr);
+  NC(g_nccl.GroupStart());
+  int rc = 0;
+  for (int i = 0; i < n && !rc; i++)
+  {
+    if (cudaSetDevice(handles[i]->cfg.device) != cudaSuccess)
+      rc = fail("cudaSetDevice failed");
+    else
+    {
+      const ncclResult_t r = g_nccl.CommInitRank(&comms[i], nranks, u, first_rank + i);
+      if (r != ncclSuccess)
+        rc = fail("ncclCommInitRank failed: %s", g_nccl.GetErrorString(r));
+    }
+  }
+  const ncclResult_t ge = g_nccl.GroupEnd(); // always closes the group
+  if (!rc && ge != ncclSuccess)
+    rc = fail("ncclGroupEnd failed: %s", g_nccl.GetErrorString(ge));
+  if (rc)
+  { // the communicators made before the failure never reach a handle: free them here
+    for (int i = 0; i < n; i++)
+      if (comms[i] && cudaSetDevice(handles[i]->cfg.device) == cudaSuccess)
+        g_nccl.CommAbort(comms[i]);
+    return rc;
+  }
+  for (int i = 0; i < n; i++)
+  {
+    handles[i]->comm = comms[i];
+    handles[i]->nranks = nranks;
+    handles[i]->rank = first_rank + i;
+  }
+  return 0;
+}
+
 extern "C" int slicer_comm_init_all(slicer_handle **handles, int n)
 {
   if (!handles || n < 1)
@@ -1999,10 +2045,14 @@ extern "C" int slicer_reduce_all_slots(slicer_handle **handles, int n, int first
     if (set_device(handles[i]) || resolve_deferred(handles[i], first_slot, nplanes))
       return 1;
   }
-  if (n == 1)
+  // the communicator's size, not the handles of this process: one handle may be one rank of a communicator over several processes
+  if (handles[0]->nranks == 1 && n == 1)
     return 0;
   if (load_nccl())
     return 1;
+  for (int i = 0; i < n; i++)
+    if (!handles[i]->comm)
+      return fail("slicer_reduce_all: handle %d has no communicator", i);
   for (int i = 0; i < n; i++)
     if (set_device(handles[i]) || reduce_fence_before(handles[i], first_slot, nplanes))
       return 1;

@@ -31,7 +31,17 @@ def lib():
         L.shost_write_fits.argtypes = [C.c_char_p, _f32p, C.c_int, C.c_int, C.POINTER(C.c_char_p), _f64p, C.c_int, C.POINTER(C.c_char_p),
                                        np.ctypeslib.ndpointer(dtype=np.int64, flags="C_CONTIGUOUS")]
         L.shost_run_light_cone.argtypes = [C.c_char_p, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
-        L.shost_run_light_cones.argtypes = [C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
+        L.shost_run_light_cones.argtypes = [C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                            C.c_int, C.c_char_p, C.c_int]
+        L.shost_launch_from_env.argtypes = [C.POINTER(C.c_char_p), C.c_int, C.c_int, _i32p, C.c_char_p, C.c_int, C.c_char_p, C.c_int]
+        L.shost_subfile_owners.argtypes = [C.c_int, _i32p, C.c_uint, C.c_uint, _i32p, _i32p]
+        L.shost_group_open.restype = C.c_void_p
+        L.shost_group_open.argtypes = [C.c_int, C.c_int, C.c_char_p, C.c_int, C.c_double, C.POINTER(C.c_int)]
+        L.shost_group_close.argtypes = [C.c_void_p]
+        L.shost_group_bcast.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_longlong), C.c_longlong]
+        L.shost_group_allgather.argtypes = [C.c_void_p, C.c_char_p, C.c_longlong, C.c_char_p, C.POINTER(C.c_longlong), C.c_longlong]
+        L.shost_group_allreduce.argtypes = [C.c_void_p, C.POINTER(C.c_longlong), C.c_int, C.c_int]
+        L.shost_group_agree.argtypes = [C.c_void_p, C.c_int]
         _lib = L
     return _lib
 
@@ -113,14 +123,84 @@ def run_light_cone(ini, devices=(0,), replication=False, fixed_vertex=False, ngp
     return lib().shost_run_light_cone(ini.encode(), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode))
 
 
-def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0, max_slots=0):
+def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0, max_slots=0, rank=0, nranks=1,
+                    master=None):
     """One light cone per ini (realisations of one plan: other seeds, other outputs), every snapshot read once for all (once per
     group of planes that fits `max_slots` accumulators per GPU, when given).  Returns 0 on success; inis that disagree on the
-    plan are refused before anything is written."""
+    plan are refused before anything is written.
+    rank / nranks / master ("host:port", where rank 0 listens): this process is one rank of a job of `nranks` processes that
+    all make this call with the same arguments but `rank` and `devices`; rank 0 writes the files.  The launcher's environment
+    is not read."""
     dev = np.ascontiguousarray(devices, np.int32)
     arr = (C.c_char_p * len(inis))(*[str(i).encode() for i in inis])
+    addr, port = (master.rsplit(":", 1) if master else ("", 0))
     return lib().shost_run_light_cones(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
-                                       int(max_slots))
+                                       int(max_slots), int(rank), int(nranks), addr.encode(), int(port))
+
+
+def launch_from_env(env, ndev=1):
+    """What SLICER_b200 makes of a launcher's environment `env` (a dict): rank, world size, local rank, meeting point and default
+    GPU among `ndev`.  Raises ValueError with the driver's message when it would refuse to start."""
+    kv = [f"{k}={v}".encode() for k, v in env.items()]
+    arr = (C.c_char_p * max(1, len(kv)))(*kv)
+    out = np.zeros(5, np.int32)
+    addr, err = C.create_string_buffer(256), C.create_string_buffer(1024)
+    if lib().shost_launch_from_env(arr, len(kv), ndev, out, addr, 256, err, 1024):
+        raise ValueError(err.value.decode())
+    return dict(rank=int(out[0]), nranks=int(out[1]), local_rank=int(out[2]), master_addr=addr.value.decode(), master_port=int(out[3]),
+                device=int(out[4]))
+
+
+def subfile_owners(ngpus, ffmin, ffmax):
+    """The job's sub-file assignment for ranks that drive ngpus[r] GPUs: -> (rank, local GPU) of each of ffmin .. ffmax-1."""
+    ng = np.ascontiguousarray(ngpus, np.int32)
+    rank_of, gpu_of = np.zeros(ffmax - ffmin, np.int32), np.zeros(ffmax - ffmin, np.int32)
+    if lib().shost_subfile_owners(len(ng), ng, ffmin, ffmax, rank_of, gpu_of):
+        raise RuntimeError("a sub-file has two owners")
+    return list(zip(rank_of.tolist(), gpu_of.tolist()))
+
+
+class Group:
+    """The driver's control channel between the processes of a job (tests): rank 0 listens on addr:port."""
+
+    OPS = {"min": 0, "max": 1, "sum": 2}
+
+    def __init__(self, rank, nranks, addr, port, timeout_s=60.0):
+        rc = C.c_int()
+        self.g = lib().shost_group_open(rank, nranks, addr.encode(), port, timeout_s, C.byref(rc))
+        self.ok = rc.value == 0
+
+    def close(self):
+        if self.g:
+            lib().shost_group_close(self.g)
+            self.g = None
+
+    def bcast(self, blob=b"", cap=1 << 20):
+        buf = C.create_string_buffer(blob, max(cap, len(blob)))
+        n = C.c_longlong(len(blob))
+        if lib().shost_group_bcast(self.g, buf, C.byref(n), cap):
+            raise RuntimeError("bcast failed")
+        return buf.raw[: n.value]
+
+    def allgather(self, blob, nranks, cap=1 << 20):
+        out = C.create_string_buffer(cap)
+        lens = (C.c_longlong * nranks)()
+        if lib().shost_group_allgather(self.g, blob, len(blob), out, lens, cap):
+            raise RuntimeError("allgather failed")
+        res, off = [], 0
+        for n in lens:
+            res.append(out.raw[off: off + n])
+            off += n
+        return res
+
+    def allreduce(self, values, op):
+        v = (C.c_longlong * len(values))(*values)
+        if lib().shost_group_allreduce(self.g, v, len(values), self.OPS[op]):
+            raise RuntimeError("allreduce failed")
+        return list(v)
+
+    def agree(self, status=0):
+        return lib().shost_group_agree(self.g, status)
 
 
 def read_fits(path):

@@ -1,8 +1,9 @@
 // driver.cpp — createDensityMaps on the GPU and the plane driver of main() (slicer-v2.cpp:130-230), restructured:
 // the reference walks the PLANES and re-reads + re-transforms a whole snapshot for each one (:138-207); here the
 // loop is over SNAPSHOTS, every sub-file is read once into page-locked memory, copied once, and one CUDA pass
-// deposits it into all the planes that use the snapshot.  Sub-files are dealt round-robin to the GPUs of the box
-// (the reference deals them to MPI ranks, :162-175) and the planes are summed with ncclReduce instead of MPI_Reduce.
+// deposits it into all the planes that use the snapshot.  Sub-files are dealt round-robin to the GPUs of the job — one
+// process or several (the reference deals them to MPI ranks, :162-175) — and the planes are summed with ncclReduce instead of
+// MPI_Reduce.
 #include "slicer_host.h"
 
 #include <atomic>
@@ -38,6 +39,11 @@ struct Engine
   // > 0: the slots are sized to free device memory each time the handles are made, want_slots at most, need_slots at least
   int want_slots = 0, need_slots = 0;
   bool comm = false;
+  // the job's processes: this rank's GPUs are the job's GPUs gpu0 .. gpu0 + devices.size() - 1 of G.  Without a group of more than
+  // one rank, gpu0 = 0 and G = devices.size()
+  Group *group = nullptr;
+  int gpu0 = 0, G = 1;
+  bool multi() const { return group && group->size() > 1; }
 };
 
 // device time of the passes the handles ran (summed over the GPUs), before they are destroyed: SLICER_B200_TIMING only
@@ -85,6 +91,12 @@ static int choose_slots(const std::vector<int> &devices, int want, int need, int
   return 0;
 }
 
+static int fail_capi(const char *what)
+{
+  std::cerr << what << ": " << slicer_last_error() << std::endl;
+  return 1;
+}
+
 static int make_handles(Engine *e)
 {
   add_gpu_time(e);
@@ -94,6 +106,13 @@ static int make_handles(Engine *e)
   e->comm = false;
   if (e->want_slots > 0 && choose_slots(e->devices, e->want_slots, e->need_slots, e->npix_max, e->per_type, e->capacity, e->max_planes))
     return 1;
+  if (e->multi())
+  { // every rank allocates the same slots: the passes, and so the reduces, are planned from them
+    std::vector<long long> s = {e->max_planes};
+    if (e->group->allreduce(s, Group::Op::Min))
+      return 1;
+    e->max_planes = (int)s[0];
+  }
   // one thread per GPU: creating a CUDA context, loading the kernels and allocating the pools takes ~2 s per device, serially
   // that was most of an 8-GPU run's wall clock
   std::vector<std::string> errs(e->devices.size());
@@ -124,15 +143,30 @@ static int make_handles(Engine *e)
     for (auto &t : th)
       t.join();
   }
+  int failed = 0;
   for (size_t g = 0; g < e->devices.size(); g++)
     if (!e->h[g])
     {
       std::cerr << "slicer_create failed on GPU " << e->devices[g] << ": " << errs[g] << std::endl;
-      return 1;
+      failed = 1;
     }
-  if (e->h.size() > 1)
+  if (e->multi() ? e->group->agree(failed) : failed) // (no rank may enter the communicator's set-up while another cannot)
+    return 1;
+  if (e->G > 1)
   {
-    if (slicer_comm_init_all(e->h.data(), (int)e->h.size()))
+    int rc = 0;
+    if (!e->multi())
+      rc = slicer_comm_init_all(e->h.data(), (int)e->h.size());
+    else
+    { // rank 0 makes the id; it is handed out again whenever the handles are rebuilt
+      std::string id(128, '\0');
+      if (e->group->rank() == 0 && slicer_comm_unique_id(&id[0]))
+        return fail_capi("slicer_comm_unique_id");
+      if (e->group->bcast(id))
+        return 1;
+      rc = slicer_comm_init_ranks(e->h.data(), (int)e->h.size(), id.data(), e->G, e->gpu0);
+    }
+    if (rc)
     {
       std::cerr << "NCCL communicator: " << slicer_last_error() << std::endl;
       return 1;
@@ -143,10 +177,13 @@ static int make_handles(Engine *e)
 }
 
 static Engine *engine_new(const std::vector<int> &devices, int npix_max, int mas, bool per_type_maps, size_t particle_capacity, int deposit_mode,
-                          int max_planes, int want_slots, int need_slots)
+                          int max_planes, int want_slots, int need_slots, Group *group = nullptr, int gpu0 = 0, int G = 0)
 {
   Engine *e = new Engine;
   e->devices = devices;
+  e->group = group;
+  e->gpu0 = gpu0;
+  e->G = G > 0 ? G : (int)devices.size();
   e->max_planes = std::min(std::max(max_planes, 1), (int)SLICER_MAX_SLOTS);
   e->want_slots = want_slots;
   e->need_slots = need_slots;
@@ -201,12 +238,6 @@ static slicer_plane_desc make_desc(const Lens &lens, const Random &random, int i
   d.fovradiants = fovradiants;
   d.npix = npix;
   return d;
-}
-
-static int fail_capi(const char *what)
-{
-  std::cerr << what << ": " << slicer_last_error() << std::endl;
-  return 1;
 }
 
 // Stage every particle type of a sub-file that is already in `buf` (types in order: the order mapParticles walks them).
@@ -315,9 +346,10 @@ static int deposit_passes(slicer_handle *h, const std::vector<slicer_plane_desc>
   return 0;
 }
 
-// Stages sub-files [ffmin, ffmax) of File and calls action(g, ff) behind each, with one host thread per GPU (the reference: one
-// MPI rank per group of sub-files, slicer-v2.cpp:162-175, densitymaps.cpp:432-484).  GPU g takes sub-files ffmin + g,
-// ffmin + g + ngpu, ...; it reads sub-file k+1 into its second page-locked buffer while the copy and the work on sub-file k run.
+// Stages this rank's sub-files of [ffmin, ffmax) of File and calls action(g, ff) behind each, with one host thread per GPU (the
+// reference: one MPI rank per group of sub-files, slicer-v2.cpp:162-175, densitymaps.cpp:432-484).  The job's GPU k takes sub-files
+// ffmin + k, ffmin + k + G, ... (subfileGpu); local GPU g is the job's GPU gpu0 + g.  It reads sub-file k+1 into its second
+// page-locked buffer while the copy and the work on sub-file k run.
 // e->used[g] counts the sub-files GPU g has staged before the current one.  Log lines (with `log_tail`, when `log` is set) and
 // errors are collected per thread and printed GPU by GPU afterwards.
 static int walk_subfiles(Engine *e, const InputParams &p, const std::string &File, unsigned ffmin, unsigned ffmax, bool log,
@@ -330,7 +362,7 @@ static int walk_subfiles(Engine *e, const InputParams &p, const std::string &Fil
   std::vector<double> read_s(ngpu, 0.0);
   auto work = [&](int g) {
     std::ostringstream out, err;
-    for (unsigned ff = ffmin + (unsigned)g; ff < ffmax && !rcs[g]; ff += (unsigned)ngpu)
+    for (unsigned ff : gpuSubfiles(ffmin, ffmax, e->gpu0 + g, e->G))
     {
       SubFile &buf = e->bufs[2 * g + (e->used[g] & 1)];
       if (e->used[g] >= 2 && slicer_wait_staging(e->h[g])) // the copy that last read this host buffer must be done
@@ -393,7 +425,9 @@ static int walk_subfiles(Engine *e, const InputParams &p, const std::string &Fil
 }
 
 // The end of a group of passes [pass, end) after walk_subfiles: a GPU without sub-files still contributes zero maps to the sum
-// (slicer-v2.cpp:162-175: ranks with no files), the group's slots are summed on GPU 0 and its jobs' maps and counts read out.
+// (slicer-v2.cpp:162-175: ranks with no files), the group's slots are summed on the job's GPU 0 and, on rank 0, its jobs' maps and
+// counts read out.  Every rank of a job agrees that all are fine before it enters the reduce: a rank that failed never leaves
+// the others waiting inside NCCL.
 static int finish_group(Engine *e, const InputParams &p, const std::string &File, unsigned ffmin, unsigned ffmax, const std::vector<PlaneJob> &jobs,
                         const std::vector<slicer_plane_desc> &descs, const PassSpan *pass, const PassSpan *end,
                         std::vector<std::valarray<float>> &mapxytot, std::vector<std::valarray<float>> &mapxytoti, std::vector<long long> &ntotxyi)
@@ -410,8 +444,12 @@ static int finish_group(Engine *e, const InputParams &p, const std::string &File
           deposit_passes(e->h[g], descs, pass, end, false))
         return fail_capi("slicer_deposit");
     }
-  if (ngpu > 1 && slicer_reduce_all_slots(e->h.data(), ngpu, 0, j1 - j0, 0)) // replaces the 7 MPI_Reduce of slicer-v2.cpp:214-217
+  if (e->multi() && e->group->agree(0))
+    return 1;
+  if (e->comm && slicer_reduce_all_slots(e->h.data(), ngpu, 0, j1 - j0, 0)) // replaces the 7 MPI_Reduce of slicer-v2.cpp:214-217
     return fail_capi("slicer_reduce_all");
+  if (e->gpu0 != 0)
+    return 0; // the sums are on rank 0
   const double tf0 = now_s();
   for (int j = j0; j < j1; j++)
   {
@@ -439,7 +477,9 @@ static int finish_group(Engine *e, const InputParams &p, const std::string &File
 // (particle, replica) pair, plane after plane, sub-file after sub-file, type after type, particle after particle —
 // one serial stream that continues from randomizeBox's last srand().  Sweep 1 counts the accepted pairs of every
 // (plane, sub-file, type); the draws are then made here, in that order, with the same libc generator; sweep 2 applies
-// them on the device by rank (slicer_count_accepted / slicer_deposit_degraded).
+// them on the device by rank (slicer_count_accepted / slicer_deposit_degraded).  In a job of several processes each rank counts
+// its own sub-files, a sum over the ranks gives every rank the whole table, and every rank makes all the draws (the same stream)
+// and keeps those of its own sub-files: the reference's one-rank stream, whatever the split.
 static int createDensityMapsDegraded(Engine *e, const InputParams &p, const std::vector<PlaneJob> &jobs, const std::vector<slicer_plane_desc> &descs,
                                      unsigned ffmin, unsigned ffmax, const std::string &File, std::vector<std::valarray<float>> &mapxytot,
                                      std::vector<std::valarray<float>> &mapxytoti, std::vector<long long> &ntotxyi, int myid)
@@ -458,6 +498,8 @@ static int createDensityMapsDegraded(Engine *e, const InputParams &p, const std:
         return slicer_count_accepted(e->h[g], descs.data(), nj, &cnt[(size_t)(ff - ffmin) * nj * 6]);
       }))
     return 1;
+  if (e->multi() && e->group->allreduce(cnt, Group::Op::Sum))
+    return 1;
   // ---- the draws, in the reference's order: plane-major, then sub-file, then type/particle/replica
   const double thr = 1. / pow(2, p.snopt);
   std::vector<std::vector<unsigned char>> keep((size_t)nj * nff);
@@ -467,6 +509,13 @@ static int createDensityMapsDegraded(Engine *e, const InputParams &p, const std:
       long long n = 0;
       for (int t = 0; t < 6; t++)
         n += cnt[((size_t)f * nj + j) * 6 + t];
+      const int gl = subfileGpu(ffmin + f, ffmin, e->G) - e->gpu0;
+      if (gl < 0 || gl >= (int)e->h.size())
+      { // another rank's sub-file: its draws still advance the stream
+        for (long long i = 0; i < n; i++)
+          sharedRand().next();
+        continue;
+      }
       std::vector<unsigned char> &k = keep[(size_t)j * nff + f];
       k.resize((size_t)n);
       for (long long i = 0; i < n; i++)
@@ -615,7 +664,9 @@ static int check_realisations(const std::vector<std::string> &inis, const std::v
 
 int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &opt)
 {
-  const int myid = opt.quiet ? 1 : 0;
+  // only rank 0 of a job prints the reference's messages and writes files
+  const bool root = opt.rank == 0;
+  const int myid = opt.quiet || !root ? 1 : 0;
   const double t_begin = now_s();
   t_read = t_submit = t_fetch = t_write = t_engine = t_gpu = 0;
   const int K = (int)inifiles.size();
@@ -623,6 +674,27 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   {
     std::cerr << "no InputParams.ini given" << std::endl;
     return 1;
+  }
+  if (opt.nranks < 1 || opt.rank < 0 || opt.rank >= opt.nranks)
+  {
+    std::cerr << "rank " << opt.rank << " of a job of " << opt.nranks << " processes" << std::endl;
+    return 1;
+  }
+  // the job's processes meet before anything else, so that a rank that stops (an unreadable ini, a refused plan) stops the
+  // others at their next collective call: every early return below closes this rank's connections
+  Group group;
+  if (group.open(opt.rank, opt.nranks, opt.master_addr, opt.master_port, opt.connect_timeout_s))
+    return 1;
+  // the job's GPUs, rank after rank: this rank's first one and how many there are
+  int gpu0 = 0, G = 0;
+  {
+    std::vector<std::string> all;
+    if (group.allgather(std::to_string(opt.devices.size()), all))
+      return 1;
+    std::vector<int> per_rank;
+    for (const std::string &n : all)
+      per_rank.push_back(atoi(n.c_str()));
+    G = jobGpus(per_rank, opt.rank, gpu0);
   }
   std::vector<InputParams> ps(K);
   for (int k = 0; k < K; k++)
@@ -654,9 +726,9 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     q.Ds = cosmo.getDl.eval(q.zs);
   }
   Lens lens;
-  if (buildPlanes(p, lens, snapred, snappath, snapbox, cosmo.getDl, cosmo.getZl, numberOfLensPerSnap, 0)) // rank 0 writes planes_list
+  if (buildPlanes(p, lens, snapred, snappath, snapbox, cosmo.getDl, cosmo.getZl, numberOfLensPerSnap, root ? 0 : 1)) // rank 0 writes planes_list
     return 1;
-  for (int k = 1; k < K; k++)
+  for (int k = 1; k < K && root; k++)
     writePlanesList(ps[k], lens);
   double fovradiants = 0;
   for (size_t i = 0; i < lens.ld.size(); i++)
@@ -666,7 +738,7 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     const double boxl = snapbox[lens.fromsnapi[i]] / 1e3 * POS_U;
     if (!opt.replication)
     {
-      if (testFov(p.fov, boxl, lens.ld2[i], 0, fovradiants))
+      if (testFov(p.fov, boxl, lens.ld2[i], root ? 0 : 1, fovradiants))
         return 1;
     }
     else
@@ -700,6 +772,15 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   if (p.partinplanes && myid == 0)
     std::cout << "!It is not possible to resume a Gadget run with partinplanes == true!" << std::endl
               << "!!               Files on Output folder will be overwritten        !!" << std::endl;
+  // resume (slicer-v2.cpp:188-196): planes already written are skipped.  Rank 0 alone looks at the output directories and tells
+  // the others, so that every rank makes the same planes whatever its view of a shared file system
+  std::string done((size_t)K * lens.nplanes, '\0');
+  if (root && !p.partinplanes)
+    for (int k = 0; k < K; k++)
+      for (int isnap = 0; isnap < lens.nplanes; isnap++)
+        done[(size_t)k * lens.nplanes + isnap] = std::ifstream(fileOutput(ps[k], plane_label(lens.pll[isnap]))) ? 1 : 0;
+  if (group.bcast(done))
+    return 1;
 
   Engine *e = nullptr;
   int status = 0;
@@ -729,11 +810,10 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     for (int k = 0; k < K; k++)
       for (int isnap = s0; isnap < s1; isnap++)
       {
-        const std::string out = fileOutput(ps[k], plane_label(lens.pll[isnap]));
-        if (!p.partinplanes && std::ifstream(out))
-        { // resume: this plane was already written (slicer-v2.cpp:188-196)
+        if (done[(size_t)k * lens.nplanes + isnap])
+        { // resume: this plane was already written
           if (myid == 0)
-            std::cout << out << " Already exists" << std::endl;
+            std::cout << fileOutput(ps[k], plane_label(lens.pll[isnap])) << " Already exists" << std::endl;
           continue;
         }
         (k == degraded ? djobs : jobs).push_back({isnap, rcase[isnap], npix[isnap], &randoms[k]});
@@ -777,7 +857,7 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
             need = std::min(need, want);
           want = std::max(want, need);
         }
-        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need);
+        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need, &group, gpu0, G);
         t_engine += now_s() - te0;
         if (!e)
         {
@@ -814,6 +894,11 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
       join_writer(); // the previous snapshot's planes
       if (status)
         break;
+      if (!root)
+      {
+        s0 = s1;
+        continue;
+      }
       struct Batch
       {
         std::vector<PlaneJob> jobs;
@@ -873,9 +958,14 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     s0 = s1;
   }
   join_writer();
+  // every rank of a job ends with the same status: one that failed leaves the job, the others learn it here at the latest
+  if (status)
+    group.close();
+  else
+    status = group.agree(0);
   engineDestroy(e);
   if (getenv("SLICER_B200_TIMING"))
-    std::cerr << "[timing] total " << now_s() - t_begin << " s: engine/CUDA set-up " << t_engine << ", sub-file reads " << t_read << ", fetch (waits for the GPU) " << t_fetch
+    std::cerr << "[timing] " << (opt.nranks > 1 ? "rank " + std::to_string(opt.rank) + ": " : "") << "total " << now_s() - t_begin << " s: engine/CUDA set-up " << t_engine << ", sub-file reads " << t_read << ", fetch (waits for the GPU) " << t_fetch
               << ", FITS writes (background thread) " << t_write << ", device passes " << t_gpu << " (" << K << " light cone" << (K > 1 ? "s" : "") << ")"
               << std::endl;
   return status;

@@ -203,11 +203,15 @@ extern "C"
     return runLightCone(ini, o);
   }
 
-  // one light cone per ini, every snapshot read once for all (runLightCones)
+  // one light cone per ini, every snapshot read once for all (runLightCones); rank / nranks / master: one process of a job
   int shost_run_light_cones(const char **inis, int nini, const int *devices, int ndev, int replication, int fixed_vertex, int ngp,
-                            int deposit_mode, int max_slots)
+                            int deposit_mode, int max_slots, int rank, int nranks, const char *master_addr, int master_port)
   {
     RunOptions o;
+    o.rank = rank;
+    o.nranks = nranks;
+    o.master_addr = master_addr ? master_addr : "";
+    o.master_port = master_port;
     o.devices.assign(devices, devices + ndev);
     o.replication = replication != 0;
     o.fixed_vertex = fixed_vertex != 0;
@@ -217,4 +221,96 @@ extern "C"
     o.max_slots = max_slots;
     return runLightCones(std::vector<std::string>(inis, inis + nini), o);
   }
+
+  // launchFromEnv over `n` "NAME=value" strings instead of the process environment; out: rank, nranks, local rank, port and the
+  // default GPU among `ndev` visible ones
+  int shost_launch_from_env(const char **vars, int n, int ndev, int *out, char *addr, int addrcap, char *err, int errcap)
+  {
+    std::vector<std::string> kv(vars, vars + n);
+    auto env = [&](const char *name) -> const char * {
+      const size_t len = strlen(name);
+      for (const std::string &s : kv)
+        if (s.size() > len && s.compare(0, len, name) == 0 && s[len] == '=')
+          return s.c_str() + len + 1;
+      return nullptr;
+    };
+    Launch l;
+    std::string e;
+    const int rc = launchFromEnv(env, l, e);
+    snprintf(err, errcap, "%s", e.c_str());
+    snprintf(addr, addrcap, "%s", l.master_addr.c_str());
+    out[0] = l.rank;
+    out[1] = l.nranks;
+    out[2] = l.local_rank;
+    out[3] = l.master_port;
+    out[4] = defaultDevice(l, ndev);
+    return rc;
+  }
+
+  // the job's GPU assignment: sub-file ff of [ffmin, ffmax) goes to rank rank_of[ff - ffmin], local GPU gpu_of[ff - ffmin]
+  // (-1: none), for ranks that drive ngpus[r] GPUs each
+  int shost_subfile_owners(int nranks, const int *ngpus, unsigned ffmin, unsigned ffmax, int *rank_of, int *gpu_of)
+  {
+    const std::vector<int> per_rank(ngpus, ngpus + nranks);
+    std::fill(rank_of, rank_of + (ffmax - ffmin), -1);
+    std::fill(gpu_of, gpu_of + (ffmax - ffmin), -1);
+    for (int r = 0; r < nranks; r++)
+    {
+      int gpu0 = 0;
+      const int G = jobGpus(per_rank, r, gpu0);
+      for (int g = 0; g < per_rank[r]; g++)
+        for (unsigned ff : gpuSubfiles(ffmin, ffmax, gpu0 + g, G))
+        {
+          if (rank_of[ff - ffmin] >= 0)
+            return 1; // two owners
+          rank_of[ff - ffmin] = r;
+          gpu_of[ff - ffmin] = g;
+        }
+    }
+    return 0;
+  }
+
+  // the control channel (Group) for the tests: one per process
+  void *shost_group_open(int rank, int nranks, const char *addr, int port, double timeout_s, int *rc)
+  {
+    Group *g = new Group;
+    *rc = g->open(rank, nranks, addr, port, timeout_s);
+    return g;
+  }
+  void shost_group_close(void *g) { delete (Group *)g; }
+  int shost_group_bcast(void *g, char *buf, long long *len, long long cap)
+  {
+    std::string b(buf, (size_t)*len);
+    if (((Group *)g)->bcast(b) || (long long)b.size() > cap)
+      return 1;
+    memcpy(buf, b.data(), b.size());
+    *len = (long long)b.size();
+    return 0;
+  }
+  // every rank's blob, concatenated in rank order into out; lens[r]: rank r's length
+  int shost_group_allgather(void *g, const char *mine, long long len, char *out, long long *lens, long long cap)
+  {
+    std::vector<std::string> all;
+    if (((Group *)g)->allgather(std::string(mine, (size_t)len), all))
+      return 1;
+    long long off = 0;
+    for (size_t r = 0; r < all.size(); r++)
+    {
+      if (off + (long long)all[r].size() > cap)
+        return 1;
+      memcpy(out + off, all[r].data(), all[r].size());
+      lens[r] = (long long)all[r].size();
+      off += (long long)all[r].size();
+    }
+    return 0;
+  }
+  int shost_group_allreduce(void *g, long long *v, int n, int op /* 0 min, 1 max, 2 sum */)
+  {
+    std::vector<long long> w(v, v + n);
+    if (((Group *)g)->allreduce(w, op == 0 ? Group::Op::Min : op == 1 ? Group::Op::Max : Group::Op::Sum))
+      return 1;
+    std::copy(w.begin(), w.end(), v);
+    return 0;
+  }
+  int shost_group_agree(void *g, int status) { return ((Group *)g)->agree(status); }
 }

@@ -16,6 +16,7 @@
 #pragma once
 #include <cstdint>
 #include <cstdio>
+#include <functional>
 #include <string>
 #include <valarray>
 #include <vector>
@@ -194,10 +195,65 @@ void writeMaps(const InputParams &p, const Header &data, const Lens &lens, int i
                const std::valarray<float> &mapxytotrecv, const std::valarray<float> *mapxytotirecv /* [6] */, const long long *ntotxyi,
                int myid);
 
+// ---- the processes of one job (group.cpp) -----------------------------------------------------------------------
+// Rank and world size as a launcher hands them to each process: OMPI_COMM_WORLD_RANK/SIZE (Open MPI), PMI_RANK/PMI_SIZE
+// (MPICH, Intel MPI), SLURM_PROCID/SLURM_STEP_NUM_TASKS (srun; an sbatch script's batch step is one process), RANK/WORLD_SIZE
+// (torchrun), the first family that is set.  The local rank comes from OMPI_COMM_WORLD_LOCAL_RANK, MPI_LOCALRANKID, SLURM_LOCALID
+// or LOCAL_RANK (the global rank without one).  With more than one rank, MASTER_ADDR / MASTER_PORT name where rank 0 listens for
+// the others; under torchrun (TORCHELASTIC_RUN_ID set), whose agent keeps its own store on MASTER_PORT, rank 0 listens on
+// MASTER_PORT + 1.
+struct Launch
+{
+  int rank = 0, nranks = 1, local_rank = 0;
+  std::string master_addr;
+  int master_port = 0;
+};
+// `env` looks a variable up (getenv in main).  Returns 1 with a message in `err` for malformed values, or more than one rank without
+// MASTER_ADDR / MASTER_PORT.
+int launchFromEnv(const std::function<const char *(const char *)> &env, Launch &out, std::string &err);
+int defaultDevice(const Launch &l, int ndevices); // a rank's GPU when --gpus is not given: local rank modulo the visible devices
+
+// The host control channel between the ranks of a job: plain TCP, every other rank connected to rank 0.  Every call is collective
+// (all ranks make it, in the same order) and returns 0, or 1 once the group is broken: a connection failed or closed (a rank left
+// the job).  A broken group fails every later call, and rank 0 then closes every connection, so each rank stops at its next call.
+class Group
+{
+public:
+  enum class Op
+  {
+    Min,
+    Max,
+    Sum
+  };
+  ~Group();
+  // rank 0 listens on `addr`:`port`, the others connect (retrying until `timeout_s`).  One rank: no sockets, every call a no-op.
+  int open(int rank, int nranks, const std::string &addr, int port, double timeout_s);
+  int bcast(std::string &blob);                                       // rank 0's blob to every rank
+  int allgather(const std::string &mine, std::vector<std::string> &all); // every rank's blob to every rank
+  int allreduce(std::vector<long long> &v, Op op);                    // elementwise, same length on every rank
+  int agree(int status);       // 1 on every rank if any rank's status is non-zero (or the group is broken)
+  void close();                // leave the job: the others fail at their next call
+  int rank() const { return rank_; }
+  int size() const { return size_; }
+
+private:
+  int broken(const std::string &what);
+  int rank_ = 0, size_ = 1, listen_fd_ = -1;
+  bool broken_ = false;
+  std::vector<int> fds_; // rank 0: one per rank; others: [0] to rank 0
+};
+
+// Global GPU (0 .. G-1 over the GPUs of every rank, rank after rank) that takes sub-file ff of a snapshot: the round-robin of
+// slicer-v2.cpp:162-175 over all GPUs of the job.
+int subfileGpu(unsigned ff, unsigned ffmin, int G);
+std::vector<unsigned> gpuSubfiles(unsigned ffmin, unsigned ffmax, int gpu, int G); // the sub-files of the job's GPU `gpu`
+// per_rank[r]: GPUs of rank r.  Returns G, the job's GPUs; gpu0 = the job's index of rank `rank`'s first GPU
+int jobGpus(const std::vector<int> &per_rank, int rank, int &gpu0);
+
 // ---- the whole Gadget branch of main() (slicer-v2.cpp:23-230) -------------------------------------------------
 struct RunOptions
 {
-  std::vector<int> devices = {0};
+  std::vector<int> devices = {0}; // this rank's GPUs
   bool replication = false;   // CMake USE_REPLICATION (-DReplicationOnPerpendicularPlane)
   bool fixed_vertex = false;  // CMake USE_FIXED_PLC_VERTEX (-DFixedPLCVertex)
   int mas = SLICER_MAS_TSC;   // densitymaps.h:22 DO_NGP
@@ -205,6 +261,13 @@ struct RunOptions
   bool quiet = false;
   int max_slots = 0;          // accumulator slots per GPU at most (0: as many as the realisations' planes of a snapshot need, up
                               // to SLICER_MAX_SLOTS, as far as device memory allows); fewer slots mean more reads of a snapshot
+  // One job of several processes (nranks > 1): every rank runs runLightCones with the same inis and switches; the sub-files are
+  // dealt over the GPUs of all ranks, the planes summed with NCCL, and rank 0 alone writes.  Rank 0 listens on
+  // master_addr:master_port for the others, which wait up to connect_timeout_s for it.
+  int rank = 0, nranks = 1;
+  std::string master_addr;
+  int master_port = 0;
+  double connect_timeout_s = 300;
 };
 // One light cone per ini.  The inis must agree on what shapes the plan and the engine (map pixels, source redshift, field of
 // view, w, snapshot list and directory, one map per particle type); seeds, simulation name, output directory and suffix may
