@@ -88,7 +88,7 @@ EXPORTS = [
     "slicer_reduce", "slicer_fetch", "slicer_fetch_fixed", "slicer_synchronize", "slicer_get_stats",
     "slicer_frac_bits", "slicer_comm_unique_id", "slicer_comm_init_rank", "slicer_comm_init_all",
     "slicer_reduce_all", "slicer_wait_staging", "slicer_count_accepted", "slicer_deposit_degraded", "slicer_reset_stats", "slicer_timer_begin", "slicer_timer_end",
-    "slicer_selftest_arith", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
+    "slicer_selftest_arith", "slicer_selftest_packed", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
     "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory", "slicer_comm_init_ranks",
 ]
 
@@ -126,6 +126,7 @@ def lib() -> C.CDLL:
     L.slicer_reset_stats.argtypes = [C.c_void_p]
     L.slicer_timer_begin.argtypes = [C.c_void_p]
     L.slicer_selftest_arith.argtypes = [C.c_void_p, C.c_ulonglong, C.c_ulonglong, C.POINTER(C.c_ulonglong)]
+    L.slicer_selftest_packed.argtypes = [C.c_void_p, C.c_ulonglong, C.c_ulonglong, C.POINTER(C.c_ulonglong)]
     L.slicer_timer_end.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
     L.slicer_stage_particles.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]
     L.slicer_stage_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]
@@ -320,6 +321,12 @@ class Slicer:
         from __fdiv_rn."""
         out = (C.c_ulonglong * 3)()
         _check(lib().slicer_selftest_arith(self.h, int(n), int(seed), out))
+        return tuple(int(v) for v in out)
+
+    def selftest_packed(self, n: int, seed: int):
+        """(fma2, add2, sub2, mul2): how many lanes of the kernels' packed FP32 operations differ from the scalar ones."""
+        out = (C.c_ulonglong * 4)()
+        _check(lib().slicer_selftest_packed(self.h, int(n), int(seed), out))
         return tuple(int(v) for v in out)
 
     def count_accepted(self, planes: Sequence[PlaneDesc]) -> np.ndarray:

@@ -2,6 +2,7 @@
 #pragma once
 #include <stdint.h>
 #include "device_chain.cuh"
+#include "packed_f32.cuh"
 
 // int64 fixed point -> float32 map, summing `ntypes` per-type accumulators first (exact integer sum).
 // Replaces the float adds of densitymaps.cpp:511-513 and the float MPI_Reduce of slicer-v2.cpp:214-217:
@@ -129,4 +130,54 @@ __global__ void selftest_fdiv_kernel(unsigned long long n, unsigned long long se
   }
   if (bad)
     atomicAdd(out + 2, bad);
+}
+
+// The packed FP32 helpers (packed_f32.cuh) against their scalar counterparts, lane by lane: n random operand sets, each operand
+// drawn from every class (any bit pattern: normals, denormals, +-0, +-inf, NaN; denormals; special values; normals of the box
+// transform's exponent range).  out[0..3] += fma2 / add2 / sub2 / mul2 lanes whose bits differ (two NaNs count as equal).
+__device__ __forceinline__ float selftest_operand(unsigned long long h)
+{
+  const unsigned m = (unsigned)h;
+  switch ((unsigned)(h >> 61))
+  {
+  case 0:
+  case 1:
+    return __uint_as_float(m);
+  case 2:
+    return __uint_as_float(m & 0x807fffffu); // denormal or +-0
+  case 3:
+  {
+    const unsigned sp[8] = {0x00000000u, 0x7f800000u, 0x7fc00000u, 0x3f800000u, 0x3f000000u, 0x00800000u, 0x7f7fffffu, 0x00000001u};
+    return __uint_as_float(sp[m & 7u] | (m & 0x80000000u));
+  }
+  default:
+    return __uint_as_float((m & 0x807fffffu) | ((unsigned)(127 - 45 + (h >> 32) % 91) << 23));
+  }
+}
+__device__ __forceinline__ unsigned long long selftest_differs(float2 p, float a, float b)
+{
+  const bool dx = __float_as_uint(p.x) != __float_as_uint(a) && !(isnan(p.x) && isnan(a));
+  const bool dy = __float_as_uint(p.y) != __float_as_uint(b) && !(isnan(p.y) && isnan(b));
+  return (unsigned long long)dx + (unsigned long long)dy;
+}
+__global__ void selftest_packed_kernel(unsigned long long n, unsigned long long seed, unsigned long long *out)
+{
+  unsigned long long bad[4] = {0, 0, 0, 0};
+  const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+  for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride)
+  {
+    float v[6];
+#pragma unroll
+    for (int k = 0; k < 6; k++)
+      v[k] = selftest_operand(selftest_mix(seed + 6 * i + k));
+    const float2 a = make_float2(v[0], v[1]), b = make_float2(v[2], v[3]), c = make_float2(v[4], v[5]);
+    bad[0] += selftest_differs(fma2_rn(a, b, c), __fmaf_rn(a.x, b.x, c.x), __fmaf_rn(a.y, b.y, c.y));
+    bad[1] += selftest_differs(add2_rn(a, b), __fadd_rn(a.x, b.x), __fadd_rn(a.y, b.y));
+    bad[2] += selftest_differs(sub2_rn(a, b), __fsub_rn(a.x, b.x), __fsub_rn(a.y, b.y));
+    bad[3] += selftest_differs(mul2_rn(a, b), __fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y));
+  }
+#pragma unroll
+  for (int k = 0; k < 4; k++)
+    if (bad[k])
+      atomicAdd(out + k, bad[k]);
 }

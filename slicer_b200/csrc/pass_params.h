@@ -5,6 +5,7 @@
 // slicer-v2.cpp:184-185) share an XformDev, so the box transform of gadget2io.cpp:204-270 is evaluated
 // once per particle and only the slab test (densitymaps.cpp:374) is per plane.
 #pragma once
+#include <stddef.h>
 #include <stdint.h>
 #include "../../include/slicer_b200.h"
 #include "lean_math.h"
@@ -23,14 +24,16 @@
 #define SLICER_CHECK(cond) ((void)0)
 #endif
 
+// The float arrays cf, sgn, sinv, offs and wadd start at multiples of 8 bytes: the kernels read their x and y entries as one
+// register pair (one 64-bit constant load) for the packed FP32 operations (deposit_pipelined.cuh: screen2, lean_axis2).
 struct XformDev
 {
   double box;    // Header.boxsize (data.h:70)
   double c[3];   // Random.x0,y0,z0 (data.h:128)
-  float boxf;    // == box when exact_f32
   float cf[3];   // == c[] when exact_f32
-  float rcase;   // slicer-v2.cpp:137,185
+  float boxf;    // == box when exact_f32
   float sgn[3];  // sign applied to output axis k (already permuted): Random.sgn of the raw axis feeding it
+  float rcase;   // slicer-v2.cpp:137,185
   int perm[3];   // raw axis (0,1,2) feeding output axis k (x,y,z): Random.face, gadget2io.cpp:223-252
   int exact_f32; // box and centre are float-representable: float ops reproduce the double chain bit for bit
   int first_plane, nplanes; // planes [first_plane, first_plane+nplanes) of PassParams::pl use this transform
@@ -40,16 +43,19 @@ struct XformDev
   // one wrap (a<0 -> a+1) gives the box coordinate.  Particles the screen cannot decide are sent to the
   // exact chain, never dropped.
   float sinv[3];
-  float offs[3];
   float tmax;       // max over this transform's planes of pre_tx (>= pre_ty)
+  float offs[3];
   float thr_m;      // additive slack of the lateral test: screen error + tmax * (z error)
   float zlo_m, zhi_m; // zmin/zmax widened by the screen's error margin
   float zamb;       // z-wrap ambiguity: |w - 0.5| > zamb  => undecidable
   float raw_hi;     // raw coordinates outside the open interval (0, raw_hi) may wrap in the exact chain => undecidable
   // --- fast box transform of the lean exact phase (deposit_pipelined.cuh: lean_axis), valid for raw in (LeanDev::umin, raw_hi) ---
-  float nboxf;      // -boxf: residual r = fma(q0, -box, u) of the division u / box
   float wadd[3];    // 1 when sgn[k] < 0 (the wrap 1 + q of gadget2io.cpp:213-214 always fires), else 0 (no wrap can fire)
+  float nboxf;      // -boxf: residual r = fma(q0, -box, u) of the division u / box
 };
+static_assert(offsetof(XformDev, cf) % 8 == 0 && offsetof(XformDev, sgn) % 8 == 0 && offsetof(XformDev, sinv) % 8 == 0 &&
+                  offsetof(XformDev, offs) % 8 == 0 && offsetof(XformDev, wadd) % 8 == 0,
+              "packed pairs of XformDev are 8-byte aligned");
 
 struct PlaneDev
 {

@@ -885,7 +885,7 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
         if (P->pl[a].zlo < P->pl[b].zhi && P->pl[b].zlo < P->pl[a].zhi)
           P->fast = 0; // overlapping slabs: a particle can belong to two planes
     }
-    // float screen of the pipelined kernel (deposit_pipelined.cuh: screen()); all margins are >= 5x the
+    // float screen of the pipelined kernel (deposit_pipelined.cuh: screen2()); all margins are >= 5x the
     // worst-case difference between the screen's coordinates and the exact chain's
     X.tmax = 0.f;
     for (int q = X.first_plane; q < X.first_plane + X.nplanes; q++)
@@ -1484,6 +1484,24 @@ extern "C" int slicer_selftest_arith(slicer_handle *h, unsigned long long n, uns
   CU(cudaGetLastError());
   CU(cudaStreamSynchronize(h->compute));
   CU(cudaMemcpy(out, d, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+extern "C" int slicer_selftest_packed(slicer_handle *h, unsigned long long n, unsigned long long seed, unsigned long long out[4])
+{
+  if (!h || !out)
+    return fail("null argument");
+  if (set_device(h))
+    return 1;
+  unsigned long long *d = (unsigned long long *)h->d_out; // npix_max^2 floats of scratch
+  if (h->npix2max * sizeof(float) < 4 * sizeof(unsigned long long))
+    return fail("slicer_selftest_packed needs npix_max >= 3");
+  CU(cudaStreamSynchronize(h->compute));
+  CU(cudaMemset(d, 0, 4 * sizeof(unsigned long long)));
+  selftest_packed_kernel<<<h->sm_count * 8, 256, 0, h->compute>>>(n, seed, d);
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(h->compute));
+  CU(cudaMemcpy(out, d, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
   return 0;
 }
 
