@@ -90,6 +90,7 @@ EXPORTS = [
     "slicer_reduce_all", "slicer_wait_staging", "slicer_count_accepted", "slicer_deposit_degraded", "slicer_reset_stats", "slicer_timer_begin", "slicer_timer_end",
     "slicer_selftest_arith", "slicer_selftest_packed", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
     "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory", "slicer_comm_init_ranks",
+    "slicer_kernels_run",
 ]
 
 
@@ -124,6 +125,7 @@ def lib() -> C.CDLL:
     L.slicer_begin_snapshot.argtypes = [C.c_void_p, C.c_double, C.POINTER(C.c_double), C.c_int]
     L.slicer_next_batch.argtypes = [C.c_void_p]
     L.slicer_reset_stats.argtypes = [C.c_void_p]
+    L.slicer_kernels_run.argtypes = [C.c_void_p, C.POINTER(C.c_ulonglong)]
     L.slicer_timer_begin.argtypes = [C.c_void_p]
     L.slicer_selftest_arith.argtypes = [C.c_void_p, C.c_ulonglong, C.c_ulonglong, C.POINTER(C.c_ulonglong)]
     L.slicer_selftest_packed.argtypes = [C.c_void_p, C.c_ulonglong, C.c_ulonglong, C.POINTER(C.c_ulonglong)]
@@ -375,6 +377,13 @@ class Slicer:
 
     def reset_stats(self):
         _check(lib().slicer_reset_stats(self.h))
+
+    def kernels_run(self) -> int:
+        """Mask of the deposit kernels launched since creation or reset_stats(): bit i = pipelined variant i, bit 40 + mas = the
+        simple kernel (include/slicer_b200.h: slicer_kernels_run)."""
+        m = C.c_ulonglong(0)
+        _check(lib().slicer_kernels_run(self.h, C.byref(m)))
+        return m.value
 
     def timer_begin(self):
         _check(lib().slicer_timer_begin(self.h))

@@ -151,6 +151,7 @@ struct slicer_handle
   int plane_npix[SLICER_MAX_SLOTS];
   bool copy_pending = false;
   slicer_stats stats;
+  unsigned long long kernels_run = 0; // slicer_kernels_run: bit i = pipelined_table() entry i, bit 40 + mas = deposit_simple_kernel
   size_t device_bytes = 0;
   ncclComm_t comm = nullptr;
   int nranks = 1, rank = 0;
@@ -1086,7 +1087,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     Q.rec_s = h->bin.rec_s;
     Q.mass_s = D.mass ? h->bin.mass_s : nullptr;
     Q.capacity = h->bin.capacity;
-    if (pipelined_launch(grid, h->cfg.mas, true, P, S, E, F, h->compute))
+    if (pipelined_launch(grid, h->cfg.mas, true, P, S, E, F, h->compute, &h->kernels_run))
       return fail("record kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     const int nwin = (nbins + binned::MAX_BINS - 1) / binned::MAX_BINS;
     const int wbins = (nbins + nwin - 1) / nwin;
@@ -1436,7 +1437,8 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
         if (binned_pass(h, P, D, F))
           return 1;
       }
-      else if (maps_ready(h) || pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F, h->compute))
+      else if (maps_ready(h) || pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F, h->compute,
+                                                         &h->kernels_run))
         return fail("pipelined launch failed: %s", cudaGetErrorString(cudaGetLastError()));
     }
     else
@@ -1450,6 +1452,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
         deposit_simple_kernel<SLICER_MAS_NGP><<<blocks, 256, 0, h->compute>>>(P, D, F);
       else
         deposit_simple_kernel<SLICER_MAS_TSC><<<blocks, 256, 0, h->compute>>>(P, D, F);
+      h->kernels_run |= 1ull << (PIPELINED_VARIANTS + h->cfg.mas);
       CU(cudaGetLastError());
     }
     h->stats.launches++;
@@ -1845,6 +1848,15 @@ extern "C" int slicer_reset_stats(slicer_handle *h)
   h->stats.deposit_launches = 0;
   h->stats.launches = 0;
   h->stats.particles_streamed = 0;
+  h->kernels_run = 0;
+  return 0;
+}
+
+extern "C" int slicer_kernels_run(slicer_handle *h, unsigned long long *mask)
+{
+  if (!h || !mask)
+    return fail("null argument");
+  *mask = h->kernels_run;
   return 0;
 }
 
