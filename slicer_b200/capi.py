@@ -24,6 +24,7 @@ MAS_TSC, MAS_NGP = 0, 1
 LAYOUT_AOS, LAYOUT_SOA = 0, 1
 KERNEL_AUTO, KERNEL_SIMPLE, KERNEL_PIPELINED = 0, 1, 2
 DEPOSIT_AUTO, DEPOSIT_DIRECT, DEPOSIT_BINNED = 0, 1, 2
+KAPPA_MAX_SOURCES = 8
 
 
 class SlicerError(RuntimeError):
@@ -90,7 +91,7 @@ EXPORTS = [
     "slicer_reduce_all", "slicer_wait_staging", "slicer_count_accepted", "slicer_deposit_degraded", "slicer_reset_stats", "slicer_timer_begin", "slicer_timer_end",
     "slicer_selftest_arith", "slicer_selftest_packed", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
     "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory", "slicer_comm_init_ranks",
-    "slicer_kernels_run",
+    "slicer_kernels_run", "slicer_kappa_maps", "slicer_kappa_add", "slicer_kappa_fetch", "slicer_kappa_load",
 ]
 
 
@@ -155,6 +156,10 @@ def lib() -> C.CDLL:
     L.slicer_comm_init_all.argtypes = [C.POINTER(C.c_void_p), C.c_int]
     L.slicer_comm_init_ranks.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_char_p, C.c_int, C.c_int]
     L.slicer_reduce_all.argtypes = [C.POINTER(C.c_void_p), C.c_int, C.c_int, C.c_int]
+    L.slicer_kappa_maps.argtypes = [C.c_void_p, C.c_int, C.c_int]
+    L.slicer_kappa_add.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+    L.slicer_kappa_fetch.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    L.slicer_kappa_load.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     _lib = L
     return L
 
@@ -374,6 +379,34 @@ class Slicer:
         out = np.empty(npix * npix, np.int64)
         _check(lib().slicer_fetch_fixed(self.h, plane, ptype, out.ctypes.data))
         return out.reshape(npix, npix)
+
+    # -- convergence maps -------------------------------------------------------------------------
+    def kappa_maps(self, nmaps: int, npix: int = 0):
+        """Allocate and zero `nmaps` float64 maps of npix^2 on the device (0 frees them)."""
+        self._kappa_npix = int(npix or self.cfg.npix_max)
+        _check(lib().slicer_kappa_maps(self.h, int(nmaps), self._kappa_npix))
+
+    def kappa_add(self, first_slot: int, maps: Sequence[int], scale, offset):
+        """Slots first_slot .. first_slot + len(maps) - 1 in order: map maps[j] + k += scale[j, k] * plane_j + offset[j, k]
+        (scale, offset: float64 [nplanes, nsrc]).  Asynchronous."""
+        m = np.ascontiguousarray(maps, np.int32)
+        sc = np.ascontiguousarray(scale, np.float64).reshape(len(m), -1)
+        of = np.ascontiguousarray(offset, np.float64).reshape(sc.shape)
+        _check(lib().slicer_kappa_add(self.h, int(first_slot), len(m), m.ctypes.data, sc.shape[1], sc.ctypes.data, of.ctypes.data))
+
+    def kappa_fetch(self, m: int) -> np.ndarray:
+        """-> float64 [npix, npix] indexed [gy, gx]"""
+        n = getattr(self, "_kappa_npix", self.cfg.npix_max)
+        out = np.empty(n * n, np.float64)
+        _check(lib().slicer_kappa_fetch(self.h, int(m), out.ctypes.data))
+        return out.reshape(n, n)
+
+    def kappa_load(self, m: int, values: np.ndarray):
+        v = np.ascontiguousarray(values, np.float64).reshape(-1)
+        n = getattr(self, "_kappa_npix", self.cfg.npix_max)
+        if v.size != n * n:
+            raise ValueError("one value per pixel")
+        _check(lib().slicer_kappa_load(self.h, int(m), v.ctypes.data))
 
     def reset_stats(self):
         _check(lib().slicer_reset_stats(self.h))

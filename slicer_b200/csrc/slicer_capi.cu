@@ -20,6 +20,7 @@
 #include "deposit_simple.cuh"
 #include "deposit_pipelined.cuh"
 #include "deposit_degrade.cuh"
+#include "kappa.cuh"
 
 #define POS_U 1.0 /* gadget2io.h:14 */
 
@@ -145,6 +146,14 @@ struct slicer_handle
   unsigned long long *d_counts = nullptr; // [max_planes][6][2]
   float *d_out = nullptr;                 // npix2max
   long long *d_sum = nullptr;             // npix2max
+  // convergence maps (slicer_kappa_*): kappa.n maps of kappa.npix^2 doubles, each starting kappa.stride doubles after the last
+  struct
+  {
+    double *maps = nullptr;
+    unsigned *ovf = nullptr; // one flag per map
+    int n = 0, npix = 0;
+    size_t stride = 0;
+  } kappa;
   double boxsize = 0;
   double massarr[SLICER_NTYPES] = {0, 0, 0, 0, 0, 0};
   int hydro = 0;
@@ -497,6 +506,8 @@ extern "C" void slicer_destroy(slicer_handle *h)
   cudaFree(h->d_counts);
   cudaFree(h->d_out);
   cudaFree(h->d_sum);
+  cudaFree(h->kappa.maps);
+  cudaFree(h->kappa.ovf);
   if (h->ev_copy)
     cudaEventDestroy(h->ev_copy);
   for (int b = 0; b < 2; b++)
@@ -1816,6 +1827,146 @@ extern "C" int slicer_fetch_fixed(slicer_handle *h, int plane, int type, long lo
     return fail("plane %d: a fixed-point accumulator exceeded 2^63 (more than %.3g mass units in one pixel at %d fraction bits); "
                 "create the handle with a smaller slicer_config.frac_bits", plane, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
   }
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// convergence maps (kappa.cuh)
+// ------------------------------------------------------------------------------------------------------------
+extern "C" int slicer_kappa_maps(slicer_handle *h, int nmaps, int npix)
+{
+  if (!h)
+    return fail("null handle");
+  if (nmaps < 0 || (nmaps > 0 && (npix < 1 || npix > h->cfg.npix_max)))
+    return fail("slicer_kappa_maps: %d maps of %d^2 (npix must be 1..%d)", nmaps, npix, h->cfg.npix_max);
+  if (set_device(h))
+    return 1;
+  if (h->kappa.maps)
+  { // (cudaFree waits for the work that still reads or writes them)
+    CU(cudaFree(h->kappa.maps));
+    CU(cudaFree(h->kappa.ovf));
+    h->device_bytes -= (size_t)h->kappa.n * (h->kappa.stride * sizeof(double) + sizeof(unsigned));
+    h->kappa.maps = nullptr;
+    h->kappa.ovf = nullptr;
+    h->kappa.n = h->kappa.npix = 0;
+  }
+  if (nmaps == 0)
+    return 0;
+  const size_t stride = ((size_t)npix * npix + 1) & ~(size_t)1; // every map starts on a 16-byte boundary
+  if (dev_alloc(h, &h->kappa.maps, (size_t)nmaps * stride))
+    return 1;
+  if (dev_alloc(h, &h->kappa.ovf, (size_t)nmaps))
+  {
+    cudaFree(h->kappa.maps);
+    h->kappa.maps = nullptr;
+    h->device_bytes -= (size_t)nmaps * stride * sizeof(double);
+    return 1;
+  }
+  h->kappa.n = nmaps;
+  h->kappa.npix = npix;
+  h->kappa.stride = stride;
+  CU(cudaMemsetAsync(h->kappa.maps, 0, (size_t)nmaps * stride * sizeof(double), h->compute));
+  CU(cudaMemsetAsync(h->kappa.ovf, 0, (size_t)nmaps * sizeof(unsigned), h->compute));
+  return 0;
+}
+
+extern "C" int slicer_kappa_add(slicer_handle *h, int first_slot, int nplanes, const int *map, int nsrc, const double *scale, const double *offset)
+{
+  if (!h || !map || !scale || !offset)
+    return fail("slicer_kappa_add: null argument");
+  if (!h->kappa.maps)
+    return fail("slicer_kappa_add: no convergence maps (slicer_kappa_maps)");
+  if (nsrc < 1 || nsrc > SLICER_KAPPA_MAX_SOURCES)
+    return fail("slicer_kappa_add: %d sources (1..%d)", nsrc, SLICER_KAPPA_MAX_SOURCES);
+  if (nplanes < 1 || first_slot < 0 || first_slot + nplanes > h->cfg.max_planes)
+    return fail("slicer_kappa_add: slots %d..%d outside 0..%d", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
+  KappaArgs A;
+  memset(&A, 0, sizeof(A));
+  for (int j = 0; j < nplanes; j++)
+  {
+    const int q = first_slot + j;
+    if (h->plane_npix[q] <= 0)
+      return fail("slicer_kappa_add: slot %d has not been deposited", q);
+    if (h->plane_npix[q] != h->kappa.npix)
+      return fail("slicer_kappa_add: slot %d holds a %d^2 plane, the maps are %d^2", q, h->plane_npix[q], h->kappa.npix);
+    if (map[j] < 0 || map[j] + nsrc > h->kappa.n)
+      return fail("slicer_kappa_add: maps %d..%d of plane %d outside 0..%d", map[j], map[j] + nsrc - 1, j, h->kappa.n - 1);
+    for (int k = 0; k < nsrc; k++)
+    {
+      const double sc = scale[(size_t)j * nsrc + k], of = offset[(size_t)j * nsrc + k];
+      A.scale[j * SLICER_KAPPA_MAX_SOURCES + k] = sc;
+      A.offset[j * SLICER_KAPPA_MAX_SOURCES + k] = of;
+      if (sc != 0 || of != 0)
+        A.plane_mask[j] |= 1u << k;
+    }
+    // runs of consecutive planes into the same maps: each map of a run is read and written once
+    if (j == 0 || map[j] != map[j - 1])
+    {
+      A.run_begin[A.nruns] = j;
+      A.run_map[A.nruns] = map[j];
+      A.nruns++;
+    }
+    A.run_mask[A.nruns - 1] |= A.plane_mask[j];
+    A.run_begin[A.nruns] = j + 1;
+  }
+  if (set_device(h) || resolve_deferred(h, first_slot, nplanes) || wait_settled(h, false) || wait_slot_reduces(h, first_slot, nplanes))
+    return 1;
+  const size_t npix2 = (size_t)h->kappa.npix * h->kappa.npix;
+  A.acc = h->d_acc + (size_t)first_slot * h->ntypes_alloc * h->npix2max;
+  A.maps = h->kappa.maps;
+  A.map_ovf = h->kappa.ovf;
+  A.slot_stride = (unsigned long long)h->ntypes_alloc * h->npix2max;
+  A.type_stride = h->npix2max;
+  A.map_stride = h->kappa.stride;
+  A.npix2 = npix2;
+  A.inv_scale = ldexp(1.0, -h->frac_bits);
+  A.ntypes = h->ntypes_alloc;
+  A.nsrc = nsrc;
+  A.nmaps = h->kappa.n;
+  // 16-byte loads when every plane, type and map starts on a 16-byte boundary and the pixels come in pairs
+  const bool vec = (npix2 % 2 == 0) && (h->npix2max % 2 == 0);
+  const size_t groups = vec ? npix2 / 2 : npix2;
+  const int blocks = (int)((groups + 255) / 256 < (size_t)h->sm_count * 8 ? (groups + 255) / 256 : (size_t)h->sm_count * 8);
+  if (vec)
+    kappa_add_kernel<true><<<blocks, 256, 0, h->compute>>>(A);
+  else
+    kappa_add_kernel<false><<<blocks, 256, 0, h->compute>>>(A);
+  CU(cudaGetLastError());
+  h->stats.launches++;
+  return 0;
+}
+
+static int check_kappa_map(slicer_handle *h, int map, const void *buf)
+{
+  if (!h || !buf)
+    return fail("null argument");
+  if (map < 0 || map >= h->kappa.n)
+    return fail("convergence map %d outside 0..%d", map, h->kappa.n - 1);
+  return set_device(h);
+}
+
+extern "C" int slicer_kappa_fetch(slicer_handle *h, int map, double *out)
+{
+  if (check_kappa_map(h, map, out))
+    return 1;
+  const size_t npix2 = (size_t)h->kappa.npix * h->kappa.npix;
+  unsigned ovf = 0;
+  CU(cudaMemcpyAsync(out, h->kappa.maps + (size_t)map * h->kappa.stride, npix2 * sizeof(double), cudaMemcpyDeviceToHost, h->compute));
+  CU(cudaMemcpyAsync(&ovf, h->kappa.ovf + map, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
+  CU(cudaStreamSynchronize(h->compute));
+  if (ovf)
+    return fail("convergence map %d: a fixed-point accumulator it summed exceeded 2^63 (more than %.3g mass units in one pixel at %d "
+                "fraction bits); create the handle with a smaller slicer_config.frac_bits", map, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
+  return 0;
+}
+
+extern "C" int slicer_kappa_load(slicer_handle *h, int map, const double *in)
+{
+  if (check_kappa_map(h, map, in))
+    return 1;
+  const size_t npix2 = (size_t)h->kappa.npix * h->kappa.npix;
+  CU(cudaMemcpyAsync(h->kappa.maps + (size_t)map * h->kappa.stride, in, npix2 * sizeof(double), cudaMemcpyHostToDevice, h->compute));
+  CU(cudaStreamSynchronize(h->compute));
   return 0;
 }
 

@@ -33,6 +33,10 @@ def lib():
         L.shost_run_light_cone.argtypes = [C.c_char_p, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]
         L.shost_run_light_cones.argtypes = [C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                             C.c_int, C.c_char_p, C.c_int]
+        L.shost_run_light_cones_kappa.argtypes = ([C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                   C.c_int, C.c_int, C.c_char_p, C.c_int, _f64p, C.c_int, C.c_int])
+        L.shost_kappa_weights.argtypes = ([C.c_double] * 4 + [C.c_int, _f64p, _f64p, C.c_double, C.c_int, C.c_int, _f64p, C.c_int,
+                                                              C.POINTER(C.c_int)] + [_f64p] * 6)
         L.shost_launch_from_env.argtypes = [C.POINTER(C.c_char_p), C.c_int, C.c_int, _i32p, C.c_char_p, C.c_int, C.c_char_p, C.c_int]
         L.shost_subfile_owners.argtypes = [C.c_int, _i32p, C.c_uint, C.c_uint, _i32p, _i32p]
         L.shost_group_open.restype = C.c_void_p
@@ -65,6 +69,27 @@ def plan(om0, oml, w, zs, snapred, snapbox, directory, suffix="t", cap=4096):
     n = nplanes.value
     return dict(nplanes=n, Ds=Ds.value, ld=ld[:n].copy(), ld2=ld2[:n].copy(), zsimlens=zsim[:n].copy(), zfromsnap=zfs[:n].copy(),
                 fromsnapi=fromsnapi[:n].copy(), randomize=randomize[:n].copy(), replication=replication[: nrepl.value].copy())
+
+
+def kappa_weights(om0, oml, w, zs, snapred, snapbox, fov, npix, zs_list, cap=4096):
+    """Born weights of the plan of (om0, oml, w, zs) on these snapshots (redshifts, boxes in kpc/h), field of `fov` degrees on npix^2
+    pixels, for each source redshift of zs_list: scale, offset [nplanes, nsrc] such that a plane adds scale * mass + offset to each
+    pixel of the convergence map (mass in 1e10 Msun/h).  Also the plane edges ld, ld2, z = getZl((ld + ld2) / 2) and chi_s = getDl(zs_k)."""
+    snapred = np.ascontiguousarray(snapred, np.float64)
+    snapbox = np.ascontiguousarray(snapbox, np.float64)
+    zl_ = np.ascontiguousarray(zs_list, np.float64)
+    S = len(zl_)
+    n = C.c_int()
+    scale, offset = np.zeros(cap * S), np.zeros(cap * S)
+    ld, ld2, z = np.zeros(cap), np.zeros(cap), np.zeros(cap)
+    chis = np.zeros(S)
+    rc = lib().shost_kappa_weights(om0, oml, w, zs, len(snapred), snapred, snapbox, fov, int(npix), S, zl_, cap, C.byref(n), scale, offset, ld,
+                                   ld2, z, chis)
+    if rc:
+        raise RuntimeError(f"shost_kappa_weights rc={rc}")
+    n = n.value
+    return dict(scale=scale[: n * S].reshape(n, S).copy(), offset=offset[: n * S].reshape(n, S).copy(), ld=ld[:n].copy(), ld2=ld2[:n].copy(),
+                z=z[:n].copy(), chis=chis)
 
 
 def randomize_box(seedcenter, seedface, seedsign, randomize, fixed_vertex=False):
@@ -124,16 +149,23 @@ def run_light_cone(ini, devices=(0,), replication=False, fixed_vertex=False, ngp
 
 
 def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0, max_slots=0, rank=0, nranks=1,
-                    master=None):
+                    master=None, kappa_zs=None, write_planes=True):
     """One light cone per ini (realisations of one plan: other seeds, other outputs), every snapshot read once for all (once per
     group of planes that fits `max_slots` accumulators per GPU, when given).  Returns 0 on success; inis that disagree on the
     plan are refused before anything is written.
     rank / nranks / master ("host:port", where rank 0 listens): this process is one rank of a job of `nranks` processes that
     all make this call with the same arguments but `rank` and `devices`; rank 0 writes the files.  The launcher's environment
-    is not read."""
+    is not read.
+    kappa_zs: source redshifts of the convergence maps to write per light cone (None: none; NaN stands for the ini's source
+    redshift); write_planes=False writes those maps only."""
     dev = np.ascontiguousarray(devices, np.int32)
     arr = (C.c_char_p * len(inis))(*[str(i).encode() for i in inis])
     addr, port = (master.rsplit(":", 1) if master else ("", 0))
+    if kappa_zs is not None or not write_planes:
+        zs = np.ascontiguousarray(list(kappa_zs or []) or [0.0], np.float64)
+        return lib().shost_run_light_cones_kappa(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
+                                                 int(max_slots), int(rank), int(nranks), addr.encode(), int(port), zs, len(kappa_zs or []),
+                                                 int(bool(write_planes)))
     return lib().shost_run_light_cones(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
                                        int(max_slots), int(rank), int(nranks), addr.encode(), int(port))
 

@@ -24,6 +24,7 @@ namespace slicer
 
 // wall-clock phase totals of the last runLightCones (seconds): printed when SLICER_B200_TIMING is set
 static double t_read = 0, t_submit = 0, t_fetch = 0, t_write = 0, t_engine = 0, t_gpu = 0; // t_gpu: device time of the passes
+static double t_kappa = 0, t_kappa_add = 0; // convergence maps: slicer_kappa_add calls (t_kappa_add) + read-out and writes of the maps
 static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 struct Engine
@@ -44,6 +45,11 @@ struct Engine
   Group *group = nullptr;
   int gpu0 = 0, G = 1;
   bool multi() const { return group && group->size() > 1; }
+  // convergence maps on the job's GPU 0 (kappa_maps of kappa_npix^2; 0: none) and the Born weights of every plane for each of the
+  // kappa_nsrc sources: [isnap * kappa_nsrc + k]
+  int kappa_maps = 0, kappa_npix = 0, kappa_nsrc = 0;
+  std::vector<double> kappa_scale, kappa_offset;
+  bool kappa_here() const { return kappa_maps > 0 && gpu0 == 0; }
 };
 
 // device time of the passes the handles ran (summed over the GPUs), before they are destroyed: SLICER_B200_TIMING only
@@ -65,13 +71,15 @@ static void add_gpu_time(Engine *e)
 // at most the particle capacity), two npix^2 read-out buffers (12 B per pixel) and the deferred-pair banks (2 x 24 B x 2^19 per
 // 16 slots); 512 MiB cover the banks, the kernels' scratch and the context's own allocations.  Checked every time the handles
 // are made, so a rebuild with a larger particle capacity (ensure_capacity) takes fewer slots rather than failing to allocate.
-static int choose_slots(const std::vector<int> &devices, int want, int need, int npix_max, bool per_type, size_t capacity, int &slots)
+// `extra0` bytes more are taken on the first device (the convergence maps on the job's GPU 0).
+static int choose_slots(const std::vector<int> &devices, int want, int need, int npix_max, bool per_type, size_t capacity, size_t extra0, int &slots)
 {
   const size_t per_slot = (size_t)(per_type ? 6 : 1) * npix_max * npix_max * 8;
-  const size_t reserve = capacity * (2 * 16 + 26) + (size_t)npix_max * npix_max * 12 + ((size_t)512 << 20);
   slots = want;
-  for (int d : devices)
+  for (size_t g = 0; g < devices.size(); g++)
   {
+    const int d = devices[g];
+    const size_t reserve = capacity * (2 * 16 + 26) + (size_t)npix_max * npix_max * 12 + ((size_t)512 << 20) + (g == 0 ? extra0 : 0);
     size_t free_b = 0, total_b = 0;
     if (slicer_device_memory(d, &free_b, &total_b))
     {
@@ -100,11 +108,22 @@ static int fail_capi(const char *what)
 static int make_handles(Engine *e)
 {
   add_gpu_time(e);
+  // partial convergence maps survive a rebuild of the handles (ensure_capacity): read out here, loaded into the new handle below
+  std::vector<std::vector<double>> kappa_saved;
+  if (e->kappa_here() && !e->h.empty() && e->h[0])
+  {
+    kappa_saved.assign(e->kappa_maps, std::vector<double>((size_t)e->kappa_npix * e->kappa_npix));
+    for (int m = 0; m < e->kappa_maps; m++)
+      if (slicer_kappa_fetch(e->h[0], m, kappa_saved[m].data()))
+        return fail_capi("slicer_kappa_fetch");
+  }
   for (auto *hh : e->h)
     slicer_destroy(hh);
   e->h.assign(e->devices.size(), nullptr);
   e->comm = false;
-  if (e->want_slots > 0 && choose_slots(e->devices, e->want_slots, e->need_slots, e->npix_max, e->per_type, e->capacity, e->max_planes))
+  const size_t kappa_bytes = e->kappa_here() ? (size_t)e->kappa_maps * ((size_t)e->kappa_npix * e->kappa_npix + 2) * 8 : 0;
+  if (e->want_slots > 0 &&
+      choose_slots(e->devices, e->want_slots, e->need_slots, e->npix_max, e->per_type, e->capacity, kappa_bytes, e->max_planes))
     return 1;
   if (e->multi())
   { // every rank allocates the same slots: the passes, and so the reduces, are planned from them
@@ -150,6 +169,20 @@ static int make_handles(Engine *e)
       std::cerr << "slicer_create failed on GPU " << e->devices[g] << ": " << errs[g] << std::endl;
       failed = 1;
     }
+  if (!failed && e->kappa_here())
+  {
+    if (slicer_kappa_maps(e->h[0], e->kappa_maps, e->kappa_npix))
+    {
+      std::cerr << "convergence maps on GPU " << e->devices[0] << ": " << slicer_last_error() << std::endl;
+      failed = 1;
+    }
+    for (int m = 0; m < (int)kappa_saved.size() && !failed; m++)
+      if (slicer_kappa_load(e->h[0], m, kappa_saved[m].data()))
+      {
+        std::cerr << "slicer_kappa_load: " << slicer_last_error() << std::endl;
+        failed = 1;
+      }
+  }
   if (e->multi() ? e->group->agree(failed) : failed) // (no rank may enter the communicator's set-up while another cannot)
     return 1;
   if (e->G > 1)
@@ -177,9 +210,12 @@ static int make_handles(Engine *e)
 }
 
 static Engine *engine_new(const std::vector<int> &devices, int npix_max, int mas, bool per_type_maps, size_t particle_capacity, int deposit_mode,
-                          int max_planes, int want_slots, int need_slots, Group *group = nullptr, int gpu0 = 0, int G = 0)
+                          int max_planes, int want_slots, int need_slots, Group *group = nullptr, int gpu0 = 0, int G = 0, int kappa_maps = 0,
+                          int kappa_npix = 0)
 {
   Engine *e = new Engine;
+  e->kappa_maps = kappa_maps;
+  e->kappa_npix = kappa_npix;
   e->devices = devices;
   e->group = group;
   e->gpu0 = gpu0;
@@ -450,9 +486,34 @@ static int finish_group(Engine *e, const InputParams &p, const std::string &File
     return fail_capi("slicer_reduce_all");
   if (e->gpu0 != 0)
     return 0; // the sums are on rank 0
+  if (e->kappa_here())
+  { // the group's planes into the convergence maps, behind the reduce: one launch for all of them
+    const double tk0 = now_s();
+    const int S = e->kappa_nsrc;
+    std::vector<int> map(j1 - j0, 0);
+    std::vector<double> scale((size_t)(j1 - j0) * S, 0.0), offset((size_t)(j1 - j0) * S, 0.0);
+    bool any = false;
+    for (int j = j0; j < j1; j++)
+      if (jobs[j].kappa_map >= 0)
+      {
+        any = true;
+        map[j - j0] = jobs[j].kappa_map;
+        for (int k = 0; k < S; k++)
+        {
+          scale[(size_t)(j - j0) * S + k] = e->kappa_scale[(size_t)jobs[j].isnap * S + k];
+          offset[(size_t)(j - j0) * S + k] = e->kappa_offset[(size_t)jobs[j].isnap * S + k];
+        }
+      }
+    if (any && slicer_kappa_add(e->h[0], 0, j1 - j0, map.data(), S, scale.data(), offset.data()))
+      return fail_capi("slicer_kappa_add");
+    t_kappa += now_s() - tk0;
+    t_kappa_add += now_s() - tk0;
+  }
   const double tf0 = now_s();
   for (int j = j0; j < j1; j++)
   {
+    if (!jobs[j].fetch)
+      continue; // a plane that is not written (convergence maps only, or its file exists)
     const int npix = jobs[j].npix;
     long long counts[6];
     mapxytot[j].resize((size_t)npix * npix);
@@ -600,7 +661,7 @@ static std::string plane_label(int pll)
 // ---- several realisations in one run ---------------------------------------------------------------------------------
 // Realisations of one run share the plan, the engine and every read of a snapshot: their inis must agree on every entry that
 // shapes them.  Checked before anything is read, allocated or written.
-static int check_realisations(const std::vector<std::string> &inis, const std::vector<InputParams> &ps)
+static int check_realisations(const std::vector<std::string> &inis, const std::vector<InputParams> &ps, const std::vector<double> &kappa_zs)
 {
   auto num = [](double v) {
     std::ostringstream o;
@@ -645,7 +706,11 @@ static int check_realisations(const std::vector<std::string> &inis, const std::v
   // no two realisations may write the same file: the planes list (output directory + suffix) or a plane (+ simulation name)
   std::map<std::string, size_t> owner;
   for (size_t k = 0; k < ps.size(); k++)
-    for (const std::string &f : {ps[k].directory + "planes_list_" + ps[k].suffix + ".txt", fileOutput(ps[k], plane_label(0))})
+  {
+    std::vector<std::string> files = {ps[k].directory + "planes_list_" + ps[k].suffix + ".txt", fileOutput(ps[k], plane_label(0))};
+    for (double z : kappa_zs)
+      files.push_back(kappaFileOutput(ps[k], z));
+    for (const std::string &f : files)
     {
       std::error_code ec;
       std::string key = std::filesystem::weakly_canonical(std::filesystem::absolute(f, ec), ec).string();
@@ -659,6 +724,49 @@ static int check_realisations(const std::vector<std::string> &inis, const std::v
         return 1;
       }
     }
+  }
+  return 0;
+}
+
+// Convergence maps are flat-sky Born sums of planes of one size, for sources behind the first plane and within the plan: what
+// cannot be made is refused before anything is read, allocated or written.
+static int check_kappa(const std::string &ini, const InputParams &p, const std::vector<double> &zs, bool write_planes)
+{
+  if (zs.empty())
+  {
+    if (write_planes)
+      return 0;
+    std::cerr << "--no-planes writes convergence maps only: give --kappa or --kappa-zs too" << std::endl;
+    return 1;
+  }
+  if ((int)zs.size() > SLICER_KAPPA_MAX_SOURCES)
+  {
+    std::cerr << "convergence maps: " << zs.size() << " source redshifts, at most " << SLICER_KAPPA_MAX_SOURCES << " per run" << std::endl;
+    return 1;
+  }
+  if (p.physical)
+  {
+    std::cerr << ini << ": entry 1 (map pixels) is negative, physical pixels: convergence maps need planes of one size (give a "
+              << "positive number of pixels)" << std::endl;
+    return 1;
+  }
+  for (size_t k = 0; k < zs.size(); k++)
+  {
+    // (entry 2 is read as a float, as the reference reads it: zs_k is compared at that precision, so that the ini's own value
+    // given as a number, e.g. 0.7 > float(0.7), is accepted)
+    if (!(zs[k] > 0) || (double)(float)zs[k] > p.zs)
+    {
+      std::cerr << "convergence maps: source redshift " << zs[k] << " outside (0, " << p.zs << "]: the planes reach entry 2 (source redshift) "
+                << "of " << ini << ", there are no planes beyond it" << std::endl;
+      return 1;
+    }
+    for (size_t k2 = 0; k2 < k; k2++)
+      if (kappaFileOutput(p, zs[k]) == kappaFileOutput(p, zs[k2]))
+      {
+        std::cerr << "convergence maps: source redshifts " << zs[k2] << " and " << zs[k] << " give one file name (4 decimals)" << std::endl;
+        return 1;
+      }
+  }
   return 0;
 }
 
@@ -668,7 +776,7 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   const bool root = opt.rank == 0;
   const int myid = opt.quiet || !root ? 1 : 0;
   const double t_begin = now_s();
-  t_read = t_submit = t_fetch = t_write = t_engine = t_gpu = 0;
+  t_read = t_submit = t_fetch = t_write = t_engine = t_gpu = t_kappa = t_kappa_add = 0;
   const int K = (int)inifiles.size();
   if (K == 0)
   {
@@ -707,7 +815,13 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
       return 1;
     }
   }
-  if (check_realisations(inifiles, ps))
+  // convergence maps: the source redshifts (NaN: the ini's), S of them
+  std::vector<double> kzs = opt.kappa_zs;
+  for (double &z : kzs)
+    if (std::isnan(z))
+      z = ps[0].zs;
+  const int S = (int)kzs.size();
+  if (check_kappa(inifiles[0], ps[0], kzs, opt.write_planes) || check_realisations(inifiles, ps, kzs))
     return 1;
   // the plan is the same for every realisation: it is made from the first ini
   InputParams &p = ps[0];
@@ -718,6 +832,12 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   Header simdata;
   if (readHeader(p.pathsnap + snappath[0] + ".0", simdata))
     return 1;
+  if (S > 0 && !(fabs(1 - simdata.om0 - simdata.oml) < 1e-5))
+  {
+    std::cerr << "convergence maps: the cosmology of " << p.pathsnap + snappath[0] << ".0 is not flat (Omega_m " << simdata.om0 << ", Omega_Lambda "
+              << simdata.oml << "); the Born weights here use comoving distances, which need a flat one" << std::endl;
+    return 1;
+  }
   CosmoTable cosmo;
   cosmo.build(simdata.om0, simdata.oml, p.w, p.zs);
   for (InputParams &q : ps)
@@ -744,6 +864,9 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     else
       computeReplications(p.fov, boxl, lens.ld2[i], myid, fovradiants, lens.nrepperp[i]);
   }
+  std::vector<double> kscale, koffset;
+  if (S > 0)
+    kappaWeights(lens, cosmo, simdata.om0, simdata.oml, fovradiants, p.npix, kzs, kscale, koffset);
   // one randomisation per realisation; a degrading one last: its draws continue the shared stream its randomizeBox left
   std::vector<Random> randoms(K);
   int degraded = -1;
@@ -773,14 +896,37 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     std::cout << "!It is not possible to resume a Gadget run with partinplanes == true!" << std::endl
               << "!!               Files on Output folder will be overwritten        !!" << std::endl;
   // resume (slicer-v2.cpp:188-196): planes already written are skipped.  Rank 0 alone looks at the output directories and tells
-  // the others, so that every rank makes the same planes whatever its view of a shared file system
-  std::string done((size_t)K * lens.nplanes, '\0');
+  // the others, so that every rank makes the same planes whatever its view of a shared file system.  With convergence maps a
+  // realisation is skipped when all its maps exist; otherwise every plane of it is deposited (a map sums them all), and only the
+  // plane files and maps that do not exist yet are written.
+  const size_t KN = (size_t)K * lens.nplanes;
+  // done[KN] (not deposited), exists[KN] (plane file present), kappa_exists[K * S] (map file present)
+  std::string state(2 * KN + (size_t)K * S, '\0');
   if (root && !p.partinplanes)
     for (int k = 0; k < K; k++)
+    {
+      bool all = S > 0;
+      for (int s = 0; s < S; s++)
+      {
+        const bool there = (bool)std::ifstream(kappaFileOutput(ps[k], kzs[s]));
+        state[2 * KN + (size_t)k * S + s] = there;
+        all = all && there;
+      }
       for (int isnap = 0; isnap < lens.nplanes; isnap++)
-        done[(size_t)k * lens.nplanes + isnap] = std::ifstream(fileOutput(ps[k], plane_label(lens.pll[isnap]))) ? 1 : 0;
-  if (group.bcast(done))
+      {
+        const bool exists = (bool)std::ifstream(fileOutput(ps[k], plane_label(lens.pll[isnap])));
+        state[KN + (size_t)k * lens.nplanes + isnap] = exists;
+        state[(size_t)k * lens.nplanes + isnap] = S > 0 ? all : exists;
+      }
+    }
+  if (group.bcast(state))
     return 1;
+  const char *done = state.data(), *exists = state.data() + KN, *kappa_exists = state.data() + 2 * KN;
+  if (myid == 0)
+    for (int k = 0; k < K; k++)
+      for (int s = 0; s < S; s++)
+        if (kappa_exists[(size_t)k * S + s])
+          std::cout << kappaFileOutput(ps[k], kzs[s]) << " Already exists" << std::endl;
 
   Engine *e = nullptr;
   int status = 0;
@@ -810,13 +956,15 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     for (int k = 0; k < K; k++)
       for (int isnap = s0; isnap < s1; isnap++)
       {
+        const bool present = exists[(size_t)k * lens.nplanes + isnap];
+        if (present && myid == 0)
+          std::cout << fileOutput(ps[k], plane_label(lens.pll[isnap])) << " Already exists" << std::endl;
         if (done[(size_t)k * lens.nplanes + isnap])
-        { // resume: this plane was already written
-          if (myid == 0)
-            std::cout << fileOutput(ps[k], plane_label(lens.pll[isnap])) << " Already exists" << std::endl;
-          continue;
-        }
-        (k == degraded ? djobs : jobs).push_back({isnap, rcase[isnap], npix[isnap], &randoms[k]});
+          continue; // resume: this plane was already written (or all the realisation's convergence maps were)
+        PlaneJob job{isnap, rcase[isnap], npix[isnap], &randoms[k]};
+        job.fetch = opt.write_planes && !present;
+        job.kappa_map = S > 0 ? k * S : -1;
+        (k == degraded ? djobs : jobs).push_back(job);
         if (k != degraded)
           owner.push_back(k);
       }
@@ -857,13 +1005,17 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
             need = std::min(need, want);
           want = std::max(want, need);
         }
-        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need, &group, gpu0, G);
+        // the convergence maps (K x S on the job's GPU 0) are allocated before the slots are sized from the free memory
+        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need, &group, gpu0, G, K * S, p.npix);
         t_engine += now_s() - te0;
         if (!e)
         {
           status = 1;
           break;
         }
+        e->kappa_nsrc = S;
+        e->kappa_scale = kscale;
+        e->kappa_offset = koffset;
       }
       std::vector<std::valarray<float>> tot, per;
       std::vector<long long> cnt;
@@ -927,6 +1079,8 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
         auto write_some = [&]() {
           for (size_t j; !failed && (j = next++) < batch->jobs.size();)
           {
+            if (!batch->jobs[j].fetch)
+              continue; // not written: convergence maps only, or the file exists
             const int isnap = batch->jobs[j].isnap;
             InputParams pj = ps[batch->owner[j]];
             pj.npix = batch->jobs[j].npix;
@@ -958,6 +1112,49 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     s0 = s1;
   }
   join_writer();
+  // the convergence maps, on rank 0 after the last snapshot: rounded once to float
+  if (!status && root && S > 0 && e)
+  {
+    const double tk0 = now_s();
+    std::vector<double> kmap((size_t)p.npix * p.npix);
+    std::vector<float> fmap(kmap.size());
+    for (int k = 0; k < K && !status; k++)
+      for (int s = 0; s < S && !status; s++)
+      {
+        if (kappa_exists[(size_t)k * S + s])
+          continue; // resume: this map was written before (its light cone may have been deposited again for another map)
+        if (slicer_kappa_fetch(e->h[0], k * S + s, kmap.data()))
+        {
+          status = fail_capi("slicer_kappa_fetch");
+          break;
+        }
+        for (size_t i = 0; i < kmap.size(); i++)
+          fmap[i] = (float)kmap[i];
+        long long nplanes = 0;
+        for (int isnap = 0; isnap < lens.nplanes; isnap++)
+          nplanes += kscale[(size_t)isnap * S + s] != 0 || koffset[(size_t)isnap * S + s] != 0;
+        const std::string f = kappaFileOutput(ps[k], kzs[s]);
+        if (myid == 0)
+          std::cout << "Saving the convergence map on: " << f << std::endl;
+        try
+        {
+          writeFitsImage(f, fmap.data(), p.npix,
+                         {{"ZSOURCE", kzs[s]},
+                          {"DS", cosmo.getDl.eval(kzs[s]) / simdata.h},
+                          {"PHYSICALSIZE", p.fov},
+                          {"HUBBLE", simdata.h},
+                          {"OMEGAMATTER", simdata.om0},
+                          {"OMEGALAMBDA", simdata.oml}},
+                         {{"NPLANES", nplanes}}, {"ZSOURCE", "DS", "PHYSICALSIZE", "NPLANES", "HUBBLE", "OMEGAMATTER", "OMEGALAMBDA"});
+        }
+        catch (const SliceError &err)
+        {
+          std::cerr << "It was not possible to create the convergence map: " << err.what << std::endl;
+          status = 1;
+        }
+      }
+    t_kappa += now_s() - tk0;
+  }
   // every rank of a job ends with the same status: one that failed leaves the job, the others learn it here at the latest
   if (status)
     group.close();
@@ -966,7 +1163,8 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   engineDestroy(e);
   if (getenv("SLICER_B200_TIMING"))
     std::cerr << "[timing] " << (opt.nranks > 1 ? "rank " + std::to_string(opt.rank) + ": " : "") << "total " << now_s() - t_begin << " s: engine/CUDA set-up " << t_engine << ", sub-file reads " << t_read << ", fetch (waits for the GPU) " << t_fetch
-              << ", FITS writes (background thread) " << t_write << ", device passes " << t_gpu << " (" << K << " light cone" << (K > 1 ? "s" : "") << ")"
+               << ", FITS writes (background thread) " << t_write << ", device passes " << t_gpu << ", convergence maps " << t_kappa << " (adds " << t_kappa_add << ", read-out and writes " << t_kappa - t_kappa_add << ")"
+              << " (" << K << " light cone" << (K > 1 ? "s" : "") << ")"
               << std::endl;
   return status;
 }

@@ -2,6 +2,7 @@
 #include "slicer_host.h"
 
 #include <chrono>
+#include <cmath>
 #include <cstring>
 
 using namespace slicer;
@@ -220,6 +221,65 @@ extern "C"
     o.quiet = true;
     o.max_slots = max_slots;
     return runLightCones(std::vector<std::string>(inis, inis + nini), o);
+  }
+
+  // the same with convergence maps: nzs source redshifts (NaN: the ini's), write_planes = 0 for the maps only
+  int shost_run_light_cones_kappa(const char **inis, int nini, const int *devices, int ndev, int replication, int fixed_vertex, int ngp,
+                                  int deposit_mode, int max_slots, int rank, int nranks, const char *master_addr, int master_port, const double *zs,
+                                  int nzs, int write_planes)
+  {
+    RunOptions o;
+    o.rank = rank;
+    o.nranks = nranks;
+    o.master_addr = master_addr ? master_addr : "";
+    o.master_port = master_port;
+    o.devices.assign(devices, devices + ndev);
+    o.replication = replication != 0;
+    o.fixed_vertex = fixed_vertex != 0;
+    o.mas = ngp ? SLICER_MAS_NGP : SLICER_MAS_TSC;
+    o.deposit_mode = deposit_mode;
+    o.quiet = true;
+    o.max_slots = max_slots;
+    o.kappa_zs.assign(zs, zs + nzs);
+    o.write_planes = write_planes != 0;
+    return runLightCones(std::vector<std::string>(inis, inis + nini), o);
+  }
+
+  // Born weights of the plan of (om0, oml, w, zs) on caller-supplied snapshots (as shost_plan) for nsrc source redshifts:
+  // scale / offset [plane * nsrc + k], and per plane its edges ld, ld2 and z = getZl((ld + ld2) / 2), per source chi_s = getDl(zs_k)
+  int shost_kappa_weights(double om0, double oml, double w, double zs, int nsnaps, const double *snapred_in, const double *snapbox_in,
+                          double fov_deg, int npix, int nsrc, const double *zs_list, int cap, int *nplanes, double *scale, double *offset, double *ld,
+                          double *ld2, double *zl, double *chis)
+  {
+    CosmoTable c;
+    c.build(om0, oml, w, zs);
+    InputParams p;
+    p.zs = zs;
+    p.Ds = c.getDl.eval(p.zs);
+    std::vector<double> snapred(snapred_in, snapred_in + nsnaps), snapbox(snapbox_in, snapbox_in + nsnaps);
+    std::vector<std::string> snappath;
+    for (int i = 0; i < nsnaps; i++)
+      snappath.push_back("snap_" + std::to_string(i));
+    Lens lens;
+    if (buildPlanes(p, lens, snapred, snappath, snapbox, c.getDl, c.getZl, numberOfLensPerSnap, 1))
+      return 1;
+    *nplanes = lens.nplanes;
+    if (lens.nplanes > cap) // (scale and offset hold cap * nsrc values)
+      return 2;
+    const double fovradiants = fov_deg / 180. * M_PI; // testFov
+    std::vector<double> sc, of;
+    kappaWeights(lens, c, om0, oml, fovradiants, npix, std::vector<double>(zs_list, zs_list + nsrc), sc, of);
+    std::copy(sc.begin(), sc.end(), scale);
+    std::copy(of.begin(), of.end(), offset);
+    for (int i = 0; i < lens.nplanes; i++)
+    {
+      ld[i] = lens.ld[i];
+      ld2[i] = lens.ld2[i];
+      zl[i] = c.getZl.eval((lens.ld[i] + lens.ld2[i]) / 2.0);
+    }
+    for (int k = 0; k < nsrc; k++)
+      chis[k] = c.getDl.eval(zs_list[k]);
+    return 0;
   }
 
   // launchFromEnv over `n` "NAME=value" strings instead of the process environment; out: rank, nranks, local rank, port and the

@@ -8,11 +8,15 @@
 //   --fixed-vertex     CMake USE_FIXED_PLC_VERTEX (-DFixedPLCVertex, CMakeLists.txt:23-26)
 //   --ngp              `#define DO_NGP true`   (densitymaps.h:22)
 //   --max-slots N      at most N plane accumulators per GPU (device memory; default: what the inis' planes of a snapshot need)
+//   --kappa            also write a convergence map per light cone for the ini's source redshift (entry 2), formed on the GPU
+//   --kappa-zs z1,z2,..  the same for up to 8 source redshifts in (0, entry 2] (implies --kappa)
+//   --no-planes        write the convergence maps only (and planes_list), no plane FITS files
 // Started by a launcher (mpirun -np N, srun, torchrun), the processes form one job: rank and world size come from the launcher's
 // environment (slicer::launchFromEnv), MASTER_ADDR / MASTER_PORT name where rank 0 listens for the others, the sub-files of every
 // snapshot are dealt over the GPUs of all ranks and rank 0 writes the planes.
 #include "slicer_host.h"
 
+#include <cmath>
 #include <cstdlib>
 #include <cstring>
 #include <iostream>
@@ -31,7 +35,7 @@ int main(int argc, char **argv)
   opt.nranks = launch.nranks;
   opt.master_addr = launch.master_addr;
   opt.master_port = launch.master_port;
-  bool gpus_given = false;
+  bool gpus_given = false, kappa_ini = false;
   std::vector<std::string> inis;
   for (int i = 1; i < argc; i++)
   {
@@ -52,14 +56,37 @@ int main(int argc, char **argv)
       opt.quiet = true;
     else if (!strcmp(argv[i], "--max-slots") && i + 1 < argc)
       opt.max_slots = atoi(argv[++i]);
+    else if (!strcmp(argv[i], "--kappa"))
+      kappa_ini = true;
+    else if (!strcmp(argv[i], "--kappa-zs") && i + 1 < argc)
+    {
+      for (char *t = strtok(argv[++i], ","); t; t = strtok(nullptr, ","))
+      {
+        char *end = nullptr;
+        const double z = strtod(t, &end);
+        if (end == t || *end)
+        {
+          std::cerr << "--kappa-zs: '" << t << "' is not a number" << std::endl;
+          return 1;
+        }
+        opt.kappa_zs.push_back(z);
+      }
+    }
+    else if (!strcmp(argv[i], "--no-planes"))
+      opt.write_planes = false;
     else
       inis.push_back(argv[i]);
   }
+  if (kappa_ini && opt.kappa_zs.empty())
+    opt.kappa_zs.push_back(std::nan("")); // the ini's source redshift
   if (inis.empty())
   {
-    std::cerr << "usage: SLICER_b200 [--gpus 0,1,..] [--replication] [--fixed-vertex] [--ngp] [--quiet] [--max-slots N] InputParams.ini [more.ini ...]\n"
+    std::cerr << "usage: SLICER_b200 [--gpus 0,1,..] [--replication] [--fixed-vertex] [--ngp] [--quiet] [--max-slots N] [--kappa | --kappa-zs z1,z2,..]\n"
+                 "                   [--no-planes] InputParams.ini [more.ini ...]\n"
                  "  one light cone per ini; the inis must agree on everything but the seeds (entries 7-9), the simulation name and\n"
-                 "  the output directory and suffix (entries 6, 11, 12), and at most one may set a particle degradation"
+                 "  the output directory and suffix (entries 6, 11, 12), and at most one may set a particle degradation.\n"
+                 "  --kappa writes a convergence map per light cone for the source redshift of entry 2 (--kappa-zs: for up to 8 others),\n"
+                 "  --no-planes only those maps"
               << std::endl;
     return 1;
   }

@@ -299,6 +299,34 @@ void CosmoTable::build(double om0, double oml, double w, double zs)
   getZl.init(dl, zl);
 }
 
+void kappaWeights(const Lens &lens, const CosmoTable &cosmo, double om0, double, double fovradiants, int npix, const std::vector<double> &zs,
+                  std::vector<double> &scale, std::vector<double> &offset)
+{
+  const size_t S = zs.size();
+  scale.assign((size_t)lens.nplanes * S, 0.0);
+  offset.assign((size_t)lens.nplanes * S, 0.0);
+  const double A = 1.5 / (speedcunit * speedcunit);
+  const double pix = fovradiants / npix, omega_pix = pix * pix; // flat sky: the cos(dec) of the (dec, ra) pixels is left out
+  for (int i = 0; i < lens.nplanes; i++)
+  {
+    const double ld = lens.ld[i], ld2 = lens.ld2[i];
+    const double chi = (ld + ld2) / 2.0;
+    const double z = cosmo.getZl.eval(chi);
+    // comoving depth of the cone segment per unit solid angle over chi^2: makes the mean term exact (ld2 - ld is 33 % off on the
+    // first plane)
+    const double V = (ld2 * ld2 * ld2 - ld * ld * ld) / (3.0 * chi * chi);
+    for (size_t k = 0; k < S; k++)
+    {
+      const double chis = cosmo.getDl.eval(zs[k]);
+      if (!(chi < chis))
+        continue;
+      const double g = (1.0 + z) * chi * (chis - chi) / chis;
+      scale[i * S + k] = A * g / (rho_crit * omega_pix * chi * chi);
+      offset[i * S + k] = -(A * om0 * g * V);
+    }
+  }
+}
+
 // The snapshot whose comoving distance is nearest to dlens (densitymaps.cpp:9-32); the first one wins ties.  The reference
 // narrows the separation to FLOAT before comparing, which decides near-ties: kept.
 int getSnap(const std::vector<double> &zsnap, const CubicSpline &getDl, double dlens)

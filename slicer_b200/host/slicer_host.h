@@ -137,6 +137,16 @@ void randomizeBox(Random &random, const Lens &lens, const InputParams &p, int nu
 int testFov(double fov, double boxl, double Ds, int myid, double &fovradiants);
 void computeReplications(double fov, double boxl, double Ds, int myid, double &fovradiants, int &nrepperp);
 
+// ---- convergence maps ----------------------------------------------------------------------------------------
+// Flat-sky, thin-plane Born weights of every plane of `lens` for each source redshift zs[k] (comoving Mpc/h, masses in the planes'
+// unit of 1e10 Msun/h).  For plane i: chi = (ld + ld2) / 2, z = getZl(chi), V = (ld2^3 - ld^3) / (3 chi^2),
+// g = (1 + z) chi (chi_s - chi) / chi_s with chi_s = getDl(zs[k]); for chi < chi_s
+//   scale[i*S + k] = A g / (rho_c Omega_pix chi^2),   offset[i*S + k] = -A om0 g V,   A = 1.5 / speedcunit^2, Omega_pix = (fov / npix)^2,
+// and 0, 0 (the plane does not contribute) otherwise.  slicer_kappa_add applies them to the int64 planes.
+constexpr double rho_crit = 27.753662724817193; // 3 (100 km/s/Mpc)^2 / (8 pi G), G = 4.30091727e-9 Mpc (km/s)^2 / Msun: 1e10 Msun/h per (Mpc/h)^3
+void kappaWeights(const Lens &lens, const CosmoTable &cosmo, double om0, double oml, double fovradiants, int npix, const std::vector<double> &zs,
+                  std::vector<double> &scale, std::vector<double> &offset);
+
 // ---- snapshot sub-files ------------------------------------------------------------------------------------
 struct SubFile
 {
@@ -179,6 +189,8 @@ struct PlaneJob
   double rcase;
   int npix;
   const Random *random = nullptr;
+  bool fetch = true;  // read the maps and counts back (mapxytot / mapxytoti / ntotxyi); false: neither (the plane is not written)
+  int kappa_map = -1; // first of the convergence maps this plane adds to (slicer_kappa_add; -1: none)
 };
 int createDensityMapsMulti(Engine *e, InputParams &p, Lens &lens, Random &random, const std::vector<PlaneJob> &jobs, unsigned ffmin,
                            unsigned ffmax, const std::string &File, double fovradiants, std::vector<std::valarray<float>> &mapxytot,
@@ -187,6 +199,7 @@ int createDensityMapsMulti(Engine *e, InputParams &p, Lens &lens, Random &random
 
 // ---- output --------------------------------------------------------------------------------------------------
 std::string fileOutput(const InputParams &p, const std::string &snappl, int label = 0);
+std::string kappaFileOutput(const InputParams &p, double zs); // <dir><sim>.kappa_<snpix>_zs<%.4f>_<suffix>.fits
 // FITS primary image (BITPIX -32, NAXIS1 = NAXIS2 = npix, pixel [gx + npix*gy], big-endian) + the reference's keys.
 // Throws SliceError if the file exists or cannot be created (CCfits FITS::CantCreate).
 void writeFitsImage(const std::string &file, const float *map, int npix, const std::vector<std::pair<std::string, double>> &dkeys,
@@ -268,6 +281,10 @@ struct RunOptions
   std::string master_addr;
   int master_port = 0;
   double connect_timeout_s = 300;
+  // Convergence maps: one per realisation and source redshift (at most SLICER_KAPPA_MAX_SOURCES), formed on the GPU from the
+  // planes; empty = none.  An entry that is NaN stands for the ini's source redshift (entry 2).
+  std::vector<double> kappa_zs;
+  bool write_planes = true; // false: convergence maps only (planes_list is still written)
 };
 // One light cone per ini.  The inis must agree on what shapes the plan and the engine (map pixels, source redshift, field of
 // view, w, snapshot list and directory, one map per particle type); seeds, simulation name, output directory and suffix may
