@@ -25,6 +25,7 @@ LAYOUT_AOS, LAYOUT_SOA = 0, 1
 KERNEL_AUTO, KERNEL_SIMPLE, KERNEL_PIPELINED = 0, 1, 2
 DEPOSIT_AUTO, DEPOSIT_DIRECT, DEPOSIT_BINNED = 0, 1, 2
 KAPPA_MAX_SOURCES = 8
+SHEAR_MAX_FFT = 32768
 
 
 class SlicerError(RuntimeError):
@@ -92,6 +93,7 @@ EXPORTS = [
     "slicer_selftest_arith", "slicer_selftest_packed", "slicer_deposit_slots", "slicer_reduce_slots", "slicer_reduce_all_slots",
     "slicer_stage_synthetic_window", "slicer_settle_slots", "slicer_device_memory", "slicer_comm_init_ranks",
     "slicer_kernels_run", "slicer_kappa_maps", "slicer_kappa_add", "slicer_kappa_fetch", "slicer_kappa_load",
+    "slicer_shear", "slicer_shear_fetch",
 ]
 
 
@@ -160,6 +162,8 @@ def lib() -> C.CDLL:
     L.slicer_kappa_add.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
     L.slicer_kappa_fetch.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
     L.slicer_kappa_load.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    L.slicer_shear.argtypes = [C.c_void_p, C.c_int, C.c_int]
+    L.slicer_shear_fetch.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     _lib = L
     return L
 
@@ -407,6 +411,18 @@ class Slicer:
         if v.size != n * n:
             raise ValueError("one value per pixel")
         _check(lib().slicer_kappa_load(self.h, int(m), v.ctypes.data))
+
+    # -- shear maps -------------------------------------------------------------------------------
+    def shear(self, m: int, fft_size: int):
+        """Enqueue the Kaiser–Squires shear of convergence map `m` on an fft_size^2 grid (a power of two >= npix).  Asynchronous."""
+        _check(lib().slicer_shear(self.h, int(m), int(fft_size)))
+
+    def shear_fetch(self):
+        """-> (g1, g2) of the last shear(): float64 [npix, npix] indexed [gy, gx]"""
+        n = getattr(self, "_kappa_npix", self.cfg.npix_max)
+        g1, g2 = np.empty(n * n, np.float64), np.empty(n * n, np.float64)
+        _check(lib().slicer_shear_fetch(self.h, g1.ctypes.data, g2.ctypes.data))
+        return g1.reshape(n, n), g2.reshape(n, n)
 
     def reset_stats(self):
         _check(lib().slicer_reset_stats(self.h))

@@ -21,6 +21,7 @@
 #include "deposit_pipelined.cuh"
 #include "deposit_degrade.cuh"
 #include "kappa.cuh"
+#include "shear.cuh"
 
 #define POS_U 1.0 /* gadget2io.h:14 */
 
@@ -154,6 +155,15 @@ struct slicer_handle
     int n = 0, npix = 0;
     size_t stride = 0;
   } kappa;
+  // shear maps (slicer_shear*): two P x P ping-pong workspaces, the twiddle table and γ1, γ2 of the last slicer_shear
+  struct
+  {
+    double2 *buf[2] = {nullptr, nullptr};
+    double2 *tw = nullptr; // P entries
+    double *g = nullptr;   // γ1 (npix^2), then γ2
+    int P = 0, npix = 0;
+    int map = -1; // κ map of the last slicer_shear (-1: none yet)
+  } shear;
   double boxsize = 0;
   double massarr[SLICER_NTYPES] = {0, 0, 0, 0, 0, 0};
   int hydro = 0;
@@ -508,6 +518,10 @@ extern "C" void slicer_destroy(slicer_handle *h)
   cudaFree(h->d_sum);
   cudaFree(h->kappa.maps);
   cudaFree(h->kappa.ovf);
+  cudaFree(h->shear.buf[0]);
+  cudaFree(h->shear.buf[1]);
+  cudaFree(h->shear.tw);
+  cudaFree(h->shear.g);
   if (h->ev_copy)
     cudaEventDestroy(h->ev_copy);
   for (int b = 0; b < 2; b++)
@@ -1841,6 +1855,7 @@ extern "C" int slicer_kappa_maps(slicer_handle *h, int nmaps, int npix)
     return fail("slicer_kappa_maps: %d maps of %d^2 (npix must be 1..%d)", nmaps, npix, h->cfg.npix_max);
   if (set_device(h))
     return 1;
+  h->shear.map = -1; // (its γ maps are of maps that go)
   if (h->kappa.maps)
   { // (cudaFree waits for the work that still reads or writes them)
     CU(cudaFree(h->kappa.maps));
@@ -1967,6 +1982,146 @@ extern "C" int slicer_kappa_load(slicer_handle *h, int map, const double *in)
   const size_t npix2 = (size_t)h->kappa.npix * h->kappa.npix;
   CU(cudaMemcpyAsync(h->kappa.maps + (size_t)map * h->kappa.stride, in, npix2 * sizeof(double), cudaMemcpyHostToDevice, h->compute));
   CU(cudaStreamSynchronize(h->compute));
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// shear maps (shear.cuh)
+// ------------------------------------------------------------------------------------------------------------
+static void shear_free(slicer_handle *h)
+{
+  auto &S = h->shear;
+  if (!S.tw)
+    return;
+  cudaFree(S.buf[0]);
+  cudaFree(S.buf[1]);
+  cudaFree(S.tw);
+  cudaFree(S.g);
+  h->device_bytes -= 2 * (size_t)S.P * S.P * sizeof(double2) + (size_t)S.P * sizeof(double2) + 2 * (size_t)S.npix * S.npix * sizeof(double);
+  S = {};
+}
+
+// workspaces for P and γ maps of npix^2: kept while both stay, made again when either changes
+static int shear_workspace(slicer_handle *h, int P, int npix)
+{
+  auto &S = h->shear;
+  if (S.tw && S.P == P && S.npix == npix)
+    return 0;
+  shear_free(h); // (cudaFree waits for the work that still uses them)
+  S.P = P;
+  S.npix = npix;
+  const size_t ws = (size_t)P * P * sizeof(double2), gs = 2 * (size_t)npix * npix * sizeof(double), ts = (size_t)P * sizeof(double2);
+  if (dev_alloc(h, &S.buf[0], (size_t)P * P) || dev_alloc(h, &S.buf[1], (size_t)P * P) || dev_alloc(h, &S.g, 2 * (size_t)npix * npix) ||
+      dev_alloc(h, &S.tw, (size_t)P))
+  {
+    const std::string err = g_err;
+    h->device_bytes -= (S.buf[0] ? ws : 0) + (S.buf[1] ? ws : 0) + (S.g ? gs : 0); // (the table is allocated last)
+    cudaFree(S.buf[0]);
+    cudaFree(S.buf[1]);
+    cudaFree(S.g);
+    S = {};
+    return fail("slicer_shear: workspace for FFT size %d (%.3g GB): %s", P, (2 * ws + gs + ts) / 1e9, err.c_str());
+  }
+  // the table, from the host's libm in exactly this expression (the restatement evaluates the same one)
+  std::vector<double2> tw(P);
+  for (int k = 0; k < P; k++)
+    tw[k] = make_double2(cos(2.0 * M_PI * k / P), sin(2.0 * M_PI * k / P));
+  CU(cudaMemcpyAsync(S.tw, tw.data(), (size_t)P * sizeof(double2), cudaMemcpyHostToDevice, h->compute));
+  CU(cudaStreamSynchronize(h->compute));
+  return 0;
+}
+
+template <int RA, int RB, bool INV, int AXIS>
+static int shear_launch(slicer_handle *h, ShearArgs &A)
+{
+  const size_t threads = (size_t)A.nlines * (A.P / (RA * RB));
+  shear_fft_pass<RA, RB, INV, AXIS><<<(unsigned)((threads + 255) / 256), 256, 0, h->compute>>>(A);
+  CU(cudaGetLastError());
+  h->stats.launches++;
+  return 0;
+}
+
+// the stages of one axis, two per launch; `first` / `last` flags go to the first / last launch
+template <bool INV, int AXIS>
+static int shear_axis(slicer_handle *h, ShearArgs &A, int nlines, int first, int last, int &cur)
+{
+  const int P = A.P;
+  A.nlines = nlines;
+  for (int n = 1; n < P;)
+  {
+    const int ra = P / n >= 4 ? 4 : 2, rb = P / (n * ra) >= 4 ? 4 : P / (n * ra) >= 2 ? 2 : 1;
+    A.n = n;
+    n *= ra * rb;
+    A.flags = (A.n == 1 ? first : 0) | (n == P ? last : 0);
+    A.src = h->shear.buf[cur];
+    A.dst = h->shear.buf[cur ^ 1];
+    int rc;
+    if (ra == 4 && rb == 4)
+      rc = shear_launch<4, 4, INV, AXIS>(h, A);
+    else if (ra == 4 && rb == 2)
+      rc = shear_launch<4, 2, INV, AXIS>(h, A);
+    else if (ra == 4)
+      rc = shear_launch<4, 1, INV, AXIS>(h, A);
+    else
+      rc = shear_launch<2, 1, INV, AXIS>(h, A);
+    if (rc)
+      return 1;
+    cur ^= 1;
+  }
+  return 0;
+}
+
+extern "C" int slicer_shear(slicer_handle *h, int map, int fft_size)
+{
+  if (!h)
+    return fail("null handle");
+  if (!h->kappa.maps)
+    return fail("slicer_shear: no convergence maps (slicer_kappa_maps)");
+  if (map < 0 || map >= h->kappa.n)
+    return fail("slicer_shear: convergence map %d outside 0..%d", map, h->kappa.n - 1);
+  const int npix = h->kappa.npix, P = fft_size;
+  if (P < 2 || P > SHEAR_MAX_FFT || (P & (P - 1)) || P < npix)
+    return fail("slicer_shear: FFT size %d must be a power of two in [%d, %d] (at least the maps' %d pixels and 2)", P, npix > 2 ? npix : 2,
+                SHEAR_MAX_FFT, npix);
+  if (set_device(h) || shear_workspace(h, P, npix))
+    return 1;
+  ShearArgs A;
+  memset(&A, 0, sizeof(A));
+  A.kappa = h->kappa.maps + (size_t)map * h->kappa.stride;
+  A.tw = h->shear.tw;
+  A.g1 = h->shear.g;
+  A.g2 = h->shear.g + (size_t)npix * npix;
+  A.scale = ldexp(1.0, -2 * ilogb((double)P));
+  A.P = P;
+  A.npix = npix;
+  // forward rows (the npix rows of κ; the others stay 0), forward columns, inverse columns, inverse rows of the window
+  int cur = 0;
+  h->shear.map = -1;
+  if (shear_axis<false, 0>(h, A, npix, SHEAR_IN_KAPPA, 0, cur) || shear_axis<false, 1>(h, A, P, SHEAR_IN_ZERO, SHEAR_OUT_MULT, cur) ||
+      shear_axis<true, 1>(h, A, P, 0, 0, cur) || shear_axis<true, 0>(h, A, npix, 0, SHEAR_OUT_GAMMA, cur))
+    return 1;
+  h->shear.map = map;
+  return 0;
+}
+
+extern "C" int slicer_shear_fetch(slicer_handle *h, double *gamma1, double *gamma2)
+{
+  if (!h || !gamma1 || !gamma2)
+    return fail("slicer_shear_fetch: null argument");
+  const int map = h->shear.map;
+  if (map < 0 || map >= h->kappa.n || h->shear.npix != h->kappa.npix)
+    return fail("slicer_shear_fetch: no shear map (slicer_shear)");
+  if (set_device(h))
+    return 1;
+  const size_t npix2 = (size_t)h->shear.npix * h->shear.npix;
+  unsigned ovf = 0;
+  CU(cudaMemcpyAsync(gamma1, h->shear.g, npix2 * sizeof(double), cudaMemcpyDeviceToHost, h->compute));
+  CU(cudaMemcpyAsync(gamma2, h->shear.g + npix2, npix2 * sizeof(double), cudaMemcpyDeviceToHost, h->compute));
+  CU(cudaMemcpyAsync(&ovf, h->kappa.ovf + map, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
+  CU(cudaStreamSynchronize(h->compute));
+  if (ovf)
+    return fail("shear of convergence map %d: a fixed-point accumulator it summed exceeded 2^63 (more than %.3g mass units in one pixel "
+                "at %d fraction bits); create the handle with a smaller slicer_config.frac_bits", map, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
   return 0;
 }
 

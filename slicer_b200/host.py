@@ -34,7 +34,7 @@ def lib():
         L.shost_run_light_cones.argtypes = [C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                             C.c_int, C.c_char_p, C.c_int]
         L.shost_run_light_cones_kappa.argtypes = ([C.POINTER(C.c_char_p), C.c_int, _i32p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                                   C.c_int, C.c_int, C.c_char_p, C.c_int, _f64p, C.c_int, C.c_int])
+                                                   C.c_int, C.c_int, C.c_char_p, C.c_int, _f64p, C.c_int, C.c_int, C.c_int])
         L.shost_kappa_weights.argtypes = ([C.c_double] * 4 + [C.c_int, _f64p, _f64p, C.c_double, C.c_int, C.c_int, _f64p, C.c_int,
                                                               C.POINTER(C.c_int)] + [_f64p] * 6)
         L.shost_launch_from_env.argtypes = [C.POINTER(C.c_char_p), C.c_int, C.c_int, _i32p, C.c_char_p, C.c_int, C.c_char_p, C.c_int]
@@ -149,7 +149,7 @@ def run_light_cone(ini, devices=(0,), replication=False, fixed_vertex=False, ngp
 
 
 def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, ngp=False, deposit_mode=0, max_slots=0, rank=0, nranks=1,
-                    master=None, kappa_zs=None, write_planes=True):
+                    master=None, kappa_zs=None, write_planes=True, shear=False):
     """One light cone per ini (realisations of one plan: other seeds, other outputs), every snapshot read once for all (once per
     group of planes that fits `max_slots` accumulators per GPU, when given).  Returns 0 on success; inis that disagree on the
     plan are refused before anything is written.
@@ -157,15 +157,16 @@ def run_light_cones(inis, devices=(0,), replication=False, fixed_vertex=False, n
     all make this call with the same arguments but `rank` and `devices`; rank 0 writes the files.  The launcher's environment
     is not read.
     kappa_zs: source redshifts of the convergence maps to write per light cone (None: none; NaN stands for the ini's source
-    redshift); write_planes=False writes those maps only."""
+    redshift); write_planes=False writes those maps only.  shear=True writes the shear maps γ1, γ2 of each convergence map too
+    (with kappa_zs None: of the ini's source redshift)."""
     dev = np.ascontiguousarray(devices, np.int32)
     arr = (C.c_char_p * len(inis))(*[str(i).encode() for i in inis])
     addr, port = (master.rsplit(":", 1) if master else ("", 0))
-    if kappa_zs is not None or not write_planes:
+    if kappa_zs is not None or not write_planes or shear:
         zs = np.ascontiguousarray(list(kappa_zs or []) or [0.0], np.float64)
         return lib().shost_run_light_cones_kappa(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
                                                  int(max_slots), int(rank), int(nranks), addr.encode(), int(port), zs, len(kappa_zs or []),
-                                                 int(bool(write_planes)))
+                                                 int(bool(write_planes)), int(bool(shear)))
     return lib().shost_run_light_cones(arr, len(inis), dev, len(dev), int(replication), int(fixed_vertex), int(ngp), int(deposit_mode),
                                        int(max_slots), int(rank), int(nranks), addr.encode(), int(port))
 

@@ -25,6 +25,7 @@ namespace slicer
 // wall-clock phase totals of the last runLightCones (seconds): printed when SLICER_B200_TIMING is set
 static double t_read = 0, t_submit = 0, t_fetch = 0, t_write = 0, t_engine = 0, t_gpu = 0; // t_gpu: device time of the passes
 static double t_kappa = 0, t_kappa_add = 0; // convergence maps: slicer_kappa_add calls (t_kappa_add) + read-out and writes of the maps
+static double t_shear = 0;                   // shear maps: slicer_shear, read-out and writes
 static double now_s() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 struct Engine
@@ -49,6 +50,7 @@ struct Engine
   // kappa_nsrc sources: [isnap * kappa_nsrc + k]
   int kappa_maps = 0, kappa_npix = 0, kappa_nsrc = 0;
   std::vector<double> kappa_scale, kappa_offset;
+  int shear_fft = 0; // shear maps are formed there too, on grids of shear_fft^2 (0: none)
   bool kappa_here() const { return kappa_maps > 0 && gpu0 == 0; }
 };
 
@@ -71,7 +73,7 @@ static void add_gpu_time(Engine *e)
 // at most the particle capacity), two npix^2 read-out buffers (12 B per pixel) and the deferred-pair banks (2 x 24 B x 2^19 per
 // 16 slots); 512 MiB cover the banks, the kernels' scratch and the context's own allocations.  Checked every time the handles
 // are made, so a rebuild with a larger particle capacity (ensure_capacity) takes fewer slots rather than failing to allocate.
-// `extra0` bytes more are taken on the first device (the convergence maps on the job's GPU 0).
+// `extra0` bytes more are taken on the first device (the convergence maps and the shear workspace on the job's GPU 0).
 static int choose_slots(const std::vector<int> &devices, int want, int need, int npix_max, bool per_type, size_t capacity, size_t extra0, int &slots)
 {
   const size_t per_slot = (size_t)(per_type ? 6 : 1) * npix_max * npix_max * 8;
@@ -121,7 +123,9 @@ static int make_handles(Engine *e)
     slicer_destroy(hh);
   e->h.assign(e->devices.size(), nullptr);
   e->comm = false;
-  const size_t kappa_bytes = e->kappa_here() ? (size_t)e->kappa_maps * ((size_t)e->kappa_npix * e->kappa_npix + 2) * 8 : 0;
+  const size_t kappa_bytes = e->kappa_here() ? (size_t)e->kappa_maps * ((size_t)e->kappa_npix * e->kappa_npix + 2) * 8 +
+                                                  (e->shear_fft ? shearWorkspaceBytes(e->shear_fft, e->kappa_npix) : 0)
+                                            : 0;
   if (e->want_slots > 0 &&
       choose_slots(e->devices, e->want_slots, e->need_slots, e->npix_max, e->per_type, e->capacity, kappa_bytes, e->max_planes))
     return 1;
@@ -211,11 +215,12 @@ static int make_handles(Engine *e)
 
 static Engine *engine_new(const std::vector<int> &devices, int npix_max, int mas, bool per_type_maps, size_t particle_capacity, int deposit_mode,
                           int max_planes, int want_slots, int need_slots, Group *group = nullptr, int gpu0 = 0, int G = 0, int kappa_maps = 0,
-                          int kappa_npix = 0)
+                          int kappa_npix = 0, int shear_fft = 0)
 {
   Engine *e = new Engine;
   e->kappa_maps = kappa_maps;
   e->kappa_npix = kappa_npix;
+  e->shear_fft = shear_fft;
   e->devices = devices;
   e->group = group;
   e->gpu0 = gpu0;
@@ -661,7 +666,8 @@ static std::string plane_label(int pll)
 // ---- several realisations in one run ---------------------------------------------------------------------------------
 // Realisations of one run share the plan, the engine and every read of a snapshot: their inis must agree on every entry that
 // shapes them.  Checked before anything is read, allocated or written.
-static int check_realisations(const std::vector<std::string> &inis, const std::vector<InputParams> &ps, const std::vector<double> &kappa_zs)
+static int check_realisations(const std::vector<std::string> &inis, const std::vector<InputParams> &ps, const std::vector<double> &kappa_zs,
+                              bool shear)
 {
   auto num = [](double v) {
     std::ostringstream o;
@@ -709,7 +715,11 @@ static int check_realisations(const std::vector<std::string> &inis, const std::v
   {
     std::vector<std::string> files = {ps[k].directory + "planes_list_" + ps[k].suffix + ".txt", fileOutput(ps[k], plane_label(0))};
     for (double z : kappa_zs)
+    {
       files.push_back(kappaFileOutput(ps[k], z));
+      if (shear)
+        files.push_back(kappaFileOutput(ps[k], z, "gamma1"));
+    }
     for (const std::string &f : files)
     {
       std::error_code ec;
@@ -730,7 +740,7 @@ static int check_realisations(const std::vector<std::string> &inis, const std::v
 
 // Convergence maps are flat-sky Born sums of planes of one size, for sources behind the first plane and within the plan: what
 // cannot be made is refused before anything is read, allocated or written.
-static int check_kappa(const std::string &ini, const InputParams &p, const std::vector<double> &zs, bool write_planes)
+static int check_kappa(const std::string &ini, const InputParams &p, const std::vector<double> &zs, bool write_planes, bool shear)
 {
   if (zs.empty())
   {
@@ -748,6 +758,12 @@ static int check_kappa(const std::string &ini, const InputParams &p, const std::
   {
     std::cerr << ini << ": entry 1 (map pixels) is negative, physical pixels: convergence maps need planes of one size (give a "
               << "positive number of pixels)" << std::endl;
+    return 1;
+  }
+  if (shear && p.npix > SLICER_SHEAR_MAX_FFT / 2)
+  {
+    std::cerr << ini << ": shear maps of " << p.npix << "^2 pixels would need an FFT of " << shearFftSize(p.npix) << "^2, at most "
+              << SLICER_SHEAR_MAX_FFT << "^2 (maps of at most " << SLICER_SHEAR_MAX_FFT / 2 << "^2 pixels)" << std::endl;
     return 1;
   }
   for (size_t k = 0; k < zs.size(); k++)
@@ -776,7 +792,7 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   const bool root = opt.rank == 0;
   const int myid = opt.quiet || !root ? 1 : 0;
   const double t_begin = now_s();
-  t_read = t_submit = t_fetch = t_write = t_engine = t_gpu = t_kappa = t_kappa_add = 0;
+  t_read = t_submit = t_fetch = t_write = t_engine = t_gpu = t_kappa = t_kappa_add = t_shear = 0;
   const int K = (int)inifiles.size();
   if (K == 0)
   {
@@ -817,11 +833,13 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   }
   // convergence maps: the source redshifts (NaN: the ini's), S of them
   std::vector<double> kzs = opt.kappa_zs;
+  if (opt.shear && kzs.empty())
+    kzs.push_back(std::nan("")); // shear maps alone: of the convergence map for the ini's source redshift
   for (double &z : kzs)
     if (std::isnan(z))
       z = ps[0].zs;
   const int S = (int)kzs.size();
-  if (check_kappa(inifiles[0], ps[0], kzs, opt.write_planes) || check_realisations(inifiles, ps, kzs))
+  if (check_kappa(inifiles[0], ps[0], kzs, opt.write_planes, opt.shear) || check_realisations(inifiles, ps, kzs, opt.shear))
     return 1;
   // the plan is the same for every realisation: it is made from the first ini
   InputParams &p = ps[0];
@@ -837,6 +855,21 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     std::cerr << "convergence maps: the cosmology of " << p.pathsnap + snappath[0] << ".0 is not flat (Omega_m " << simdata.om0 << ", Omega_Lambda "
               << simdata.oml << "); the Born weights here use comoving distances, which need a flat one" << std::endl;
     return 1;
+  }
+  // shear maps: formed on the job's GPU 0 on grids of shear_fft^2; its workspace must fit there beside the convergence maps
+  const int shear_fft = opt.shear ? shearFftSize(ps[0].npix) : 0;
+  if (shear_fft && gpu0 == 0)
+  {
+    const size_t need = shearWorkspaceBytes(shear_fft, ps[0].npix) + (size_t)K * S * ((size_t)ps[0].npix * ps[0].npix + 2) * 8;
+    size_t free_b = 0, total_b = 0;
+    if (slicer_device_memory(opt.devices[0], &free_b, &total_b))
+      return fail_capi("slicer_device_memory");
+    if (need > free_b)
+    {
+      std::cerr << "shear maps: the FFT workspace (" << shear_fft << "^2) and " << K * S << " convergence maps need " << need / double(1 << 30)
+                << " GiB on GPU " << opt.devices[0] << ", which has " << free_b / double(1 << 30) << " GiB free" << std::endl;
+      return 1;
+    }
   }
   CosmoTable cosmo;
   cosmo.build(simdata.om0, simdata.oml, p.w, p.zs);
@@ -900,18 +933,22 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   // realisation is skipped when all its maps exist; otherwise every plane of it is deposited (a map sums them all), and only the
   // plane files and maps that do not exist yet are written.
   const size_t KN = (size_t)K * lens.nplanes;
-  // done[KN] (not deposited), exists[KN] (plane file present), kappa_exists[K * S] (map file present)
-  std::string state(2 * KN + (size_t)K * S, '\0');
+  // done[KN] (not deposited), exists[KN] (plane file present), kappa_exists[K * S * F] (map file present: κ, and with shear maps
+  // γ1 and γ2, [(k * S + s) * F + f])
+  const int F = opt.shear ? 3 : 1;
+  static const char *const map_kind[3] = {"kappa", "gamma1", "gamma2"};
+  std::string state(2 * KN + (size_t)K * S * F, '\0');
   if (root && !p.partinplanes)
     for (int k = 0; k < K; k++)
     {
       bool all = S > 0;
       for (int s = 0; s < S; s++)
-      {
-        const bool there = (bool)std::ifstream(kappaFileOutput(ps[k], kzs[s]));
-        state[2 * KN + (size_t)k * S + s] = there;
-        all = all && there;
-      }
+        for (int f = 0; f < F; f++)
+        {
+          const bool there = (bool)std::ifstream(kappaFileOutput(ps[k], kzs[s], map_kind[f]));
+          state[2 * KN + ((size_t)k * S + s) * F + f] = there;
+          all = all && there;
+        }
       for (int isnap = 0; isnap < lens.nplanes; isnap++)
       {
         const bool exists = (bool)std::ifstream(fileOutput(ps[k], plane_label(lens.pll[isnap])));
@@ -925,8 +962,9 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   if (myid == 0)
     for (int k = 0; k < K; k++)
       for (int s = 0; s < S; s++)
-        if (kappa_exists[(size_t)k * S + s])
-          std::cout << kappaFileOutput(ps[k], kzs[s]) << " Already exists" << std::endl;
+        for (int f = 0; f < F; f++)
+          if (kappa_exists[((size_t)k * S + s) * F + f])
+            std::cout << kappaFileOutput(ps[k], kzs[s], map_kind[f]) << " Already exists" << std::endl;
 
   Engine *e = nullptr;
   int status = 0;
@@ -1006,7 +1044,8 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
           want = std::max(want, need);
         }
         // the convergence maps (K x S on the job's GPU 0) are allocated before the slots are sized from the free memory
-        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need, &group, gpu0, G, K * S, p.npix);
+        e = engine_new(opt.devices, npix_max, opt.mas, p.partinplanes, cap, opt.deposit_mode, want, want, need, &group, gpu0, G, K * S, p.npix,
+                       shear_fft);
         t_engine += now_s() - te0;
         if (!e)
         {
@@ -1118,42 +1157,68 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
     const double tk0 = now_s();
     std::vector<double> kmap((size_t)p.npix * p.npix);
     std::vector<float> fmap(kmap.size());
+    std::vector<double> g1(F > 1 ? kmap.size() : 0), g2(g1.size());
     for (int k = 0; k < K && !status; k++)
       for (int s = 0; s < S && !status; s++)
       {
-        if (kappa_exists[(size_t)k * S + s])
-          continue; // resume: this map was written before (its light cone may have been deposited again for another map)
-        if (slicer_kappa_fetch(e->h[0], k * S + s, kmap.data()))
-        {
-          status = fail_capi("slicer_kappa_fetch");
-          break;
-        }
-        for (size_t i = 0; i < kmap.size(); i++)
-          fmap[i] = (float)kmap[i];
         long long nplanes = 0;
         for (int isnap = 0; isnap < lens.nplanes; isnap++)
           nplanes += kscale[(size_t)isnap * S + s] != 0 || koffset[(size_t)isnap * S + s] != 0;
-        const std::string f = kappaFileOutput(ps[k], kzs[s]);
-        if (myid == 0)
-          std::cout << "Saving the convergence map on: " << f << std::endl;
-        try
+        const char *there = kappa_exists + ((size_t)k * S + s) * F;
+        // (a map file written before is kept: its light cone may have been deposited again for another one)
+        auto write = [&](int f, const std::vector<double> &map, const char *what) {
+          for (size_t i = 0; i < map.size(); i++)
+            fmap[i] = (float)map[i];
+          const std::string fn = kappaFileOutput(ps[k], kzs[s], map_kind[f]);
+          if (myid == 0)
+            std::cout << "Saving the " << what << " on: " << fn << std::endl;
+          std::vector<std::pair<std::string, double>> dkeys = {{"ZSOURCE", kzs[s]},
+                                                               {"DS", cosmo.getDl.eval(kzs[s]) / simdata.h},
+                                                               {"PHYSICALSIZE", p.fov},
+                                                               {"HUBBLE", simdata.h},
+                                                               {"OMEGAMATTER", simdata.om0},
+                                                               {"OMEGALAMBDA", simdata.oml}};
+          std::vector<std::pair<std::string, long long>> ikeys = {{"NPLANES", nplanes}};
+          std::vector<std::string> order = {"ZSOURCE", "DS", "PHYSICALSIZE", "NPLANES", "HUBBLE", "OMEGAMATTER", "OMEGALAMBDA"};
+          if (f > 0)
+          {
+            ikeys.push_back({"FFTSIZE", shear_fft});
+            order.push_back("FFTSIZE");
+          }
+          try
+          {
+            writeFitsImage(fn, fmap.data(), p.npix, dkeys, ikeys, order);
+          }
+          catch (const SliceError &err)
+          {
+            std::cerr << "It was not possible to create the " << what << ": " << err.what << std::endl;
+            status = 1;
+          }
+        };
+        if (!there[0])
         {
-          writeFitsImage(f, fmap.data(), p.npix,
-                         {{"ZSOURCE", kzs[s]},
-                          {"DS", cosmo.getDl.eval(kzs[s]) / simdata.h},
-                          {"PHYSICALSIZE", p.fov},
-                          {"HUBBLE", simdata.h},
-                          {"OMEGAMATTER", simdata.om0},
-                          {"OMEGALAMBDA", simdata.oml}},
-                         {{"NPLANES", nplanes}}, {"ZSOURCE", "DS", "PHYSICALSIZE", "NPLANES", "HUBBLE", "OMEGAMATTER", "OMEGALAMBDA"});
+          if (slicer_kappa_fetch(e->h[0], k * S + s, kmap.data()))
+          {
+            status = fail_capi("slicer_kappa_fetch");
+            break;
+          }
+          write(0, kmap, "convergence map");
         }
-        catch (const SliceError &err)
+        if (F == 1 || status || (there[1] && there[2]))
+          continue;
+        const double ts0 = now_s();
+        if (slicer_shear(e->h[0], k * S + s, shear_fft) || slicer_shear_fetch(e->h[0], g1.data(), g2.data()))
         {
-          std::cerr << "It was not possible to create the convergence map: " << err.what << std::endl;
-          status = 1;
+          status = fail_capi("slicer_shear");
+          break;
         }
+        if (!there[1])
+          write(1, g1, "shear map");
+        if (!there[2] && !status)
+          write(2, g2, "shear map");
+        t_shear += now_s() - ts0;
       }
-    t_kappa += now_s() - tk0;
+    t_kappa += now_s() - tk0 - t_shear;
   }
   // every rank of a job ends with the same status: one that failed leaves the job, the others learn it here at the latest
   if (status)
@@ -1164,6 +1229,7 @@ int runLightCones(const std::vector<std::string> &inifiles, const RunOptions &op
   if (getenv("SLICER_B200_TIMING"))
     std::cerr << "[timing] " << (opt.nranks > 1 ? "rank " + std::to_string(opt.rank) + ": " : "") << "total " << now_s() - t_begin << " s: engine/CUDA set-up " << t_engine << ", sub-file reads " << t_read << ", fetch (waits for the GPU) " << t_fetch
                << ", FITS writes (background thread) " << t_write << ", device passes " << t_gpu << ", convergence maps " << t_kappa << " (adds " << t_kappa_add << ", read-out and writes " << t_kappa - t_kappa_add << ")"
+              << (opt.shear ? ", shear maps " + std::to_string(t_shear) : std::string())
               << " (" << K << " light cone" << (K > 1 ? "s" : "") << ")"
               << std::endl;
   return status;

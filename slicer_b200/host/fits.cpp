@@ -25,11 +25,11 @@ std::string fileOutput(const InputParams &p, const std::string &snappl, int labe
   throw SliceError{"Output name format not recognized"};
 }
 
-std::string kappaFileOutput(const InputParams &p, double zs)
+std::string kappaFileOutput(const InputParams &p, double zs, const char *map)
 {
   char z[64];
   snprintf(z, sizeof(z), "%.4f", zs);
-  return p.directory + p.simulation + ".kappa_" + p.snpix + "_zs" + z + "_" + p.suffix + ".fits";
+  return p.directory + p.simulation + "." + map + "_" + p.snpix + "_zs" + z + "_" + p.suffix + ".fits";
 }
 
 static void card(std::string &hdr, const std::string &text)

@@ -223,10 +223,11 @@ extern "C"
     return runLightCones(std::vector<std::string>(inis, inis + nini), o);
   }
 
-  // the same with convergence maps: nzs source redshifts (NaN: the ini's), write_planes = 0 for the maps only
+  // the same with convergence maps: nzs source redshifts (NaN: the ini's), write_planes = 0 for the maps only, shear = 1 for their
+  // shear maps too
   int shost_run_light_cones_kappa(const char **inis, int nini, const int *devices, int ndev, int replication, int fixed_vertex, int ngp,
                                   int deposit_mode, int max_slots, int rank, int nranks, const char *master_addr, int master_port, const double *zs,
-                                  int nzs, int write_planes)
+                                  int nzs, int write_planes, int shear)
   {
     RunOptions o;
     o.rank = rank;
@@ -242,6 +243,7 @@ extern "C"
     o.max_slots = max_slots;
     o.kappa_zs.assign(zs, zs + nzs);
     o.write_planes = write_planes != 0;
+    o.shear = shear != 0;
     return runLightCones(std::vector<std::string>(inis, inis + nini), o);
   }
 

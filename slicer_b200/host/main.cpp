@@ -11,6 +11,7 @@
 //   --kappa            also write a convergence map per light cone for the ini's source redshift (entry 2), formed on the GPU
 //   --kappa-zs z1,z2,..  the same for up to 8 source redshifts in (0, entry 2] (implies --kappa)
 //   --no-planes        write the convergence maps only (and planes_list), no plane FITS files
+//   --shear            also write the shear maps γ1, γ2 of every convergence map (Kaiser–Squires on the GPU; alone: implies --kappa)
 // Started by a launcher (mpirun -np N, srun, torchrun), the processes form one job: rank and world size come from the launcher's
 // environment (slicer::launchFromEnv), MASTER_ADDR / MASTER_PORT name where rank 0 listens for the others, the sub-files of every
 // snapshot are dealt over the GPUs of all ranks and rank 0 writes the planes.
@@ -74,6 +75,8 @@ int main(int argc, char **argv)
     }
     else if (!strcmp(argv[i], "--no-planes"))
       opt.write_planes = false;
+    else if (!strcmp(argv[i], "--shear"))
+      opt.shear = true;
     else
       inis.push_back(argv[i]);
   }
@@ -82,11 +85,12 @@ int main(int argc, char **argv)
   if (inis.empty())
   {
     std::cerr << "usage: SLICER_b200 [--gpus 0,1,..] [--replication] [--fixed-vertex] [--ngp] [--quiet] [--max-slots N] [--kappa | --kappa-zs z1,z2,..]\n"
-                 "                   [--no-planes] InputParams.ini [more.ini ...]\n"
+                 "                   [--shear] [--no-planes] InputParams.ini [more.ini ...]\n"
                  "  one light cone per ini; the inis must agree on everything but the seeds (entries 7-9), the simulation name and\n"
                  "  the output directory and suffix (entries 6, 11, 12), and at most one may set a particle degradation.\n"
                  "  --kappa writes a convergence map per light cone for the source redshift of entry 2 (--kappa-zs: for up to 8 others),\n"
-                 "  --no-planes only those maps"
+                 "  --shear also the shear maps gamma1, gamma2 of each (alone: of the source redshift of entry 2), --no-planes only\n"
+                 "  those maps"
               << std::endl;
     return 1;
   }

@@ -147,6 +147,19 @@ constexpr double rho_crit = 27.753662724817193; // 3 (100 km/s/Mpc)^2 / (8 pi G)
 void kappaWeights(const Lens &lens, const CosmoTable &cosmo, double om0, double oml, double fovradiants, int npix, const std::vector<double> &zs,
                   std::vector<double> &scale, std::vector<double> &offset);
 
+// ---- shear maps -----------------------------------------------------------------------------------------------
+// Kaiser–Squires γ1, γ2 of each convergence map (slicer_shear, csrc/shear.cuh) on a zero-padded grid of P^2: the smallest power of
+// two >= 2 npix, so that mass near one edge does not wrap onto the other.  The device workspace that takes: two P^2 grids of
+// complex doubles, the P-entry twiddle table and the two npix^2 double maps.
+inline int shearFftSize(int npix)
+{
+  int P = 1;
+  while (P < 2 * npix)
+    P *= 2;
+  return P;
+}
+inline size_t shearWorkspaceBytes(int P, int npix) { return 2 * 16 * (size_t)P * P + 16 * (size_t)P + 16 * (size_t)npix * npix; }
+
 // ---- snapshot sub-files ------------------------------------------------------------------------------------
 struct SubFile
 {
@@ -199,7 +212,8 @@ int createDensityMapsMulti(Engine *e, InputParams &p, Lens &lens, Random &random
 
 // ---- output --------------------------------------------------------------------------------------------------
 std::string fileOutput(const InputParams &p, const std::string &snappl, int label = 0);
-std::string kappaFileOutput(const InputParams &p, double zs); // <dir><sim>.kappa_<snpix>_zs<%.4f>_<suffix>.fits
+// <dir><sim>.<map>_<snpix>_zs<%.4f>_<suffix>.fits, map = kappa, gamma1 or gamma2
+std::string kappaFileOutput(const InputParams &p, double zs, const char *map = "kappa");
 // FITS primary image (BITPIX -32, NAXIS1 = NAXIS2 = npix, pixel [gx + npix*gy], big-endian) + the reference's keys.
 // Throws SliceError if the file exists or cannot be created (CCfits FITS::CantCreate).
 void writeFitsImage(const std::string &file, const float *map, int npix, const std::vector<std::pair<std::string, double>> &dkeys,
@@ -285,6 +299,8 @@ struct RunOptions
   // planes; empty = none.  An entry that is NaN stands for the ini's source redshift (entry 2).
   std::vector<double> kappa_zs;
   bool write_planes = true; // false: convergence maps only (planes_list is still written)
+  // Shear maps γ1, γ2 of every convergence map (a run with none makes the one of the ini's source redshift), formed on the GPU
+  bool shear = false;
 };
 // One light cone per ini.  The inis must agree on what shapes the plan and the engine (map pixels, source redshift, field of
 // view, w, snapshot list and directory, one map per particle type); seeds, simulation name, output directory and suffix may
