@@ -11,7 +11,9 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <memory>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/slicer_b200.h"
@@ -39,15 +41,124 @@ static int fail(const char *fmt, ...)
   return 1;
 }
 
+// The failure branch clears the thread's last error: a refused call (an allocation too large, say) must not fail the next launch
+// check of this thread, on this handle or another.
 #define CU(expr)                                                                                   \
   do                                                                                               \
   {                                                                                                \
     cudaError_t _e = (expr);                                                                       \
     if (_e != cudaSuccess)                                                                         \
+    {                                                                                              \
+      cudaGetLastError();                                                                          \
       return fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, __LINE__);     \
+    }                                                                                              \
   } while (0)
 
 extern "C" const char *slicer_last_error(void) { return g_err; }
+
+// ------------------------------------------------------------------------------------------------------------
+// owned CUDA resources: move-only; each takes what the call that made it returned, and releases it when it is destroyed or
+// assigned over
+// ------------------------------------------------------------------------------------------------------------
+// n device elements of T, counted in *counter (the handle's device_bytes) while they are held
+template <typename T>
+class DevArray
+{
+  T *p_ = nullptr;
+  size_t n_ = 0;
+  size_t *counter_ = nullptr;
+
+public:
+  DevArray() = default;
+  DevArray(T *p, size_t n, size_t *counter) : p_(p), n_(n), counter_(counter) { *counter_ += n * sizeof(T); }
+  DevArray(DevArray &&o) noexcept { *this = std::move(o); }
+  DevArray &operator=(DevArray &&o) noexcept
+  {
+    if (this != &o)
+    {
+      reset();
+      std::swap(p_, o.p_);
+      std::swap(n_, o.n_);
+      std::swap(counter_, o.counter_);
+    }
+    return *this;
+  }
+  ~DevArray() { reset(); }
+  void reset()
+  {
+    if (p_)
+    {
+      cudaFree(p_);
+      *counter_ -= n_ * sizeof(T);
+    }
+    p_ = nullptr;
+    n_ = 0;
+  }
+  size_t size() const { return n_; }
+  T *get() const { return p_; }
+  operator T *() const { return p_; }
+};
+
+// a stream, an event or a pinned host block
+template <typename H, cudaError_t (*Release)(H)>
+class Owned
+{
+  H h_ = nullptr;
+
+public:
+  Owned() = default;
+  explicit Owned(H h) : h_(h) {}
+  Owned(Owned &&o) noexcept { *this = std::move(o); }
+  Owned &operator=(Owned &&o) noexcept
+  {
+    if (this != &o)
+    {
+      reset();
+      std::swap(h_, o.h_);
+    }
+    return *this;
+  }
+  ~Owned() { reset(); }
+  void reset()
+  {
+    if (h_)
+      Release(h_);
+    h_ = nullptr;
+  }
+  H get() const { return h_; }
+  operator H() const { return h_; }
+};
+template <typename T>
+cudaError_t free_host(T *p) { return cudaFreeHost(p); }
+using Stream = Owned<cudaStream_t, cudaStreamDestroy>;
+using Event = Owned<cudaEvent_t, cudaEventDestroy>;
+template <typename T>
+using Pinned = Owned<T *, free_host<T>>;
+
+template <typename T>
+static int host_alloc(Pinned<T> &a, size_t n)
+{
+  void *p = nullptr;
+  CU(cudaHostAlloc(&p, n * sizeof(T), cudaHostAllocDefault));
+  a = Pinned<T>((T *)p);
+  return 0;
+}
+
+static int make_stream(Stream &s)
+{
+  cudaStream_t r = nullptr;
+  CU(cudaStreamCreateWithFlags(&r, cudaStreamNonBlocking));
+  s = Stream(r);
+  return 0;
+}
+
+static int make_event(Event &e, unsigned flags)
+{
+  cudaEvent_t r = nullptr;
+  CU(cudaEventCreateWithFlags(&r, flags));
+  e = Event(r);
+  return 0;
+}
 
 // ------------------------------------------------------------------------------------------------------------
 // NCCL, loaded lazily so that single-GPU use has no dependency on it
@@ -123,55 +234,55 @@ struct slicer_handle
   int ntypes_alloc;
   size_t npix2max;
   int sm_count;
-  cudaStream_t compute = nullptr, copy = nullptr, comm_stream = nullptr;
-  cudaStream_t aux = nullptr;                      // zeroing of large accumulators, concurrent with the record kernel of a binned pass
-  cudaEvent_t ev_zero_start = nullptr, ev_zero_done = nullptr;
-  bool zero_pending = false;                       // the compute stream has not yet waited for ev_zero_done
-  cudaEvent_t ev_pass_done = nullptr;              // compute -> comm_stream: the passes a reduce sums
-  cudaEvent_t ev_slot[SLICER_MAX_SLOTS];           // comm_stream -> compute: the last reduce of accumulator slot q
-  bool slot_reducing[SLICER_MAX_SLOTS];            // ev_slot[q] is pending
-  cudaEvent_t ev_copy = nullptr;
-  cudaEvent_t ev_buf_done[2] = {nullptr, nullptr}; // last pass that read staging pool b
-  cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;    // slicer_timer_*
-  std::vector<cudaEvent_t> pass_ev;                // ring of (start, stop) pairs, resolved lazily
-  size_t pass_head = 0, pass_tail = 0;             // pairs [tail, head) are pending
+  size_t device_bytes = 0; // what the DevArray members below hold (declared before them: they count in it until they go)
+  Stream compute, copy, comm_stream;
+  Stream aux;                                // zeroing of large accumulators, concurrent with the record kernel of a binned pass
+  Event ev_zero_start, ev_zero_done;
+  bool zero_pending = false;                 // the compute stream has not yet waited for ev_zero_done
+  Event ev_pass_done;                        // compute -> comm_stream: the passes a reduce sums
+  Event ev_slot[SLICER_MAX_SLOTS];           // comm_stream -> compute: the last reduce of accumulator slot q (q < max_planes)
+  bool slot_reducing[SLICER_MAX_SLOTS] = {}; // ev_slot[q] is pending
+  Event ev_copy;
+  Event ev_buf_done[2];                      // last pass that read staging pool b
+  Event ev_t0, ev_t1;                        // slicer_timer_*
+  std::vector<Event> pass_ev;                // ring of (start, stop) pairs, resolved lazily
+  size_t pass_head = 0, pass_tail = 0;       // pairs [tail, head) are pending
   int nbuf = 1, cur_buf = 0;
-  float *d_pos_pool = nullptr;  // nbuf * (particle_capacity * 3 + 64) floats
-  float *d_mass_pool = nullptr; // nbuf * (mass_capacity + 64) floats
+  DevArray<float> d_pos_pool;  // nbuf * (particle_capacity * 3 + 64) floats
+  DevArray<float> d_mass_pool; // nbuf * (mass_capacity + 64) floats
   float *d_pos = nullptr;  // current pool
   float *d_mass = nullptr;
   size_t pos_used = 0;     // in particles
   size_t mass_used = 0;
   std::vector<Segment> segs;
-  unsigned long long *d_acc = nullptr;    // [max_planes][ntypes_alloc][npix2max]
-  unsigned long long *d_counts = nullptr; // [max_planes][6][2]
-  float *d_out = nullptr;                 // npix2max
-  long long *d_sum = nullptr;             // npix2max
+  DevArray<unsigned long long> d_acc;    // [max_planes][ntypes_alloc][npix2max]
+  DevArray<unsigned long long> d_counts; // [max_planes][6][2]
+  DevArray<float> d_out;                 // npix2max
+  DevArray<long long> d_sum;             // npix2max
   // convergence maps (slicer_kappa_*): kappa.n maps of kappa.npix^2 doubles, each starting kappa.stride doubles after the last
   struct
   {
-    double *maps = nullptr;
-    unsigned *ovf = nullptr; // one flag per map
+    DevArray<double> maps;
+    DevArray<unsigned> ovf; // one flag per map
     int n = 0, npix = 0;
     size_t stride = 0;
   } kappa;
   // shear maps (slicer_shear*): two P x P ping-pong workspaces, the twiddle table and γ1, γ2 of the last slicer_shear
   struct
   {
-    double2 *buf[2] = {nullptr, nullptr};
-    double2 *tw = nullptr; // P entries
-    double *g = nullptr;   // γ1 (npix^2), then γ2
+    DevArray<double2> buf[2];
+    DevArray<double2> tw; // P entries
+    DevArray<double> g;   // γ1 (npix^2), then γ2
     int P = 0, npix = 0;
     int map = -1; // κ map of the last slicer_shear (-1: none yet)
   } shear;
   double boxsize = 0;
   double massarr[SLICER_NTYPES] = {0, 0, 0, 0, 0, 0};
   int hydro = 0;
-  int plane_npix[SLICER_MAX_SLOTS];
+  int plane_npix[SLICER_MAX_SLOTS] = {};
   bool copy_pending = false;
-  slicer_stats stats;
+  slicer_stats stats = {};
   unsigned long long kernels_run = 0; // slicer_kernels_run: bit i = pipelined_table() entry i, bit 40 + mas = deposit_simple_kernel
-  size_t device_bytes = 0;
   ncclComm_t comm = nullptr;
   int nranks = 1, rank = 0;
   int grid_max = 0; // CTAs of a persistent pipelined-kernel grid (pipelined_init)
@@ -187,13 +298,13 @@ struct slicer_handle
   // Which bank a new set takes: run_pass.
   struct DeferBank
   {
-    DeferEntry *buf = nullptr;
-    unsigned *count = nullptr;      // device: entries appended since the bank was last settled
-    DeferEntry *host = nullptr;     // pinned mirror
-    unsigned *host_count = nullptr; // pinned: the counter as of the end of the bank's last pass (copied behind every pass)
-    std::vector<SavedPass> passes;  // passes since the last settle; DeferEntry::pass indexes it
-    cudaEvent_t ev_done = nullptr;  // behind the bank's last pass and the copies of its counter / list head
-    uint64_t slot_mask = 0;         // accumulator slots the bank's passes deposit into (bit q: slot q)
+    DevArray<DeferEntry> buf;
+    DevArray<unsigned> count;      // device: entries appended since the bank was last settled
+    Pinned<DeferEntry> host;       // pinned mirror
+    Pinned<unsigned> host_count;   // pinned: the counter as of the end of the bank's last pass (copied behind every pass)
+    std::vector<SavedPass> passes; // passes since the last settle; DeferEntry::pass indexes it
+    Event ev_done;                 // behind the bank's last pass and the copies of its counter / list head
+    uint64_t slot_mask = 0;        // accumulator slots the bank's passes deposit into (bit q: slot q)
   };
   struct
   {
@@ -202,13 +313,13 @@ struct slicer_handle
     unsigned cap = 0;
     bool failed = false;
   } defer;
-  unsigned *d_ovf = nullptr;        // device flag: an accumulator ran past 2^63 (raised at read-out)
-  cudaStream_t settle = nullptr;    // deposits of the pairs libm settled, beside the passes running on `compute`
-  cudaEvent_t ev_settled = nullptr; // settle -> compute / comm_stream
+  DevArray<unsigned> d_ovf;         // device flag: an accumulator ran past 2^63 (raised at read-out)
+  Stream settle;                    // deposits of the pairs libm settled, beside the passes running on `compute`
+  Event ev_settled;                 // settle -> compute / comm_stream
   bool settle_pending = false;      // `compute` has not yet waited for ev_settled
   bool settle_pending_comm = false; // nor has `comm_stream`
-  cudaEvent_t slot_pass_ev[SLICER_MAX_SLOTS]; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
-  unsigned long long slot_epoch[SLICER_MAX_SLOTS];
+  cudaEvent_t slot_pass_ev[SLICER_MAX_SLOTS] = {}; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
+  unsigned long long slot_epoch[SLICER_MAX_SLOTS] = {};
   size_t pos_stride = 0, mass_stride = 0; // floats per staging pool (16-byte multiples)
   size_t pcap = 0, mcap = 0;              // particles / masses a pool holds, padding of the segments included
   // particles per slice the binned path will use (before allocation: what it would allocate)
@@ -222,22 +333,25 @@ struct slicer_handle
   // binned deposit (deposit_binned.cuh): buffers allocated on first use
   struct
   {
-    float2 *rec_u = nullptr, *rec_s = nullptr;
-    unsigned short *key_u = nullptr;
-    float *mass_u = nullptr, *mass_s = nullptr;
-    unsigned *region_count = nullptr, *region_hist = nullptr, *bin_count = nullptr, *bin_start = nullptr;
-    size_t slice = 0;    // particles per slice
+    DevArray<float2> rec_u, rec_s;
+    DevArray<unsigned short> key_u;
+    DevArray<float> mass_u, mass_s;
+    DevArray<unsigned> region_count, region_hist, bin_count, bin_start;
+    size_t slice = 0;    // particles per slice (0: no buffers yet)
     size_t capacity = 0; // records the buffers hold
   } bin;
   // Part. Degradation (deposit_degrade.cuh): per-particle accepted counts and ranks of the resident batch
   struct
   {
-    unsigned char *cnt = nullptr, *keep = nullptr;
-    unsigned *rank = nullptr, *block_sums = nullptr;
-    size_t stride = 0, nblocks = 0, keep_cap = 0;
-    size_t bytes = 0; // device bytes of cnt, rank and block_sums
-    int nplanes = 0;
-    bool valid = false;
+    struct // per plane: cnt a row of stride, rank of stride + 1, block_sums of nblocks
+    {
+      DevArray<unsigned char> cnt;
+      DevArray<unsigned> rank, block_sums;
+      size_t stride = 0, nblocks = 0;
+      int nplanes = 0;
+    } scratch;
+    DevArray<unsigned char> keep;
+    int counted = 0; // planes slicer_count_accepted counted for the resident batch (plane_total); 0: none
     unsigned long long plane_total[SLICER_MAX_PLANES];
   } deg;
 };
@@ -268,7 +382,10 @@ extern "C" int slicer_device_memory(int device, size_t *free_bytes, size_t *tota
   const cudaError_t e = cudaMemGetInfo(free_bytes, total_bytes);
   cudaSetDevice(prev);
   if (e != cudaSuccess)
+  {
+    cudaGetLastError();
     return fail("cudaMemGetInfo failed: %s", cudaGetErrorString(e));
+  }
   return 0;
 }
 
@@ -284,12 +401,14 @@ extern "C" int slicer_free_pinned(void *p)
   return 0;
 }
 
+// Releases what `a` held before it allocates, so that a workspace made again never holds both sets; on failure `a` stays empty.
 template <typename T>
-static int dev_alloc(slicer_handle *h, T **p, size_t count)
+static int dev_alloc(slicer_handle *h, DevArray<T> &a, size_t count)
 {
-  size_t bytes = count * sizeof(T);
-  CU(cudaMalloc((void **)p, bytes));
-  h->device_bytes += bytes;
+  a.reset();
+  void *p = nullptr;
+  CU(cudaMalloc(&p, count * sizeof(T)));
+  a = DevArray<T>((T *)p, count, &h->device_bytes);
   return 0;
 }
 
@@ -305,255 +424,109 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
     return fail("slicer_create: unknown mass-assignment scheme %d", cfg->mas);
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
+  if (e != cudaSuccess)
+    cudaGetLastError();
   if (e != cudaSuccess || ndev == 0)
     return fail("slicer_create: no usable CUDA device (%s); this library has no CPU path",
                 e == cudaSuccess ? "device count is 0" : cudaGetErrorString(e));
   if (cfg->device < 0 || cfg->device >= ndev)
     return fail("slicer_create: device %d out of range (have %d)", cfg->device, ndev);
-  slicer_handle *h = new slicer_handle;
-  for (int q = 0; q < SLICER_MAX_SLOTS; q++)
-  {
-    h->ev_slot[q] = nullptr;
-    h->slot_reducing[q] = false;
-    h->slot_pass_ev[q] = nullptr;
-  }
+  std::unique_ptr<slicer_handle> owner(new slicer_handle); // on any failure below, what was made so far goes with it
+  slicer_handle *h = owner.get();
   h->cfg = *cfg;
   h->frac_bits = cfg->frac_bits > 0 ? cfg->frac_bits : 40;
   if (h->frac_bits > 60)
-  {
-    delete h;
     return fail("slicer_create: frac_bits must be <= 60");
-  }
   if (h->cfg.max_m <= 0)
     h->cfg.max_m = 1e3; /* densitymaps.h:21 */
   h->ntypes_alloc = cfg->per_type_maps ? SLICER_NTYPES : 1;
   h->npix2max = (size_t)cfg->npix_max * (size_t)cfg->npix_max;
-  memset(&h->stats, 0, sizeof(h->stats));
-  memset(h->plane_npix, 0, sizeof(h->plane_npix));
-  int rc = 0;
   // SLICER_B200_TIMING: wall-clock of the set-up phases on stderr (context, allocations, kernel set-up)
   const bool timing = getenv("SLICER_B200_TIMING") != nullptr;
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   const double t_start = now();
-  double t_ctx = 0, t_alloc = 0;
-  do
+  if (set_device(h)) // (cudaSetDevice makes the device's context: the phases are attributed correctly)
+    return 1;
+  const double t_ctx = now();
+  cudaDeviceProp prop;
+  CU(cudaGetDeviceProperties(&prop, cfg->device));
+  if (prop.major < 10)
+    return fail("slicer_create: device %d is sm_%d%d; this library is built for sm_100a (B200) only", cfg->device, prop.major,
+                prop.minor);
+  h->sm_count = prop.multiProcessorCount;
+  for (Stream *s : {&h->compute, &h->copy, &h->comm_stream, &h->aux, &h->settle})
+    if (make_stream(*s))
+      return 1;
+  for (Event *ev : {&h->ev_settled, &h->defer.bank[0].ev_done, &h->defer.bank[1].ev_done, &h->ev_zero_start, &h->ev_zero_done,
+                    &h->ev_pass_done, &h->ev_copy, &h->ev_buf_done[0], &h->ev_buf_done[1]})
+    if (make_event(*ev, cudaEventDisableTiming))
+      return 1;
+  for (int q = 0; q < cfg->max_planes; q++)
+    if (make_event(h->ev_slot[q], cudaEventDisableTiming))
+      return 1;
+  h->pass_ev.resize(2 * PASS_RING);
+  for (Event *ev : {&h->ev_t0, &h->ev_t1})
+    if (make_event(*ev, cudaEventDefault))
+      return 1;
+  for (Event &ev : h->pass_ev)
+    if (make_event(ev, cudaEventDefault))
+      return 1;
+  h->nbuf = cfg->staging_buffers >= 2 ? 2 : 1;
+  // +64 floats of slack so 16-byte bulk copies may over-read the tail of the last chunk; every pool starts on a 16-byte
+  // boundary whatever the capacity (cp.async.bulk needs 16-byte aligned sources)
+  // (internal capacities: the caller's, rounded up to a multiple of 4, plus room for the 16-byte padding of up to 8 segments)
+  h->pcap = cfg->particle_capacity ? ((cfg->particle_capacity + 3) & ~(size_t)3) + 32 : 0;
+  h->mcap = cfg->mass_capacity ? ((cfg->mass_capacity + 3) & ~(size_t)3) + 32 : 0;
+  h->pos_stride = h->pcap * 3 + 64;
+  h->mass_stride = h->mcap + 64;
+  if (cfg->particle_capacity && dev_alloc(h, h->d_pos_pool, h->nbuf * h->pos_stride))
+    return 1;
+  if (cfg->mass_capacity && dev_alloc(h, h->d_mass_pool, h->nbuf * h->mass_stride))
+    return 1;
+  // 2^19 entries (12 MiB) per bank and per 16 slots: one bank may hold the passes of every slot range (run_pass), and the
+  // flagged pairs (about 8 per million accepted pairs at the default guard) grow with the planes deposited between settles
+  h->defer.cap = (1u << 19) * (unsigned)((cfg->max_planes + SLICER_MAX_PLANES - 1) / SLICER_MAX_PLANES);
+  if (dev_alloc(h, h->d_ovf, 1))
+    return 1;
+  for (slicer_handle::DeferBank &B : h->defer.bank)
   {
-    if ((rc = set_device(h)))
-      break;
-    if (timing)
-      cudaFree(nullptr); // force the context now, so that the phases are attributed correctly
-    t_ctx = now();
-    cudaDeviceProp prop;
-    if (cudaGetDeviceProperties(&prop, cfg->device) != cudaSuccess)
-    {
-      rc = fail("cudaGetDeviceProperties failed");
-      break;
-    }
-    if (prop.major < 10)
-    {
-      rc = fail("slicer_create: device %d is sm_%d%d; this library is built for sm_100a (B200) only", cfg->device,
-                prop.major, prop.minor);
-      break;
-    }
-    h->sm_count = prop.multiProcessorCount;
-#define TRY(expr)                                                        \
-  if ((expr) != cudaSuccess)                                             \
-  {                                                                      \
-    rc = fail("%s failed: %s", #expr, cudaGetErrorString(cudaGetLastError())); \
-    break;                                                               \
+    if (dev_alloc(h, B.buf, (size_t)h->defer.cap) || dev_alloc(h, B.count, 1) || host_alloc(B.host, (size_t)h->defer.cap) ||
+        host_alloc(B.host_count, 2))
+      return 1;
+    B.host_count[0] = 0;
   }
-    TRY(cudaStreamCreateWithFlags(&h->compute, cudaStreamNonBlocking));
-    TRY(cudaStreamCreateWithFlags(&h->copy, cudaStreamNonBlocking));
-    TRY(cudaStreamCreateWithFlags(&h->comm_stream, cudaStreamNonBlocking));
-    TRY(cudaStreamCreateWithFlags(&h->aux, cudaStreamNonBlocking));
-    TRY(cudaStreamCreateWithFlags(&h->settle, cudaStreamNonBlocking));
-    TRY(cudaEventCreateWithFlags(&h->ev_settled, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->defer.bank[0].ev_done, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->defer.bank[1].ev_done, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_zero_start, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_zero_done, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_pass_done, cudaEventDisableTiming));
-    for (int q = 0; q < cfg->max_planes; q++)
-      TRY(cudaEventCreateWithFlags(&h->ev_slot[q], cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_copy, cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_buf_done[0], cudaEventDisableTiming));
-    TRY(cudaEventCreateWithFlags(&h->ev_buf_done[1], cudaEventDisableTiming));
-    TRY(cudaEventCreate(&h->ev_t0));
-    TRY(cudaEventCreate(&h->ev_t1));
-    h->pass_ev.resize(2 * PASS_RING, nullptr);
-    {
-      bool bad = false;
-      for (size_t i = 0; i < h->pass_ev.size() && !bad; i++)
-        bad = cudaEventCreate(&h->pass_ev[i]) != cudaSuccess;
-      if (bad)
-      {
-        rc = fail("cudaEventCreate failed: %s", cudaGetErrorString(cudaGetLastError()));
-        break;
-      }
-    }
-#undef TRY
-    h->nbuf = cfg->staging_buffers >= 2 ? 2 : 1;
-    // +64 floats of slack so 16-byte bulk copies may over-read the tail of the last chunk; every pool starts on a 16-byte
-    // boundary whatever the capacity (cp.async.bulk needs 16-byte aligned sources)
-    // (internal capacities: the caller's, rounded up to a multiple of 4, plus room for the 16-byte padding of up to 8 segments)
-    h->pcap = cfg->particle_capacity ? ((cfg->particle_capacity + 3) & ~(size_t)3) + 32 : 0;
-    h->mcap = cfg->mass_capacity ? ((cfg->mass_capacity + 3) & ~(size_t)3) + 32 : 0;
-    h->pos_stride = h->pcap * 3 + 64;
-    h->mass_stride = h->mcap + 64;
-    if (cfg->particle_capacity && (rc = dev_alloc(h, &h->d_pos_pool, h->nbuf * h->pos_stride)))
-      break;
-    if (cfg->mass_capacity && (rc = dev_alloc(h, &h->d_mass_pool, h->nbuf * h->mass_stride)))
-      break;
-    // 2^19 entries (12 MiB) per bank and per 16 slots: one bank may hold the passes of every slot range (run_pass), and the
-    // flagged pairs (about 8 per million accepted pairs at the default guard) grow with the planes deposited between settles
-    h->defer.cap = (1u << 19) * (unsigned)((cfg->max_planes + SLICER_MAX_PLANES - 1) / SLICER_MAX_PLANES);
-    if ((rc = dev_alloc(h, &h->d_ovf, 1)))
-      break;
-    for (int b = 0; b < 2 && !rc; b++)
-    {
-      slicer_handle::DeferBank &B = h->defer.bank[b];
-      if ((rc = dev_alloc(h, &B.buf, (size_t)h->defer.cap)) || (rc = dev_alloc(h, &B.count, 1)))
-        break;
-      if (cudaHostAlloc((void **)&B.host, (size_t)h->defer.cap * sizeof(DeferEntry), cudaHostAllocDefault) != cudaSuccess ||
-          cudaHostAlloc((void **)&B.host_count, 2 * sizeof(unsigned), cudaHostAllocDefault) != cudaSuccess)
-      {
-        rc = fail("cudaHostAlloc failed: %s", cudaGetErrorString(cudaGetLastError()));
-        break;
-      }
-      B.host_count[0] = 0;
-    }
-    if (rc)
-      break;
-    memset(h->slot_epoch, 0, sizeof(h->slot_epoch));
-    h->d_pos = h->d_pos_pool;
-    h->d_mass = h->d_mass_pool;
-    if ((rc = dev_alloc(h, &h->d_acc, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max)))
-      break;
-    if ((rc = dev_alloc(h, &h->d_counts, (size_t)cfg->max_planes * SLICER_NTYPES * 2)))
-      break;
-    if ((rc = dev_alloc(h, &h->d_out, h->npix2max)))
-      break;
-    if ((rc = dev_alloc(h, &h->d_sum, h->npix2max)))
-      break;
-    t_alloc = now();
-    if ((rc = pipelined_init(h->sm_count, &h->grid_max)))
-    {
-      rc = fail("pipelined kernel set-up failed: %s", cudaGetErrorString(cudaGetLastError()));
-      break;
-    }
-    if (cudaMemsetAsync(h->d_acc, 0, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max * 8, h->compute) != cudaSuccess ||
-        cudaMemsetAsync(h->d_counts, 0, (size_t)cfg->max_planes * SLICER_NTYPES * 2 * 8, h->compute) != cudaSuccess ||
-        cudaMemsetAsync(h->defer.bank[0].count, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
-        cudaMemsetAsync(h->defer.bank[1].count, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
-        cudaMemsetAsync(h->d_ovf, 0, sizeof(unsigned), h->compute) != cudaSuccess ||
-        cudaStreamSynchronize(h->compute) != cudaSuccess)
-    {
-      rc = fail("initial memset failed: %s", cudaGetErrorString(cudaGetLastError()));
-      break;
-    }
-    if (timing)
-      fprintf(stderr, "[timing] slicer_create(device %d): context %.3f s, streams + device allocations %.3f s, kernel set-up %.3f s\n", cfg->device,
-              t_ctx - t_start, t_alloc - t_ctx, now() - t_alloc);
-  } while (0);
-  if (rc)
-  {
-    slicer_destroy(h);
-    return rc;
-  }
-  *out = h;
+  h->d_pos = h->d_pos_pool;
+  h->d_mass = h->d_mass_pool;
+  if (dev_alloc(h, h->d_acc, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max) ||
+      dev_alloc(h, h->d_counts, (size_t)cfg->max_planes * SLICER_NTYPES * 2) || dev_alloc(h, h->d_out, h->npix2max) ||
+      dev_alloc(h, h->d_sum, h->npix2max))
+    return 1;
+  const double t_alloc = now();
+  if (pipelined_init(h->sm_count, &h->grid_max))
+    return fail("pipelined kernel set-up failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CU(cudaMemsetAsync(h->d_acc, 0, (size_t)cfg->max_planes * h->ntypes_alloc * h->npix2max * 8, h->compute));
+  CU(cudaMemsetAsync(h->d_counts, 0, (size_t)cfg->max_planes * SLICER_NTYPES * 2 * 8, h->compute));
+  CU(cudaMemsetAsync(h->defer.bank[0].count, 0, sizeof(unsigned), h->compute));
+  CU(cudaMemsetAsync(h->defer.bank[1].count, 0, sizeof(unsigned), h->compute));
+  CU(cudaMemsetAsync(h->d_ovf, 0, sizeof(unsigned), h->compute));
+  CU(cudaStreamSynchronize(h->compute));
+  if (timing)
+    fprintf(stderr, "[timing] slicer_create(device %d): context %.3f s, streams + device allocations %.3f s, kernel set-up %.3f s\n", cfg->device,
+            t_ctx - t_start, t_alloc - t_ctx, now() - t_alloc);
+  *out = owner.release();
   return 0;
 }
 
+// waits for the handle's work; its members release what they own
 extern "C" void slicer_destroy(slicer_handle *h)
 {
   if (!h)
     return;
   cudaSetDevice(h->cfg.device);
-  if (h->compute)
-    cudaStreamSynchronize(h->compute);
-  if (h->copy)
-    cudaStreamSynchronize(h->copy);
-  if (h->comm_stream)
-    cudaStreamSynchronize(h->comm_stream);
+  for (const Stream *s : {&h->compute, &h->copy, &h->comm_stream, &h->aux, &h->settle})
+    cudaStreamSynchronize(*s);
   if (h->comm && g_nccl.CommDestroy)
     g_nccl.CommDestroy(h->comm);
-  cudaFree(h->deg.cnt);
-  cudaFree(h->deg.keep);
-  cudaFree(h->deg.rank);
-  cudaFree(h->deg.block_sums);
-  cudaFree(h->bin.rec_u);
-  cudaFree(h->bin.rec_s);
-  cudaFree(h->bin.key_u);
-  cudaFree(h->bin.mass_u);
-  cudaFree(h->bin.mass_s);
-  cudaFree(h->bin.region_count);
-  cudaFree(h->bin.bin_count);
-  cudaFree(h->bin.bin_start);
-  cudaFree(h->bin.region_hist);
-  if (h->settle)
-  {
-    cudaStreamSynchronize(h->settle);
-    cudaStreamDestroy(h->settle);
-  }
-  if (h->ev_settled)
-    cudaEventDestroy(h->ev_settled);
-  cudaFree(h->d_ovf);
-  for (int b = 0; b < 2; b++)
-  {
-    slicer_handle::DeferBank &B = h->defer.bank[b];
-    cudaFree(B.buf);
-    cudaFree(B.count);
-    if (B.host)
-      cudaFreeHost(B.host);
-    if (B.host_count)
-      cudaFreeHost(B.host_count);
-    if (B.ev_done)
-      cudaEventDestroy(B.ev_done);
-  }
-  cudaFree(h->d_pos_pool);
-  cudaFree(h->d_mass_pool);
-  cudaFree(h->d_acc);
-  cudaFree(h->d_counts);
-  cudaFree(h->d_out);
-  cudaFree(h->d_sum);
-  cudaFree(h->kappa.maps);
-  cudaFree(h->kappa.ovf);
-  cudaFree(h->shear.buf[0]);
-  cudaFree(h->shear.buf[1]);
-  cudaFree(h->shear.tw);
-  cudaFree(h->shear.g);
-  if (h->ev_copy)
-    cudaEventDestroy(h->ev_copy);
-  for (int b = 0; b < 2; b++)
-    if (h->ev_buf_done[b])
-      cudaEventDestroy(h->ev_buf_done[b]);
-  if (h->ev_t0)
-    cudaEventDestroy(h->ev_t0);
-  if (h->ev_t1)
-    cudaEventDestroy(h->ev_t1);
-  for (size_t i = 0; i < h->pass_ev.size(); i++)
-    if (h->pass_ev[i])
-      cudaEventDestroy(h->pass_ev[i]);
-  if (h->aux)
-  {
-    cudaStreamSynchronize(h->aux);
-    cudaStreamDestroy(h->aux);
-  }
-  if (h->ev_zero_start)
-    cudaEventDestroy(h->ev_zero_start);
-  if (h->ev_zero_done)
-    cudaEventDestroy(h->ev_zero_done);
-  if (h->ev_pass_done)
-    cudaEventDestroy(h->ev_pass_done);
-  for (int q = 0; q < SLICER_MAX_SLOTS; q++)
-    if (h->ev_slot[q])
-      cudaEventDestroy(h->ev_slot[q]);
-  if (h->compute)
-    cudaStreamDestroy(h->compute);
-  if (h->copy)
-    cudaStreamDestroy(h->copy);
-  if (h->comm_stream)
-    cudaStreamDestroy(h->comm_stream);
   delete h;
 }
 
@@ -593,7 +566,7 @@ extern "C" int slicer_next_batch(slicer_handle *h)
   h->segs.clear();
   h->pos_used = 0;
   h->mass_used = 0;
-  h->deg.valid = false;
+  h->deg.counted = 0;
   return 0;
 }
 
@@ -1011,15 +984,21 @@ static int use_binned(const slicer_handle *h, const PassParams &P, double est_ac
   return est_accept > (h->bin_slice_hint() >= D.n || big_maps ? 0.015 : 0.03) ? 1 : 0;
 }
 
+// Each set is made whole or not at all: the buffers on first use, the masses on the first segment that has them.
 static int binned_alloc(slicer_handle *h, bool need_mass)
 {
-  if (h->bin.rec_u && need_mass && !h->bin.mass_u)
-  { // first segment with per-particle masses on this handle (e.g. staged from device memory without a mass_capacity)
-    if (dev_alloc(h, &h->bin.mass_u, h->bin.capacity) || dev_alloc(h, &h->bin.mass_s, h->bin.capacity))
+  if (h->bin.slice)
+  {
+    if (!need_mass || h->bin.mass_u)
+      return 0;
+    // first segment with per-particle masses on this handle (e.g. staged from device memory without a mass_capacity)
+    DevArray<float> mass_u, mass_s;
+    if (dev_alloc(h, mass_u, h->bin.capacity) || dev_alloc(h, mass_s, h->bin.capacity))
       return 1;
-  }
-  if (h->bin.rec_u)
+    h->bin.mass_u = std::move(mass_u);
+    h->bin.mass_s = std::move(mass_s);
     return 0;
+  }
   size_t slice = h->cfg.record_capacity ? h->cfg.record_capacity : ((size_t)1 << 28);
   if (slice > ((size_t)1 << 31))
     slice = (size_t)1 << 31; // record offsets are 32-bit
@@ -1029,16 +1008,17 @@ static int binned_alloc(slicer_handle *h, bool need_mass)
   slice = (slice + pipe::CHUNK - 1) / pipe::CHUNK * pipe::CHUNK;
   // every CTA region is rounded up to whole chunks, times the randomisations of a pass (one record per particle and randomisation)
   const size_t cap = slice + ((size_t)h->grid_max + 1) * pipe::CHUNK * SLICER_MAX_XFORMS;
-  if (dev_alloc(h, &h->bin.rec_u, cap) || dev_alloc(h, &h->bin.rec_s, cap) || dev_alloc(h, &h->bin.key_u, cap))
+  decltype(h->bin) B;
+  if (dev_alloc(h, B.rec_u, cap) || dev_alloc(h, B.rec_s, cap) || dev_alloc(h, B.key_u, cap))
     return 1;
-  if ((h->cfg.mass_capacity || need_mass) && (dev_alloc(h, &h->bin.mass_u, cap) || dev_alloc(h, &h->bin.mass_s, cap)))
+  if ((h->cfg.mass_capacity || need_mass) && (dev_alloc(h, B.mass_u, cap) || dev_alloc(h, B.mass_s, cap)))
     return 1;
-  if (dev_alloc(h, &h->bin.region_count, (size_t)h->grid_max) ||
-      dev_alloc(h, &h->bin.region_hist, (size_t)binned::MAX_BINS * h->grid_max) ||
-      dev_alloc(h, &h->bin.bin_count, (size_t)binned::MAX_BINS) || dev_alloc(h, &h->bin.bin_start, (size_t)binned::MAX_BINS + 1))
+  if (dev_alloc(h, B.region_count, (size_t)h->grid_max) || dev_alloc(h, B.region_hist, (size_t)binned::MAX_BINS * h->grid_max) ||
+      dev_alloc(h, B.bin_count, (size_t)binned::MAX_BINS) || dev_alloc(h, B.bin_start, (size_t)binned::MAX_BINS + 1))
     return 1;
-  h->bin.slice = slice;
-  h->bin.capacity = cap;
+  B.slice = slice;
+  B.capacity = cap;
+  h->bin = std::move(B);
   return 0;
 }
 
@@ -1083,7 +1063,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     binned::EmitDev E;
     E.rec = h->bin.rec_u;
     E.key = h->bin.key_u;
-    E.mass = D.mass ? h->bin.mass_u : nullptr;
+    E.mass = D.mass ? h->bin.mass_u.get() : nullptr;
     E.region_count = h->bin.region_count;
     E.region_cap = cmax * pipe::CHUNK * (unsigned long long)P.nxform; // one region per K1 CTA: every (particle, randomisation) pair of its chunks could be accepted
     E.ntile = nt;
@@ -1092,7 +1072,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     const int nregions = grid;
     // few bins (one sort window of at most HIST_BINS): the record kernel counts its region's records per bin itself
     const bool k1_hist = nbins <= binned::HIST_BINS && nbins <= binned::MAX_BINS;
-    E.region_hist = k1_hist ? h->bin.region_hist : nullptr;
+    E.region_hist = k1_hist ? h->bin.region_hist.get() : nullptr;
     E.nregions = nregions;
     E.nbins = nbins;
     if ((unsigned long long)nregions * E.region_cap > h->bin.capacity)
@@ -1110,10 +1090,10 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
     Q.bin_count = h->bin.bin_count;
     Q.bin_start = h->bin.bin_start;
     Q.rec_s = h->bin.rec_s;
-    Q.mass_s = D.mass ? h->bin.mass_s : nullptr;
+    Q.mass_s = D.mass ? h->bin.mass_s.get() : nullptr;
     Q.capacity = h->bin.capacity;
-    if (pipelined_launch(grid, h->cfg.mas, true, P, S, E, F, h->compute, &h->kernels_run))
-      return fail("record kernel launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (const cudaError_t e = pipelined_launch(grid, h->cfg.mas, true, P, S, E, F, h->compute, &h->kernels_run))
+      return fail("record kernel launch failed: %s", cudaGetErrorString(e));
     const int nwin = (nbins + binned::MAX_BINS - 1) / binned::MAX_BINS;
     const int wbins = (nbins + nwin - 1) / nwin;
     for (int lo = 0; lo < nbins; lo += wbins)
@@ -1260,8 +1240,8 @@ static int resolve_bank(slicer_handle *h, int bi)
       out[e.pass].push_back(r);
     }
     // (the list itself is the staging area of the settled pairs: the bank's passes are over, nothing appends to it)
-    ResolvedRec *dev = reinterpret_cast<ResolvedRec *>(B.buf);
-    ResolvedRec *stage = reinterpret_cast<ResolvedRec *>(B.host);
+    ResolvedRec *dev = reinterpret_cast<ResolvedRec *>(B.buf.get());
+    ResolvedRec *stage = reinterpret_cast<ResolvedRec *>(B.host.get());
     size_t off = 0;
     for (size_t k = 0; k < np; k++)
     {
@@ -1462,9 +1442,14 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
         if (binned_pass(h, P, D, F))
           return 1;
       }
-      else if (maps_ready(h) || pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F, h->compute,
-                                                         &h->kernels_run))
-        return fail("pipelined launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+      else
+      {
+        if (maps_ready(h))
+          return 1;
+        if (const cudaError_t e = pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F,
+                                                   h->compute, &h->kernels_run))
+          return fail("pipelined launch failed: %s", cudaGetErrorString(e));
+      }
     }
     else
     {
@@ -1503,7 +1488,7 @@ extern "C" int slicer_selftest_arith(slicer_handle *h, unsigned long long n, uns
     return fail("null argument");
   if (set_device(h))
     return 1;
-  unsigned long long *d = (unsigned long long *)h->d_out; // npix_max^2 floats of scratch
+  unsigned long long *d = (unsigned long long *)h->d_out.get(); // npix_max^2 floats of scratch
   if (h->npix2max * sizeof(float) < 3 * sizeof(unsigned long long))
     return fail("slicer_selftest_arith needs npix_max >= 3");
   CU(cudaStreamSynchronize(h->compute));
@@ -1521,7 +1506,7 @@ extern "C" int slicer_selftest_packed(slicer_handle *h, unsigned long long n, un
     return fail("null argument");
   if (set_device(h))
     return 1;
-  unsigned long long *d = (unsigned long long *)h->d_out; // npix_max^2 floats of scratch
+  unsigned long long *d = (unsigned long long *)h->d_out.get(); // npix_max^2 floats of scratch
   if (h->npix2max * sizeof(float) < 4 * sizeof(unsigned long long))
     return fail("slicer_selftest_packed needs npix_max >= 3");
   CU(cudaStreamSynchronize(h->compute));
@@ -1604,45 +1589,37 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
     return fail("slicer_count_accepted: null output");
   for (int i = 0; i < nplanes * SLICER_NTYPES; i++)
     counts[i] = 0;
-  h->deg.valid = false;
+  h->deg.counted = 0;
   if (total == 0)
   {
     for (int q = 0; q < nplanes; q++)
       h->deg.plane_total[q] = 0;
-    h->deg.nplanes = nplanes;
-    h->deg.stride = 0;
-    h->deg.valid = true;
+    h->deg.counted = nplanes;
     return 0;
   }
-  if (h->deg.stride < total || h->deg.nplanes < nplanes)
+  auto &W = h->deg.scratch;
+  if (W.stride < total || W.nplanes < nplanes)
   {
     CU(cudaStreamSynchronize(h->compute));
-    cudaFree(h->deg.cnt);
-    cudaFree(h->deg.rank);
-    cudaFree(h->deg.block_sums);
-    h->device_bytes -= h->deg.bytes;
-    h->deg.cnt = nullptr;
-    h->deg.rank = nullptr;
-    h->deg.block_sums = nullptr;
+    const int np = nplanes > W.nplanes ? nplanes : W.nplanes;
+    W = {}; // (the old set goes before the new one is made)
+    decltype(h->deg.scratch) N;
     const size_t stride = total + total / 8 + 1024;
     const size_t nblocks = (stride + 1 + degrade::SCAN_BLOCK * degrade::SCAN_PER - 1) / (degrade::SCAN_BLOCK * degrade::SCAN_PER);
-    const int np = nplanes > h->deg.nplanes ? nplanes : h->deg.nplanes;
-    const size_t before = h->device_bytes;
-    const int rc = dev_alloc(h, &h->deg.cnt, (size_t)np * stride) || dev_alloc(h, &h->deg.rank, (size_t)np * (stride + 1)) ||
-                   dev_alloc(h, &h->deg.block_sums, (size_t)np * nblocks);
-    h->deg.bytes = h->device_bytes - before;
-    if (rc)
+    if (dev_alloc(h, N.cnt, (size_t)np * stride) || dev_alloc(h, N.rank, (size_t)np * (stride + 1)) ||
+        dev_alloc(h, N.block_sums, (size_t)np * nblocks))
       return 1;
-    h->deg.stride = stride;
-    h->deg.nblocks = nblocks;
-    h->deg.nplanes = np;
+    N.stride = stride;
+    N.nblocks = nblocks;
+    N.nplanes = np;
+    W = std::move(N);
   }
-  const size_t stride = h->deg.stride;
-  CU(cudaMemsetAsync(h->deg.cnt, 0, (size_t)nplanes * stride, h->compute));
+  const size_t stride = W.stride;
+  CU(cudaMemsetAsync(W.cnt, 0, (size_t)nplanes * stride, h->compute));
   degrade::Dev G;
   memset(&G, 0, sizeof(G));
-  G.cnt = h->deg.cnt;
-  G.rank = h->deg.rank;
+  G.cnt = W.cnt;
+  G.rank = W.rank;
   G.stride = stride;
   if (degrade_launch<degrade::MARK>(h, P, G))
     return 1;
@@ -1651,16 +1628,16 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
     seg_start.push_back(seg_start.back() + sg.n);
   const size_t nb = (total + 1 + degrade::SCAN_BLOCK * degrade::SCAN_PER - 1) / (degrade::SCAN_BLOCK * degrade::SCAN_PER);
   const dim3 grid((unsigned)nb, (unsigned)nplanes);
-  degrade::scan_block_sums<<<grid, degrade::SCAN_BLOCK, 0, h->compute>>>(h->deg.cnt, stride, total, h->deg.block_sums, h->deg.nblocks);
-  degrade::scan_of_block_sums<<<dim3(1, nplanes), 1024, 0, h->compute>>>(h->deg.block_sums, h->deg.nblocks);
-  degrade::scan_finish<<<grid, degrade::SCAN_BLOCK, 0, h->compute>>>(h->deg.cnt, stride, total, h->deg.block_sums, h->deg.nblocks, h->deg.rank);
+  degrade::scan_block_sums<<<grid, degrade::SCAN_BLOCK, 0, h->compute>>>(W.cnt, stride, total, W.block_sums, W.nblocks);
+  degrade::scan_of_block_sums<<<dim3(1, nplanes), 1024, 0, h->compute>>>(W.block_sums, W.nblocks);
+  degrade::scan_finish<<<grid, degrade::SCAN_BLOCK, 0, h->compute>>>(W.cnt, stride, total, W.block_sums, W.nblocks, W.rank);
   CU(cudaGetLastError());
   h->stats.launches += 3;
   // accepted pairs per (plane, segment) = differences of the ranks at the segment boundaries
   std::vector<unsigned> edge((size_t)nplanes * seg_start.size());
   for (int q = 0; q < nplanes; q++)
     for (size_t k = 0; k < seg_start.size(); k++)
-      CU(cudaMemcpyAsync(&edge[q * seg_start.size() + k], h->deg.rank + (size_t)q * (stride + 1) + seg_start[k], sizeof(unsigned),
+      CU(cudaMemcpyAsync(&edge[q * seg_start.size() + k], W.rank + (size_t)q * (stride + 1) + seg_start[k], sizeof(unsigned),
                          cudaMemcpyDeviceToHost, h->compute));
   CU(cudaStreamSynchronize(h->compute));
   for (int q = 0; q < nplanes; q++)
@@ -1669,7 +1646,7 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
       counts[q * SLICER_NTYPES + h->segs[k].type] += (long long)(edge[q * seg_start.size() + k + 1] - edge[q * seg_start.size() + k]);
     h->deg.plane_total[q] = edge[q * seg_start.size() + seg_start.size() - 1];
   }
-  h->deg.valid = true;
+  h->deg.counted = nplanes;
   return 0;
 }
 
@@ -1684,7 +1661,7 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
     return 1;
   if (snopt < 1 || snopt > 30)
     return fail("slicer_deposit_degraded: snopt %d outside 1..30", snopt);
-  if (!h->deg.valid || h->deg.nplanes < nplanes)
+  if (h->deg.counted < nplanes)
     return fail("slicer_deposit_degraded: call slicer_count_accepted for this batch and these planes first");
   degrade::Dev G;
   memset(&G, 0, sizeof(G));
@@ -1700,24 +1677,19 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
     return 1;
   if (total == 0)
     return maps_ready(h) || slots_written(h, 0, nplanes, nullptr);
-  if (need > h->deg.keep_cap)
+  if (need > h->deg.keep.size())
   {
     CU(cudaStreamSynchronize(h->compute));
-    cudaFree(h->deg.keep);
-    h->device_bytes -= h->deg.keep_cap;
-    h->deg.keep = nullptr;
-    h->deg.keep_cap = 0;
-    if (dev_alloc(h, &h->deg.keep, need + need / 4 + 4096))
+    if (dev_alloc(h, h->deg.keep, need + need / 4 + 4096))
       return 1;
-    h->deg.keep_cap = need + need / 4 + 4096;
   }
   for (int q = 0; q < nplanes; q++)
     if (h->deg.plane_total[q])
       CU(cudaMemcpyAsync(h->deg.keep + G.keep_off[q], keep[q], h->deg.plane_total[q], cudaMemcpyHostToDevice, h->compute));
-  G.cnt = h->deg.cnt;
-  G.rank = h->deg.rank;
+  G.cnt = h->deg.scratch.cnt;
+  G.rank = h->deg.scratch.rank;
   G.keep = h->deg.keep;
-  G.stride = h->deg.stride;
+  G.stride = h->deg.scratch.stride;
   G.snopt = snopt;
   if (maps_ready(h) || degrade_launch<degrade::DEPOSIT>(h, P, G) || slots_written(h, 0, nplanes, nullptr))
     return 1;
@@ -1856,32 +1828,19 @@ extern "C" int slicer_kappa_maps(slicer_handle *h, int nmaps, int npix)
   if (set_device(h))
     return 1;
   h->shear.map = -1; // (its γ maps are of maps that go)
-  if (h->kappa.maps)
-  { // (cudaFree waits for the work that still reads or writes them)
-    CU(cudaFree(h->kappa.maps));
-    CU(cudaFree(h->kappa.ovf));
-    h->device_bytes -= (size_t)h->kappa.n * (h->kappa.stride * sizeof(double) + sizeof(unsigned));
-    h->kappa.maps = nullptr;
-    h->kappa.ovf = nullptr;
-    h->kappa.n = h->kappa.npix = 0;
-  }
+  h->kappa = {};     // (cudaFree waits for the work that still reads or writes them)
   if (nmaps == 0)
     return 0;
   const size_t stride = ((size_t)npix * npix + 1) & ~(size_t)1; // every map starts on a 16-byte boundary
-  if (dev_alloc(h, &h->kappa.maps, (size_t)nmaps * stride))
+  decltype(h->kappa) K;
+  if (dev_alloc(h, K.maps, (size_t)nmaps * stride) || dev_alloc(h, K.ovf, (size_t)nmaps))
     return 1;
-  if (dev_alloc(h, &h->kappa.ovf, (size_t)nmaps))
-  {
-    cudaFree(h->kappa.maps);
-    h->kappa.maps = nullptr;
-    h->device_bytes -= (size_t)nmaps * stride * sizeof(double);
-    return 1;
-  }
-  h->kappa.n = nmaps;
-  h->kappa.npix = npix;
-  h->kappa.stride = stride;
-  CU(cudaMemsetAsync(h->kappa.maps, 0, (size_t)nmaps * stride * sizeof(double), h->compute));
-  CU(cudaMemsetAsync(h->kappa.ovf, 0, (size_t)nmaps * sizeof(unsigned), h->compute));
+  CU(cudaMemsetAsync(K.maps, 0, (size_t)nmaps * stride * sizeof(double), h->compute));
+  CU(cudaMemsetAsync(K.ovf, 0, (size_t)nmaps * sizeof(unsigned), h->compute));
+  K.n = nmaps;
+  K.npix = npix;
+  K.stride = stride;
+  h->kappa = std::move(K);
   return 0;
 }
 
@@ -1988,38 +1947,18 @@ extern "C" int slicer_kappa_load(slicer_handle *h, int map, const double *in)
 // ------------------------------------------------------------------------------------------------------------
 // shear maps (shear.cuh)
 // ------------------------------------------------------------------------------------------------------------
-static void shear_free(slicer_handle *h)
-{
-  auto &S = h->shear;
-  if (!S.tw)
-    return;
-  cudaFree(S.buf[0]);
-  cudaFree(S.buf[1]);
-  cudaFree(S.tw);
-  cudaFree(S.g);
-  h->device_bytes -= 2 * (size_t)S.P * S.P * sizeof(double2) + (size_t)S.P * sizeof(double2) + 2 * (size_t)S.npix * S.npix * sizeof(double);
-  S = {};
-}
-
 // workspaces for P and γ maps of npix^2: kept while both stay, made again when either changes
 static int shear_workspace(slicer_handle *h, int P, int npix)
 {
-  auto &S = h->shear;
-  if (S.tw && S.P == P && S.npix == npix)
+  if (h->shear.tw && h->shear.P == P && h->shear.npix == npix)
     return 0;
-  shear_free(h); // (cudaFree waits for the work that still uses them)
-  S.P = P;
-  S.npix = npix;
-  const size_t ws = (size_t)P * P * sizeof(double2), gs = 2 * (size_t)npix * npix * sizeof(double), ts = (size_t)P * sizeof(double2);
-  if (dev_alloc(h, &S.buf[0], (size_t)P * P) || dev_alloc(h, &S.buf[1], (size_t)P * P) || dev_alloc(h, &S.g, 2 * (size_t)npix * npix) ||
-      dev_alloc(h, &S.tw, (size_t)P))
+  h->shear = {}; // (cudaFree waits for the work that still uses them)
+  decltype(h->shear) S;
+  if (dev_alloc(h, S.buf[0], (size_t)P * P) || dev_alloc(h, S.buf[1], (size_t)P * P) || dev_alloc(h, S.g, 2 * (size_t)npix * npix) ||
+      dev_alloc(h, S.tw, (size_t)P))
   {
     const std::string err = g_err;
-    h->device_bytes -= (S.buf[0] ? ws : 0) + (S.buf[1] ? ws : 0) + (S.g ? gs : 0); // (the table is allocated last)
-    cudaFree(S.buf[0]);
-    cudaFree(S.buf[1]);
-    cudaFree(S.g);
-    S = {};
+    const size_t ws = (size_t)P * P * sizeof(double2), gs = 2 * (size_t)npix * npix * sizeof(double), ts = (size_t)P * sizeof(double2);
     return fail("slicer_shear: workspace for FFT size %d (%.3g GB): %s", P, (2 * ws + gs + ts) / 1e9, err.c_str());
   }
   // the table, from the host's libm in exactly this expression (the restatement evaluates the same one)
@@ -2028,6 +1967,9 @@ static int shear_workspace(slicer_handle *h, int P, int npix)
     tw[k] = make_double2(cos(2.0 * M_PI * k / P), sin(2.0 * M_PI * k / P));
   CU(cudaMemcpyAsync(S.tw, tw.data(), (size_t)P * sizeof(double2), cudaMemcpyHostToDevice, h->compute));
   CU(cudaStreamSynchronize(h->compute));
+  S.P = P;
+  S.npix = npix;
+  h->shear = std::move(S);
   return 0;
 }
 
@@ -2237,9 +2179,7 @@ extern "C" int slicer_comm_init_ranks(slicer_handle **handles, int n, const char
   int rc = 0;
   for (int i = 0; i < n && !rc; i++)
   {
-    if (cudaSetDevice(handles[i]->cfg.device) != cudaSuccess)
-      rc = fail("cudaSetDevice failed");
-    else
+    if (!(rc = set_device(handles[i])))
     {
       const ncclResult_t r = g_nccl.CommInitRank(&comms[i], nranks, u, first_rank + i);
       if (r != ncclSuccess)
@@ -2254,6 +2194,7 @@ extern "C" int slicer_comm_init_ranks(slicer_handle **handles, int n, const char
     for (int i = 0; i < n; i++)
       if (comms[i] && cudaSetDevice(handles[i]->cfg.device) == cudaSuccess)
         g_nccl.CommAbort(comms[i]);
+    cudaGetLastError(); // (nor a cudaSetDevice that failed here)
     return rc;
   }
   for (int i = 0; i < n; i++)
@@ -2395,12 +2336,7 @@ extern "C" int slicer_reduce_all_slots(slicer_handle **handles, int n, int first
   NC(g_nccl.GroupStart());
   int rc = 0;
   for (int i = 0; i < n && !rc; i++)
-  {
-    if (cudaSetDevice(handles[i]->cfg.device) != cudaSuccess)
-      rc = fail("cudaSetDevice failed");
-    else
-      rc = enqueue_reduce(handles[i], first_slot, nplanes, root);
-  }
+    rc = set_device(handles[i]) || enqueue_reduce(handles[i], first_slot, nplanes, root);
   const ncclResult_t ge = g_nccl.GroupEnd();
   if (rc)
     return rc;
