@@ -160,6 +160,32 @@ static int make_event(Event &e, unsigned flags)
   return 0;
 }
 
+// One stream's dependency on another: signal() records the event on the stream that produces, wait() makes the stream that
+// consumes wait for the last signal, once.  A dependency with two consuming streams takes one fence for each.
+class Fence
+{
+  Event ev_;
+  bool pending_ = false;
+
+public:
+  int make() { return make_event(ev_, cudaEventDisableTiming); }
+  int signal(cudaStream_t s)
+  {
+    CU(cudaEventRecord(ev_, s));
+    pending_ = true;
+    return 0;
+  }
+  int wait(cudaStream_t s)
+  {
+    if (pending_)
+    {
+      CU(cudaStreamWaitEvent(s, ev_, 0));
+      pending_ = false;
+    }
+    return 0;
+  }
+};
+
 // ------------------------------------------------------------------------------------------------------------
 // NCCL, loaded lazily so that single-GPU use has no dependency on it
 // ------------------------------------------------------------------------------------------------------------
@@ -237,13 +263,10 @@ struct slicer_handle
   size_t device_bytes = 0; // what the DevArray members below hold (declared before them: they count in it until they go)
   Stream compute, copy, comm_stream;
   Stream aux;                                // zeroing of large accumulators, concurrent with the record kernel of a binned pass
-  Event ev_zero_start, ev_zero_done;
-  bool zero_pending = false;                 // the compute stream has not yet waited for ev_zero_done
-  Event ev_pass_done;                        // compute -> comm_stream: the passes a reduce sums
-  Event ev_slot[SLICER_MAX_SLOTS];           // comm_stream -> compute: the last reduce of accumulator slot q (q < max_planes)
-  bool slot_reducing[SLICER_MAX_SLOTS] = {}; // ev_slot[q] is pending
-  Event ev_copy;
-  Event ev_buf_done[2];                      // last pass that read staging pool b
+  Fence zero_start, zeroed;                  // compute -> aux before a zeroing, aux -> compute after it
+  Fence passes_done;                         // compute -> comm_stream: the passes a reduce sums
+  Fence staged;                              // copy -> compute: the staged particles
+  Fence pool_read[2];                        // compute -> copy: the last pass that read staging pool b
   Event ev_t0, ev_t1;                        // slicer_timer_*
   std::vector<Event> pass_ev;                // ring of (start, stop) pairs, resolved lazily
   size_t pass_head = 0, pass_tail = 0;       // pairs [tail, head) are pending
@@ -279,8 +302,14 @@ struct slicer_handle
   double boxsize = 0;
   double massarr[SLICER_NTYPES] = {0, 0, 0, 0, 0, 0};
   int hydro = 0;
-  int plane_npix[SLICER_MAX_SLOTS] = {};
-  bool copy_pending = false;
+  // accumulator slot q (events made for q < max_planes)
+  struct Slot
+  {
+    int npix = 0;                  // side of the plane last deposited into it (0: none yet)
+    unsigned long long epoch = 0;  // times it was zeroed
+    cudaEvent_t written = nullptr; // the stop event (pass_ev ring) of the last pass into it; nullptr: the whole compute stream
+    Fence reduced;                 // comm_stream -> compute: its last reduce
+  } slots[SLICER_MAX_SLOTS];
   slicer_stats stats = {};
   unsigned long long kernels_run = 0; // slicer_kernels_run: bit i = pipelined_table() entry i, bit 40 + mas = deposit_simple_kernel
   ncclComm_t comm = nullptr;
@@ -315,11 +344,7 @@ struct slicer_handle
   } defer;
   DevArray<unsigned> d_ovf;         // device flag: an accumulator ran past 2^63 (raised at read-out)
   Stream settle;                    // deposits of the pairs libm settled, beside the passes running on `compute`
-  Event ev_settled;                 // settle -> compute / comm_stream
-  bool settle_pending = false;      // `compute` has not yet waited for ev_settled
-  bool settle_pending_comm = false; // nor has `comm_stream`
-  cudaEvent_t slot_pass_ev[SLICER_MAX_SLOTS] = {}; // the stop event (pass_ev ring) of the last pass into accumulator slot q, or nullptr
-  unsigned long long slot_epoch[SLICER_MAX_SLOTS] = {};
+  Fence settled, settled_comm;      // settle -> compute, settle -> comm_stream
   size_t pos_stride = 0, mass_stride = 0; // floats per staging pool (16-byte multiples)
   size_t pcap = 0, mcap = 0;              // particles / masses a pool holds, padding of the segments included
   // particles per slice the binned path will use (before allocation: what it would allocate)
@@ -457,12 +482,15 @@ extern "C" int slicer_create(const slicer_config *cfg, slicer_handle **out)
   for (Stream *s : {&h->compute, &h->copy, &h->comm_stream, &h->aux, &h->settle})
     if (make_stream(*s))
       return 1;
-  for (Event *ev : {&h->ev_settled, &h->defer.bank[0].ev_done, &h->defer.bank[1].ev_done, &h->ev_zero_start, &h->ev_zero_done,
-                    &h->ev_pass_done, &h->ev_copy, &h->ev_buf_done[0], &h->ev_buf_done[1]})
+  for (Event *ev : {&h->defer.bank[0].ev_done, &h->defer.bank[1].ev_done})
     if (make_event(*ev, cudaEventDisableTiming))
       return 1;
+  for (Fence *f : {&h->settled, &h->settled_comm, &h->zero_start, &h->zeroed, &h->passes_done, &h->staged, &h->pool_read[0],
+                   &h->pool_read[1]})
+    if (f->make())
+      return 1;
   for (int q = 0; q < cfg->max_planes; q++)
-    if (make_event(h->ev_slot[q], cudaEventDisableTiming))
+    if (h->slots[q].reduced.make())
       return 1;
   h->pass_ev.resize(2 * PASS_RING);
   for (Event *ev : {&h->ev_t0, &h->ev_t1})
@@ -560,7 +588,8 @@ extern "C" int slicer_next_batch(slicer_handle *h)
     return 1;
   h->cur_buf = (h->cur_buf + 1) % h->nbuf;
   // this pool is about to be overwritten: copies must wait for the pass that last read it
-  CU(cudaStreamWaitEvent(h->copy, h->ev_buf_done[h->cur_buf], 0));
+  if (h->pool_read[h->cur_buf].wait(h->copy))
+    return 1;
   h->d_pos = h->d_pos_pool ? h->d_pos_pool + (size_t)h->cur_buf * h->pos_stride : nullptr;
   h->d_mass = h->d_mass_pool ? h->d_mass_pool + (size_t)h->cur_buf * h->mass_stride : nullptr;
   h->segs.clear();
@@ -629,8 +658,7 @@ extern "C" int slicer_stage_particles(slicer_handle *h, int type, const float *p
   }
   h->pos_used += npad;
   h->segs.push_back(s);
-  h->copy_pending = true;
-  return 0;
+  return h->staged.signal(h->copy);
 }
 
 extern "C" int slicer_stage_device(slicer_handle *h, int type, const void *dev_pos, int layout, const void *dev_mass, size_t n)
@@ -690,8 +718,7 @@ extern "C" int slicer_stage_synthetic_window(slicer_handle *h, int type, unsigne
   h->stats.launches++;
   h->pos_used += npad;
   h->segs.push_back(s);
-  h->copy_pending = true;
-  return 0;
+  return h->staged.signal(h->copy);
 }
 
 extern "C" int slicer_download_segment(slicer_handle *h, int segment, float *pos_out, float *mass_out)
@@ -869,7 +896,7 @@ static int build_pass(slicer_handle *h, const slicer_plane_desc *planes, int npl
       L.counts = h->d_counts + (size_t)slot * SLICER_NTYPES * 2;
       L.type_stride = h->cfg.per_type_maps ? h->npix2max : 0;
       L.slot = slot;
-      h->plane_npix[slot] = d.npix;
+      h->slots[slot].npix = d.npix;
       {
         // fraction of a uniform snapshot this plane accepts: slab thickness x (field width / box)^2 at mid-distance
         const double w = L.T < 1.5 ? 2.0 * tan(L.T) * 0.5 * (minDist + maxDist) : 1.0;
@@ -1022,18 +1049,6 @@ static int binned_alloc(slicer_handle *h, bool need_mass)
   return 0;
 }
 
-// Large accumulators are zeroed on a side stream (run_pass) so that the write overlaps the record kernel of a binned pass, which
-// does not touch the maps; whatever does touch them calls this first.
-static int maps_ready(slicer_handle *h)
-{
-  if (h->zero_pending)
-  {
-    CU(cudaStreamWaitEvent(h->compute, h->ev_zero_done, 0));
-    h->zero_pending = false;
-  }
-  return 0;
-}
-
 static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &D, const DeferDev &F)
 {
   if (binned_alloc(h, D.mass != nullptr))
@@ -1105,7 +1120,7 @@ static int binned_pass(slicer_handle *h, const PassParams &P, const SegmentDev &
       binned::bin_region_scan_kernel<<<Q.nbins, 1024, 0, h->compute>>>(Q);
       binned::bin_scan_kernel<<<1, 1024, 0, h->compute>>>(Q);
       binned::launch_bin_scatter(Q, nwin > 1, h->compute);
-      if (maps_ready(h))
+      if (h->zeroed.wait(h->compute))
         return 1;
       if (h->cfg.mas == SLICER_MAS_NGP)
         binned::tile_deposit_kernel<SLICER_MAS_NGP><<<Q.nbins << gshift, binned::DEPOSIT_THREADS, binned::TCELLS * 8, h->compute>>>(P, Q, nt, ntx, gshift, D.type, D.const_mass);
@@ -1225,7 +1240,7 @@ static int resolve_bank(slicer_handle *h, int bi)
         return fail("corrupt deferred entry (internal error)");
       const slicer_handle::SavedPass &sp = B.passes[e.pass];
       const PlaneDev &L = sp.P.pl[e.plane];
-      if (sp.epoch[e.plane] != h->slot_epoch[L.slot])
+      if (sp.epoch[e.plane] != h->slots[L.slot].epoch)
       {
         h->stats.flagged_void++;
         continue; // the accumulator was zeroed after that pass
@@ -1262,8 +1277,8 @@ static int resolve_bank(slicer_handle *h, int bi)
     B.host_count[0] = 0;
     // whatever touches the accumulators or this bank next (a pass, a read-out, a reduce) waits for these on the device;
     // the next use of the pinned mirror is behind the next cudaEventSynchronize(B.ev_done), which these precede in stream order
-    CU(cudaEventRecord(h->ev_settled, h->settle));
-    h->settle_pending = h->settle_pending_comm = true;
+    if (h->settled.signal(h->settle) || h->settled_comm.signal(h->settle))
+      return 1;
   }
   B.passes.clear();
   B.slot_mask = 0;
@@ -1289,52 +1304,16 @@ static int resolve_deferred(slicer_handle *h, int lo = 0, int n = -1)
   return 0;
 }
 
-// the compute stream (or the communication stream) must see the deposits of the settled pairs before it touches accumulators
-static int wait_settled(slicer_handle *h, bool comm)
-{
-  if (!comm && h->settle_pending)
-  {
-    CU(cudaStreamWaitEvent(h->compute, h->ev_settled, 0));
-    h->settle_pending = false;
-  }
-  if (comm && h->settle_pending_comm)
-  {
-    CU(cudaStreamWaitEvent(h->comm_stream, h->ev_settled, 0));
-    h->settle_pending_comm = false;
-  }
-  return 0;
-}
-
-// compute-stream work on accumulator slots [lo, lo + n) must follow the reduces still running on them
-static int wait_slot_reduces(slicer_handle *h, int lo, int n)
-{
-  for (int q = lo; q < lo + n && q < SLICER_MAX_SLOTS; q++)
-    if (h->slot_reducing[q])
-    {
-      CU(cudaStreamWaitEvent(h->compute, h->ev_slot[q], 0));
-      h->slot_reducing[q] = false;
-    }
-  return 0;
-}
-
-// staged particles must be on the device before the compute stream reads them
-static int staging_fence(slicer_handle *h)
-{
-  if (h->copy_pending)
-  {
-    CU(cudaEventRecord(h->ev_copy, h->copy));
-    CU(cudaStreamWaitEvent(h->compute, h->ev_copy, 0));
-    h->copy_pending = false;
-  }
-  return 0;
-}
-
-// Every write into accumulator slots [lo, lo + n) on the compute stream claims them first: it follows the reduces still reading
+// Every use of accumulator slots [lo, lo + n) on the compute stream claims them first: it follows the reduces still reading
 // them and the deposits of the pairs libm settled.  A write that does not accumulate also zeroes them and voids the pairs earlier
-// passes into them deferred; large accumulators are zeroed on `aux`, so the writer calls maps_ready before it touches them.
+// passes into them deferred.  Large accumulators are zeroed on `aux`, so that the write overlaps the record kernel of a binned
+// pass, which does not touch the maps; the writer waits for `zeroed` before it touches them.
 static int claim_slots(slicer_handle *h, int lo, int n, bool accumulate)
 {
-  if (wait_slot_reduces(h, lo, n) || wait_settled(h, false))
+  for (int q = lo; q < lo + n; q++)
+    if (h->slots[q].reduced.wait(h->compute))
+      return 1;
+  if (h->settled.wait(h->compute))
     return 1;
   if (accumulate)
     return 0;
@@ -1342,30 +1321,30 @@ static int claim_slots(slicer_handle *h, int lo, int n, bool accumulate)
   unsigned long long *zptr = h->d_acc + (size_t)lo * h->ntypes_alloc * h->npix2max;
   if (zbytes >= ((size_t)64 << 20))
   { // (8192^2 planes: 2 GiB per pass, 0.7 ms on the compute stream) after everything queued so far, beside what comes next
-    if (maps_ready(h))
+    if (h->zeroed.wait(h->compute) || h->zero_start.signal(h->compute) || h->zero_start.wait(h->aux))
       return 1;
-    CU(cudaEventRecord(h->ev_zero_start, h->compute));
-    CU(cudaStreamWaitEvent(h->aux, h->ev_zero_start, 0));
     CU(cudaMemsetAsync(zptr, 0, zbytes, h->aux));
-    CU(cudaEventRecord(h->ev_zero_done, h->aux));
-    h->zero_pending = true;
+    if (h->zeroed.signal(h->aux))
+      return 1;
   }
   else
     CU(cudaMemsetAsync(zptr, 0, zbytes, h->compute));
   CU(cudaMemsetAsync(h->d_counts + (size_t)lo * SLICER_NTYPES * 2, 0, (size_t)n * SLICER_NTYPES * 2 * sizeof(unsigned long long), h->compute));
   for (int q = lo; q < lo + n; q++)
-    h->slot_epoch[q]++; // deferred particles of earlier passes into these accumulators are void
+    h->slots[q].epoch++; // deferred particles of earlier passes into these accumulators are void
   return 0;
 }
+
+// A read of slots [lo, lo + n) on the compute stream: settles the pairs the passes into them deferred, then claims them.
+static int read_slots(slicer_handle *h, int lo, int n) { return resolve_deferred(h, lo, n) || claim_slots(h, lo, n, true); }
 
 // After a write into slots [lo, lo + n) on the compute stream: a reduce of them waits for `done`, or for the whole compute stream
 // when `done` is nullptr; the staging pool the write read may be overwritten behind it.
 static int slots_written(slicer_handle *h, int lo, int n, cudaEvent_t done)
 {
   for (int q = lo; q < lo + n; q++)
-    h->slot_pass_ev[q] = done;
-  CU(cudaEventRecord(h->ev_buf_done[h->cur_buf], h->compute));
-  return 0;
+    h->slots[q].written = done;
+  return h->pool_read[h->cur_buf].signal(h->compute);
 }
 
 static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, bool accumulate, int first_slot = 0)
@@ -1378,7 +1357,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     return fail("slicer_deposit: slots %d..%d outside 0..%d (max_planes)", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
   PassParams P;
   double est_accept = 0;
-  if (build_pass(h, planes, nplanes, &P, first_slot, &est_accept) || staging_fence(h))
+  if (build_pass(h, planes, nplanes, &P, first_slot, &est_accept) || h->staged.wait(h->compute))
     return 1;
   // A new set of planes takes the other bank when that bank is settled (a caller that alternates between two slot ranges and
   // settles or reduces one range behind the next pass finds it so every time), or when it zeroes slots the current bank holds
@@ -1414,7 +1393,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     sp.P = P;
     for (int k = 0; k < P.nplanes; k++)
     {
-      sp.epoch[k] = h->slot_epoch[P.pl[k].slot];
+      sp.epoch[k] = h->slots[P.pl[k].slot].epoch;
       B.slot_mask |= (uint64_t)1 << P.pl[k].slot;
     }
     B.passes.push_back(sp);
@@ -1444,7 +1423,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
       }
       else
       {
-        if (maps_ready(h))
+        if (h->zeroed.wait(h->compute))
           return 1;
         if (const cudaError_t e = pipelined_launch(pipelined_grid(h->grid_max, D.n), h->cfg.mas, false, P, D, binned::EmitDev{}, F,
                                                    h->compute, &h->kernels_run))
@@ -1456,7 +1435,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
       size_t want = (D.n + 255) / 256;
       size_t cap = (size_t)h->sm_count * 8;
       int blocks = (int)(want < cap ? want : cap);
-      if (maps_ready(h))
+      if (h->zeroed.wait(h->compute))
         return 1;
       if (h->cfg.mas == SLICER_MAS_NGP)
         deposit_simple_kernel<SLICER_MAS_NGP><<<blocks, 256, 0, h->compute>>>(P, D, F);
@@ -1469,7 +1448,7 @@ static int run_pass(slicer_handle *h, const slicer_plane_desc *planes, int nplan
     h->stats.deposit_launches++;
     h->stats.particles_streamed += D.n;
   }
-  if (maps_ready(h)) // (a pass without particles still leaves zeroed planes behind it in stream order)
+  if (h->zeroed.wait(h->compute)) // (a pass without particles still leaves zeroed planes behind it in stream order)
     return 1;
   CU(cudaEventRecord(e1, h->compute));
   // the bank's deferred list as of now, for resolve_bank
@@ -1583,7 +1562,7 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
 {
   PassParams P;
   size_t total = 0;
-  if (degrade_prepare(h, planes, nplanes, &P, &total) || staging_fence(h))
+  if (degrade_prepare(h, planes, nplanes, &P, &total) || h->staged.wait(h->compute))
     return 1;
   if (!counts)
     return fail("slicer_count_accepted: null output");
@@ -1650,7 +1629,7 @@ extern "C" int slicer_count_accepted(slicer_handle *h, const slicer_plane_desc *
   return 0;
 }
 
-// Writes accumulator slots [0, nplanes) like a pass, but leaves their slot_pass_ev empty: a reduce of them waits for the whole
+// Writes accumulator slots [0, nplanes) like a pass, but leaves their `written` empty: a reduce of them waits for the whole
 // compute stream.
 extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc *planes, int nplanes, int snopt,
                                        const unsigned char *const *keep, int accumulate)
@@ -1673,10 +1652,10 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
     if (h->deg.plane_total[q] && (!keep || !keep[q]))
       return fail("slicer_deposit_degraded: keep table of plane %d is missing", q);
   }
-  if (staging_fence(h) || claim_slots(h, 0, nplanes, accumulate != 0))
+  if (h->staged.wait(h->compute) || claim_slots(h, 0, nplanes, accumulate != 0))
     return 1;
   if (total == 0)
-    return maps_ready(h) || slots_written(h, 0, nplanes, nullptr);
+    return h->zeroed.wait(h->compute) || slots_written(h, 0, nplanes, nullptr);
   if (need > h->deg.keep.size())
   {
     CU(cudaStreamSynchronize(h->compute));
@@ -1691,7 +1670,7 @@ extern "C" int slicer_deposit_degraded(slicer_handle *h, const slicer_plane_desc
   G.keep = h->deg.keep;
   G.stride = h->deg.scratch.stride;
   G.snopt = snopt;
-  if (maps_ready(h) || degrade_launch<degrade::DEPOSIT>(h, P, G) || slots_written(h, 0, nplanes, nullptr))
+  if (h->zeroed.wait(h->compute) || degrade_launch<degrade::DEPOSIT>(h, P, G) || slots_written(h, 0, nplanes, nullptr))
     return 1;
   CU(cudaStreamSynchronize(h->compute)); // the caller's keep tables may be freed on return
   return 0;
@@ -1742,7 +1721,7 @@ static int check_plane(slicer_handle *h, int plane, int type)
     return fail("null handle");
   if (plane < 0 || plane >= h->cfg.max_planes)
     return fail("plane %d outside 0..%d", plane, h->cfg.max_planes - 1);
-  if (h->plane_npix[plane] <= 0)
+  if (h->slots[plane].npix <= 0)
     return fail("plane %d has not been deposited", plane);
   if (type < -1 || type >= SLICER_NTYPES)
     return fail("type %d outside -1..5", type);
@@ -1751,27 +1730,44 @@ static int check_plane(slicer_handle *h, int plane, int type)
   return set_device(h);
 }
 
-extern "C" int slicer_fetch(slicer_handle *h, int plane, int type, float *out_map, long long counts[SLICER_NTYPES],
-                            long long ingrid[SLICER_NTYPES])
+// The failure of a read-out that met an accumulator past 2^63: `what` names what was read
+static int fail_overflow(const slicer_handle *h, const char *what, int index)
 {
-  if (check_plane(h, plane, type) || resolve_deferred(h, plane, 1) || wait_settled(h, false) || wait_slot_reduces(h, plane, 1))
+  return fail("%s %d: a fixed-point accumulator exceeded 2^63 (more than %.3g mass units in one pixel at %d fraction bits); create the "
+              "handle with a smaller slicer_config.frac_bits", what, index, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
+}
+
+// Slot `plane`, type `type` (-1: all types) as floats into `map` and as fixed-point sums into `fixed`, and its counters into
+// `counts` and `ingrid`; any of the four may be nullptr
+static int read_plane(slicer_handle *h, int plane, int type, float *map, long long *fixed, long long counts[SLICER_NTYPES],
+                      long long ingrid[SLICER_NTYPES])
+{
+  if (check_plane(h, plane, type) || read_slots(h, plane, 1))
     return 1;
-  const size_t npix2 = (size_t)h->plane_npix[plane] * h->plane_npix[plane];
+  const size_t npix2 = (size_t)h->slots[plane].npix * h->slots[plane].npix;
   const unsigned long long *base = h->d_acc + (size_t)plane * h->ntypes_alloc * h->npix2max;
-  if (out_map)
+  const unsigned long long *src = type >= 0 ? base + (size_t)type * h->npix2max : base;
+  const int nt = type >= 0 ? 1 : h->ntypes_alloc;
+  const int blocks = (int)((npix2 + 255) / 256 < (size_t)h->sm_count * 8 ? (npix2 + 255) / 256 : (size_t)h->sm_count * 8);
+  if (map)
   {
-    const unsigned long long *src = type >= 0 ? base + (size_t)type * h->npix2max : base;
-    const int nt = type >= 0 ? 1 : h->ntypes_alloc;
-    const int blocks = (int)((npix2 + 255) / 256 < (size_t)h->sm_count * 8 ? (npix2 + 255) / 256 : (size_t)h->sm_count * 8);
     finalize_map_kernel<<<blocks, 256, 0, h->compute>>>(src, h->npix2max, nt, npix2, ldexp(1.0, -h->frac_bits), h->d_out, h->d_ovf);
     CU(cudaGetLastError());
     h->stats.launches++;
-    CU(cudaMemcpyAsync(out_map, h->d_out, npix2 * sizeof(float), cudaMemcpyDeviceToHost, h->compute));
+    CU(cudaMemcpyAsync(map, h->d_out, npix2 * sizeof(float), cudaMemcpyDeviceToHost, h->compute));
+  }
+  if (fixed)
+  {
+    sum_types_kernel<<<blocks, 256, 0, h->compute>>>(src, h->npix2max, nt, npix2, h->d_sum, h->d_ovf);
+    CU(cudaGetLastError());
+    h->stats.launches++;
+    CU(cudaMemcpyAsync(fixed, h->d_sum, npix2 * sizeof(long long), cudaMemcpyDeviceToHost, h->compute));
   }
   unsigned ovf = 0;
   CU(cudaMemcpyAsync(&ovf, h->d_ovf, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
   unsigned long long c[SLICER_NTYPES * 2];
-  CU(cudaMemcpyAsync(c, h->d_counts + (size_t)plane * SLICER_NTYPES * 2, sizeof(c), cudaMemcpyDeviceToHost, h->compute));
+  if (counts || ingrid)
+    CU(cudaMemcpyAsync(c, h->d_counts + (size_t)plane * SLICER_NTYPES * 2, sizeof(c), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaStreamSynchronize(h->compute));
   for (int t = 0; t < SLICER_NTYPES; t++)
   {
@@ -1783,37 +1779,22 @@ extern "C" int slicer_fetch(slicer_handle *h, int plane, int type, float *out_ma
   if (ovf)
   {
     CU(cudaMemsetAsync(h->d_ovf, 0, sizeof(unsigned), h->compute));
-    return fail("plane %d: a fixed-point accumulator exceeded 2^63 (more than %.3g mass units in one pixel at %d fraction bits); "
-                "create the handle with a smaller slicer_config.frac_bits", plane, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
+    return fail_overflow(h, "plane", plane);
   }
   return 0;
 }
 
+extern "C" int slicer_fetch(slicer_handle *h, int plane, int type, float *out_map, long long counts[SLICER_NTYPES],
+                            long long ingrid[SLICER_NTYPES])
+{
+  return read_plane(h, plane, type, out_map, nullptr, counts, ingrid);
+}
+
 extern "C" int slicer_fetch_fixed(slicer_handle *h, int plane, int type, long long *out)
 {
-  if (check_plane(h, plane, type) || resolve_deferred(h, plane, 1) || wait_settled(h, false) || wait_slot_reduces(h, plane, 1))
-    return 1;
   if (!out)
     return fail("slicer_fetch_fixed: null output");
-  const size_t npix2 = (size_t)h->plane_npix[plane] * h->plane_npix[plane];
-  const unsigned long long *base = h->d_acc + (size_t)plane * h->ntypes_alloc * h->npix2max;
-  const unsigned long long *src = type >= 0 ? base + (size_t)type * h->npix2max : base;
-  const int nt = type >= 0 ? 1 : h->ntypes_alloc;
-  const int blocks = (int)((npix2 + 255) / 256 < (size_t)h->sm_count * 8 ? (npix2 + 255) / 256 : (size_t)h->sm_count * 8);
-  sum_types_kernel<<<blocks, 256, 0, h->compute>>>(src, h->npix2max, nt, npix2, h->d_sum, h->d_ovf);
-  CU(cudaGetLastError());
-  h->stats.launches++;
-  CU(cudaMemcpyAsync(out, h->d_sum, npix2 * sizeof(long long), cudaMemcpyDeviceToHost, h->compute));
-  unsigned ovf = 0;
-  CU(cudaMemcpyAsync(&ovf, h->d_ovf, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
-  CU(cudaStreamSynchronize(h->compute));
-  if (ovf)
-  {
-    CU(cudaMemsetAsync(h->d_ovf, 0, sizeof(unsigned), h->compute));
-    return fail("plane %d: a fixed-point accumulator exceeded 2^63 (more than %.3g mass units in one pixel at %d fraction bits); "
-                "create the handle with a smaller slicer_config.frac_bits", plane, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
-  }
-  return 0;
+  return read_plane(h, plane, type, nullptr, out, nullptr, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -1859,10 +1840,10 @@ extern "C" int slicer_kappa_add(slicer_handle *h, int first_slot, int nplanes, c
   for (int j = 0; j < nplanes; j++)
   {
     const int q = first_slot + j;
-    if (h->plane_npix[q] <= 0)
+    if (h->slots[q].npix <= 0)
       return fail("slicer_kappa_add: slot %d has not been deposited", q);
-    if (h->plane_npix[q] != h->kappa.npix)
-      return fail("slicer_kappa_add: slot %d holds a %d^2 plane, the maps are %d^2", q, h->plane_npix[q], h->kappa.npix);
+    if (h->slots[q].npix != h->kappa.npix)
+      return fail("slicer_kappa_add: slot %d holds a %d^2 plane, the maps are %d^2", q, h->slots[q].npix, h->kappa.npix);
     if (map[j] < 0 || map[j] + nsrc > h->kappa.n)
       return fail("slicer_kappa_add: maps %d..%d of plane %d outside 0..%d", map[j], map[j] + nsrc - 1, j, h->kappa.n - 1);
     for (int k = 0; k < nsrc; k++)
@@ -1883,7 +1864,7 @@ extern "C" int slicer_kappa_add(slicer_handle *h, int first_slot, int nplanes, c
     A.run_mask[A.nruns - 1] |= A.plane_mask[j];
     A.run_begin[A.nruns] = j + 1;
   }
-  if (set_device(h) || resolve_deferred(h, first_slot, nplanes) || wait_settled(h, false) || wait_slot_reduces(h, first_slot, nplanes))
+  if (set_device(h) || read_slots(h, first_slot, nplanes))
     return 1;
   const size_t npix2 = (size_t)h->kappa.npix * h->kappa.npix;
   A.acc = h->d_acc + (size_t)first_slot * h->ntypes_alloc * h->npix2max;
@@ -1928,10 +1909,7 @@ extern "C" int slicer_kappa_fetch(slicer_handle *h, int map, double *out)
   CU(cudaMemcpyAsync(out, h->kappa.maps + (size_t)map * h->kappa.stride, npix2 * sizeof(double), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaMemcpyAsync(&ovf, h->kappa.ovf + map, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaStreamSynchronize(h->compute));
-  if (ovf)
-    return fail("convergence map %d: a fixed-point accumulator it summed exceeded 2^63 (more than %.3g mass units in one pixel at %d "
-                "fraction bits); create the handle with a smaller slicer_config.frac_bits", map, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
-  return 0;
+  return ovf ? fail_overflow(h, "convergence map", map) : 0;
 }
 
 extern "C" int slicer_kappa_load(slicer_handle *h, int map, const double *in)
@@ -2061,10 +2039,7 @@ extern "C" int slicer_shear_fetch(slicer_handle *h, double *gamma1, double *gamm
   CU(cudaMemcpyAsync(gamma2, h->shear.g + npix2, npix2 * sizeof(double), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaMemcpyAsync(&ovf, h->kappa.ovf + map, sizeof(unsigned), cudaMemcpyDeviceToHost, h->compute));
   CU(cudaStreamSynchronize(h->compute));
-  if (ovf)
-    return fail("shear of convergence map %d: a fixed-point accumulator it summed exceeded 2^63 (more than %.3g mass units in one pixel "
-                "at %d fraction bits); create the handle with a smaller slicer_config.frac_bits", map, ldexp(1.0, 63 - h->frac_bits), h->frac_bits);
-  return 0;
+  return ovf ? fail_overflow(h, "shear of convergence map", map) : 0;
 }
 
 extern "C" int slicer_get_stats(slicer_handle *h, slicer_stats *out)
@@ -2147,22 +2122,6 @@ extern "C" int slicer_comm_unique_id(char id[128])
   return 0;
 }
 
-extern "C" int slicer_comm_init_rank(slicer_handle *h, const char id[128], int nranks, int rank)
-{
-  if (!h)
-    return fail("null handle");
-  if (load_nccl() || set_device(h))
-    return 1;
-  if (h->comm)
-    return fail("communicator already initialised");
-  ncclUniqueId u;
-  memcpy(&u, id, 128);
-  NC(g_nccl.CommInitRank(&h->comm, nranks, u, rank));
-  h->nranks = nranks;
-  h->rank = rank;
-  return 0;
-}
-
 extern "C" int slicer_comm_init_ranks(slicer_handle **handles, int n, const char id[128], int nranks, int first_rank)
 {
   if (!handles || n < 1 || first_rank < 0 || first_rank + n > nranks)
@@ -2206,6 +2165,11 @@ extern "C" int slicer_comm_init_ranks(slicer_handle **handles, int n, const char
   return 0;
 }
 
+extern "C" int slicer_comm_init_rank(slicer_handle *h, const char id[128], int nranks, int rank)
+{
+  return slicer_comm_init_ranks(&h, 1, id, nranks, rank);
+}
+
 extern "C" int slicer_comm_init_all(slicer_handle **handles, int n)
 {
   if (!handles || n < 1)
@@ -2236,7 +2200,7 @@ static int enqueue_reduce(slicer_handle *h, int first_slot, int nplanes, int roo
 {
   for (int q = first_slot; q < first_slot + nplanes; q++)
   {
-    const size_t npix2 = h->plane_npix[q] > 0 ? (size_t)h->plane_npix[q] * h->plane_npix[q] : h->npix2max;
+    const size_t npix2 = h->slots[q].npix > 0 ? (size_t)h->slots[q].npix * h->slots[q].npix : h->npix2max;
     for (int t = 0; t < h->ntypes_alloc; t++)
     {
       unsigned long long *a = h->d_acc + ((size_t)q * h->ntypes_alloc + t) * h->npix2max;
@@ -2248,63 +2212,34 @@ static int enqueue_reduce(slicer_handle *h, int first_slot, int nplanes, int roo
   return 0;
 }
 
-// order the reduce after the passes submitted so far, and everything that touches these slots later after the reduce
+// order the reduce after the last pass into each of these slots (not after passes into other slots submitted since) and after the
+// deposits of the pairs libm settled
 static int reduce_fence_before(slicer_handle *h, int first_slot, int nplanes)
 {
-  if (wait_slot_reduces(h, first_slot, nplanes)) // an earlier reduce of the same slots (same stream anyway)
-    return 1;
-  // after the last pass into each of these slots (not after passes into other slots submitted since) and after the deposits
-  // of the pairs libm settled
   bool all = false;
   for (int q = first_slot; q < first_slot + nplanes; q++)
-    all = all || !h->slot_pass_ev[q];
+    all = all || !h->slots[q].written;
   if (all)
   {
-    CU(cudaEventRecord(h->ev_pass_done, h->compute));
-    CU(cudaStreamWaitEvent(h->comm_stream, h->ev_pass_done, 0));
+    if (h->passes_done.signal(h->compute) || h->passes_done.wait(h->comm_stream))
+      return 1;
   }
   else
   {
     cudaEvent_t seen = nullptr;
     for (int q = first_slot; q < first_slot + nplanes; q++)
-      if (h->slot_pass_ev[q] != seen)
+      if (h->slots[q].written != seen)
       {
-        seen = h->slot_pass_ev[q];
+        seen = h->slots[q].written;
         CU(cudaStreamWaitEvent(h->comm_stream, seen, 0));
       }
   }
-  return wait_settled(h, true);
-}
-static int reduce_fence_after(slicer_handle *h, int first_slot, int nplanes)
-{
-  for (int q = first_slot; q < first_slot + nplanes; q++)
-  {
-    CU(cudaEventRecord(h->ev_slot[q], h->comm_stream));
-    h->slot_reducing[q] = true;
-  }
-  return 0;
+  return h->settled_comm.wait(h->comm_stream);
 }
 
 extern "C" int slicer_reduce_slots(slicer_handle *h, int first_slot, int nplanes, int root)
 {
-  if (!h)
-    return fail("null handle");
-  if (nplanes < 1 || first_slot < 0 || first_slot + nplanes > h->cfg.max_planes)
-    return fail("slicer_reduce: slots %d..%d outside 0..%d", first_slot, first_slot + nplanes - 1, h->cfg.max_planes - 1);
-  if (set_device(h) || resolve_deferred(h, first_slot, nplanes))
-    return 1;
-  if (!h->comm || h->nranks == 1)
-    return 0;
-  if (reduce_fence_before(h, first_slot, nplanes))
-    return 1;
-  NC(g_nccl.GroupStart());
-  const int rc = enqueue_reduce(h, first_slot, nplanes, root);
-  const ncclResult_t ge = g_nccl.GroupEnd(); // always closes the group, also when a reduce could not be enqueued
-  if (rc)
-    return rc;
-  if (ge != ncclSuccess)
-    return fail("ncclGroupEnd failed: %s", g_nccl.GetErrorString(ge));
-  return reduce_fence_after(h, first_slot, nplanes);
+  return slicer_reduce_all_slots(&h, 1, first_slot, nplanes, root);
 }
 
 extern "C" int slicer_reduce(slicer_handle *h, int nplanes, int root) { return slicer_reduce_slots(h, 0, nplanes, root); }
@@ -2337,14 +2272,20 @@ extern "C" int slicer_reduce_all_slots(slicer_handle **handles, int n, int first
   int rc = 0;
   for (int i = 0; i < n && !rc; i++)
     rc = set_device(handles[i]) || enqueue_reduce(handles[i], first_slot, nplanes, root);
-  const ncclResult_t ge = g_nccl.GroupEnd();
+  const ncclResult_t ge = g_nccl.GroupEnd(); // always closes the group, also when a reduce could not be enqueued
   if (rc)
     return rc;
   if (ge != ncclSuccess)
     return fail("ncclGroupEnd failed: %s", g_nccl.GetErrorString(ge));
+  // everything that touches these slots later follows the reduce
   for (int i = 0; i < n; i++)
-    if (set_device(handles[i]) || reduce_fence_after(handles[i], first_slot, nplanes))
+  {
+    if (set_device(handles[i]))
       return 1;
+    for (int q = first_slot; q < first_slot + nplanes; q++)
+      if (handles[i]->slots[q].reduced.signal(handles[i]->comm_stream))
+        return 1;
+  }
   return 0;
 }
 

@@ -290,16 +290,19 @@ def test_slots_above_sixteen(oracle):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("finish", ["settle", "reduce"])
+@pytest.mark.parametrize("finish", ["settle", "reduce", "reduce_in_one_rank"])
 def test_interleaved_sets_with_the_libm_path(oracle, finish):
     """guard_eta = 2^-34 sends thousands of pairs per pass to the host's libm.  Three slot ranges are deposited as the driver
     does with three realisations: A, B, C non-accumulating over batch 1, then A, B, C accumulating over batch 2; then each
-    range is settled (or reduced) and read.  Every plane equals the oracle on batch 1 + batch 2 bit for bit."""
+    range is settled (or reduced, also as the only rank of a communicator) and read.  Every plane equals the oracle on batch 1 +
+    batch 2 bit for bit."""
     npix, n = 256, 1 << 20
     batches = [synth.uniform_positions(n, BOX, 81), synth.uniform_positions(n, BOX, 82)]
     sets = [random_planes(seed_triples(1, 500 + 10 * i), [(40.0, 100.0, 0.0), (100.0, 128.0, 0.0)], 0.55, npix) for i in range(3)]
     ranges = [0, 2, 4]
     with capi.Slicer(npix_max=npix, max_planes=6, particle_capacity=n + 64, staging_buffers=2, guard_eta=2.0 ** -34) as s:
+        if finish == "reduce_in_one_rank":
+            s.comm_init_rank(capi.Slicer.comm_unique_id(), 1, 0)
         fb = s.frac_bits
         f0 = int(s.stats().flagged_pairs)
         for b, pos in enumerate(batches):

@@ -276,7 +276,7 @@ def test_library_refusals():
 
 @pytest.mark.gpu
 def test_overflowed_kappa_map_fails_the_fetch():
-    """The accumulator overflow of tests/test_gpu_parity.py, summed into a κ map: its shear is not returned."""
+    """The accumulator overflow of tests/test_gpu_parity.py, summed into a κ map: neither the map nor its shear is returned."""
     box, n = 128000.0, 48
     pos = np.tile(np.array([[0.5, 0.5, 0.3]], np.float32) * np.float32(box), (n, 1))
     d = capi.plane_desc([1, 1, 1], 1, [0.0, 0.0, 0.0], 0.0, 10.0, 100.0, 0.5, 64)
@@ -289,6 +289,8 @@ def test_overflowed_kappa_map_fails_the_fetch():
         s.shear(0, 128)
         with pytest.raises(capi.SlicerError, match="exceeded 2\\^63"):
             s.shear_fetch()
+        with pytest.raises(capi.SlicerError, match="frac_bits"):
+            s.kappa_fetch(0)
 
 
 @pytest.mark.gpu
